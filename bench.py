@@ -1,8 +1,12 @@
 #!/usr/bin/env python
 """bench.py -- frames/s of the per-frame hot path on synthetic 640x512 uint16 IR movies.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+`--dump-outputs DIR` writes what the last timed step returned on rank 0 as DIR/<name>.npy (float32, a
+fixed sample of frames; float64 for the statistics), so that two builds can be compared output for
+output: the inputs depend only on the arguments.
 
 A "step" is one pass of the full per-frame pipeline (bad-pixel correct -> Gaussian u16->f32 ->
 sub-pixel translate with per-frame shifts -> delta + byte-plane pre-coder -> min/max/histogram)
@@ -400,6 +404,34 @@ def workload_config(chunk, n_gpus):
     }
 
 
+DUMP_FRAMES = 8  # 5 outputs x 8 frames x 640x512 x 4 bytes: 52 MB per dump
+
+
+def dump_outputs(path, outs, stats):
+    """Write a fixed sample of frames of each array process_chunk returned (corrected, smoothed, registered, lo, hi) as
+    float32, the sampled frame indices, and the step's statistics (min / max, histogram) as float64, to path/<name>.npy.
+    The sample is frame 0, a key frame of the pre-coder (the chunk starts on a GOP boundary), and seeded others."""
+    import numpy as np
+    import torch
+
+    os.makedirs(path, exist_ok=True)
+    n = outs[0].shape[0]
+    rest = np.random.default_rng(2024).choice(np.arange(1, n), min(n, DUMP_FRAMES) - 1, replace=False)
+    idx = np.concatenate(([0], np.sort(rest)))
+    sel = torch.from_numpy(idx).to(outs[0].device)
+    arrays = {"frame_index": idx.astype(np.float64)}
+    for name, t in zip(("corrected", "smoothed", "registered", "lo", "hi"), outs):
+        if t.dtype == torch.uint16:  # read the bits as signed, then back to unsigned: few torch ops take uint16
+            t = t.view(torch.int16).index_select(0, sel).to(torch.int32) & 0xFFFF
+        else:
+            t = t.index_select(0, sel)
+        arrays[name] = t.to(torch.float32).cpu().numpy()
+    arrays["stats_minmax"] = np.array([stats.min(), stats.max()], dtype=np.float64)
+    arrays["stats_histogram"] = stats.histogram().astype(np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------
 # GPU arm
 # ------------------------------------------------------------------------------------------------
@@ -453,13 +485,18 @@ def run_ours(args, out):
     launches0 = _lib.launch_count()
     t_start.record()
     for k in range(args.steps):
-        pipe.process_chunk(frames, dx, dy, shard.start, events=ev[k])
+        # a dump's statistics are the last step's alone, not a fold of every pass over the same chunk (one launch more)
+        if args.dump_outputs and k == args.steps - 1:
+            pipe.stats.reset()
+        outs = pipe.process_chunk(frames, dx, dy, shard.start, events=ev[k])
     t_stop.record()
     barrier()
     launches = _lib.launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
     ms = t_start.elapsed_time(t_stop)
     per_stage = [sum(ev[k][i].elapsed_time(ev[k][i + 1]) for k in range(args.steps)) / args.steps for i in range(nst)]
+    if args.dump_outputs and rank == 0:  # before the later passes reuse the pipeline's buffers and statistics
+        dump_outputs(args.dump_outputs, outs, pipe.stats)
 
     # the only collective of the path: statistics all-reduce (once per movie; timed for the record)
     warm = movie.MovieStats(dev)  # the first NCCL call of a shape pays its set-up: not what a movie pays per reduction
@@ -689,7 +726,12 @@ def main():
     ap.add_argument("--no-e2e-all", action="store_true", help="skip the host-path figure that also downloads the smoothed frames")
     ap.add_argument("--stream-frames", type=int, default=100000,
                     help="distinct frames (all GPUs together) streamed once through the chunk ring: config 3 as named; 0 = skip")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a sample of the last timed step's outputs to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU path computed: it needs --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     with JsonOnlyStdout() as out:
         if args.impl == "reference":
