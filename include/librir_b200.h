@@ -286,6 +286,18 @@ RIRB_API int rirb_z_image_size(int handle, int* width, int* height);
 RIRB_API int rirb_z_get_timestamps(int handle, long long* times);
 RIRB_API int rirb_z_read_image(int handle, int pos, unsigned short* img, long long* timestamp);
 RIRB_API int rirb_z_read_images(int handle, int pos, int count, unsigned short* out, long long* timestamps, int threads);
+/* Entropy coder of the records written after the call: 0 = host zstd at the file's clevel (the default), 1 = the device
+ * coder (rirb_zstd_encode_batch; clevel is ignored).  Every record is a standalone zstd frame, so a file may mix them.
+ * Returns -1 for an unknown coder, a read handle, or coder 1 without a CUDA device (no CPU fallback). */
+RIRB_API int rirb_z_set_coder(int handle, int coder);
+
+/* Device zstd coder: n payloads of bytes_each bytes back to back at src -> one zstd frame each (RFC 8878: Huffman-coded
+ * literals, no sequences; RLE / raw blocks where they are smaller), frame i at dst + i * dst_stride, its size in sizes[i].
+ * Blocks are at most 128 KiB and never cross a multiple of `segment` bytes (0 = no segments; methods 2/3 pass w*h so that
+ * each byte plane gets its own tables).  src, dst and sizes are DEVICE pointers; the call is asynchronous on the current
+ * stream.  dst_stride must be at least 9 + 3 * blocks + bytes_each (the frame when every block is raw). */
+RIRB_API int rirb_zstd_encode_batch(const unsigned char* src, long long n, long long bytes_each, long long segment,
+                                    unsigned char* dst, long long dst_stride, long long* sizes);
 
 /* ===================== Part 4: the registration front end (SURVEY.md 8f-4) ==================
  * MaskedRegistratorECC.compute, librir/registration/masked_registration_ecc.py:105-191: quantile clamp,

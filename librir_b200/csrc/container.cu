@@ -25,10 +25,10 @@
 // plane] (w*h bytes each) of the image (method 2) or of its temporal residual (method 3: key frame every GOP frames,
 // otherwise (frame[t] - frame[t-1]) mod 2^16; the GOP is stored in trigger word 12 and as the global attribute "GOP").
 // The split / delta and their inverses run on the GPU (rirb_precode_movie / rirb_decode_movie), whole GOPs per launch.
-// The entropy stage stays on the host (the north star's choice).  What this file adds over the
-// reference is that a run of frames is compressed / decompressed by a pool of host threads while the
-// records keep their order, and that frames may be handed over as device pointers (downloaded /
-// uploaded in one copy per call).
+// The entropy stage is host zstd by default.  What this file adds over the reference is that a run of frames is compressed /
+// decompressed by a pool of host threads while the records keep their order, that frames may be handed over as device
+// pointers (downloaded / uploaded in one copy per call), and that a writer may switch to the device coder (zcoder.cu,
+// rirb_z_set_coder): the payloads are then encoded in HBM and one copy per pass brings back the packed records.
 #include <dlfcn.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -452,6 +452,42 @@ static bool z_unpark_buffers(size_t host_bytes, size_t dev_bytes, int device, ch
     return true;
 }
 
+// The device coder's buffers: its scratch, the packed records of a pass on the device and their pinned copy.  Parked like the
+// pair above when a file closes (pinning is the expensive part), so that the next file of the process starts warm.
+struct ZcBuffers {
+    char* scratch = nullptr;
+    char* dev = nullptr;
+    char* host = nullptr;
+    size_t scratch_bytes = 0, dev_bytes = 0, host_bytes = 0;
+    int device = -1;
+};
+static std::mutex g_zc_mu;
+static ZcBuffers g_zc_parked;
+static void zc_free(ZcBuffers& b)
+{
+    if (b.scratch) cudaFree(b.scratch);
+    if (b.dev) cudaFree(b.dev);
+    if (b.host) cudaFreeHost(b.host);
+    (void)cudaGetLastError();
+    b = ZcBuffers();
+}
+static void zc_park(ZcBuffers& b)
+{
+    if (!b.scratch && !b.dev && !b.host) return;
+    {
+        std::lock_guard<std::mutex> lock(g_zc_mu);
+        std::swap(b, g_zc_parked);  // the newer set is kept, the older one freed
+    }
+    zc_free(b);
+}
+static void zc_unpark(ZcBuffers& b, int device)
+{
+    std::lock_guard<std::mutex> lock(g_zc_mu);
+    if (g_zc_parked.device != device) return;
+    b = g_zc_parked;
+    g_zc_parked = ZcBuffers();
+}
+
 struct ZMovie {
     bool writing = false;
     std::string filename;
@@ -478,10 +514,14 @@ struct ZMovie {
     long long cache_first = -1, cache_count = 0;  // reading: decoded frames [cache_first, +cache_count) still in dev_buf
     std::mutex mu;
     size_t host_bytes = 0, dev_bytes = 0;  // what the two buffers really hold (a pair taken over may be larger than asked)
+    // writing with the device coder (coder 1): its scratch, the packed records of a pass on the device and their pinned copy
+    int coder = 0;
+    ZcBuffers zc;
     ~ZMovie()
     {
         if (f) fclose(f);
         z_park_buffers(host_planes, host_bytes, dev_buf, dev_bytes, dev_device);
+        zc_park(zc);
     }
     // grow-only work space for m frames; false + set_error when memory runs out
     bool reserve(size_t m)
@@ -809,9 +849,97 @@ int rirb_z_write_images(int handle, const unsigned short* frames, long long nfra
                           : z_write_precoded(z.get(), frames, nframes, timestamps, threads);
 }
 
+// grow-only buffers of the device coder; false + set_error when memory runs out
+static bool z_grow(char** p, size_t* have, size_t need, bool pinned)
+{
+    if (*have >= need) return true;
+    if (*p) (void)(pinned ? cudaFreeHost(*p) : cudaFree(*p));
+    *p = nullptr;
+    *have = 0;
+    if ((pinned ? cudaMallocHost((void**)p, need) : cudaMalloc((void**)p, need)) != cudaSuccess) {
+        cudaGetLastError();
+        *p = nullptr;
+        set_error("zstd movie file: out of %s memory for the device coder (%zu bytes)", pinned ? "pinned host" : "device", need);
+        return false;
+    }
+    *have = need;
+    return true;
+}
+
+// m payloads of bytes_each bytes on the DEVICE -> device coder -> records packed back to back -> host -> one pwrite
+static int z_encode_records(ZMovie* z, const u8* src, long long m, long long bytes_each, long long segment, const long long* timestamps)
+{
+    cudaStream_t st = current_stream();
+    const size_t records = (size_t)m * (size_t)(12 + zcoder_frame_bound(bytes_each, segment));
+    const size_t head = ((size_t)(m + 1) * 8 + 63) & ~(size_t)63;  // pinned: the record offsets, then the records
+    ZcBuffers& b = z->zc;
+    int dev = 0;
+    cudaGetDevice(&dev);
+    if (b.device != dev) {
+        zc_free(b);
+        zc_unpark(b, dev);
+        b.device = dev;
+    }
+    if (!z_grow(&b.scratch, &b.scratch_bytes, zcoder_scratch_bytes(m, bytes_each, segment), false) ||
+        !z_grow(&b.dev, &b.dev_bytes, records, false) || !z_grow(&b.host, &b.host_bytes, head + records, true))
+        return -1;
+    long long* dev_off = nullptr;
+    if (launch_zstd_encode(src, m, bytes_each, segment, (u8*)b.dev, 0, 12, nullptr, &dev_off, b.scratch, st) != 0) return -1;
+    long long* off = (long long*)b.host;
+    char* rec = b.host + head;
+    RIRB_CUDA_OK(cudaMemcpyAsync(off, dev_off, (size_t)(m + 1) * 8, cudaMemcpyDeviceToHost, st));
+    RIRB_CUDA_OK(cudaStreamSynchronize(st));
+    const long long total = off[m];
+    RIRB_CUDA_OK(cudaMemcpyAsync(rec, b.dev, (size_t)total, cudaMemcpyDeviceToHost, st));
+    RIRB_CUDA_OK(cudaStreamSynchronize(st));
+    for (long long i = 0; i < m; ++i) {  // record = i64 timestamp, u32 size, payload
+        const int64_t ts = timestamps[i];
+        const uint32_t c32 = (uint32_t)((i + 1 < m ? off[i + 1] : total) - off[i] - 12);
+        memcpy(rec + off[i], &ts, 8);
+        memcpy(rec + off[i] + 8, &c32, 4);
+    }
+    const int fd = fileno(z->f);
+    for (long long done = 0; done < total;) {
+        const ssize_t w = pwrite(fd, rec + done, (size_t)(total - done), (off_t)(z->pos + done));
+        if (w <= 0) {
+            set_error("z_write_images: write failed");
+            return -1;
+        }
+        done += w;
+    }
+    for (long long i = 0; i < m; ++i) {
+        z->times.push_back(timestamps[i]);
+        z->positions.push_back(z->pos + off[i]);
+    }
+    z->pos += total;
+    return 0;
+}
+
+// method 1 with the device coder: device frames are encoded where they are, host frames go up in passes of ~64 MB
+static int z_write_records_device(ZMovie* z, const void* frames, long long nframes, const long long* timestamps)
+{
+    const size_t fbytes = (size_t)z->w * z->h * 2;
+    const long long chunk = std::max<long long>(1, (64ll << 20) / (long long)fbytes);
+    const bool on_device = device_pointer(frames);
+    cudaStream_t st = current_stream();
+    for (long long done = 0; done < nframes;) {
+        const long long m = std::min(chunk, nframes - done);
+        const u8* src = (const u8*)frames + (size_t)done * fbytes;
+        if (!on_device) {
+            if (!z->reserve((size_t)chunk)) return -1;
+            RIRB_CUDA_OK(cudaMemcpyAsync(z->dev_movie(), src, (size_t)m * fbytes, cudaMemcpyHostToDevice, st));
+            src = (const u8*)z->dev_movie();
+        }
+        if (z_encode_records(z, src, m, (long long)fbytes, 0, timestamps + done) != 0) return -1;
+        done += m;
+    }
+    return 0;
+}
+
 // `nframes` payloads of w*h*2 bytes each, back to back at `frames` (host or device) -> zstd -> records
 static int z_write_records(ZMovie* z, const void* frames, long long nframes, const long long* timestamps, int threads)
 {
+    if (z->coder == 1) return z_write_records_device(z, frames, nframes, timestamps);
     const size_t fbytes = (size_t)z->w * z->h * 2;
     const size_t bound = zstd().compressBound(fbytes);
     const int workers = pool_size(threads, nframes);
@@ -918,6 +1046,15 @@ static int z_flush_gops(ZMovie* z, const u16* dev_frames, long long m, long long
     cudaStream_t st = current_stream();
     ZPhase ph;
     if (rirb_precode_movie(dev_frames, m, z->w, z->h, z->gop, z->method == 3, first, z->dev_lo(), z->dev_hi()) != 0) return -1;
+    if (z->coder == 1) {
+        // per frame [lo | hi] into the frames' part of dev_buf (the pre-coder has read them by now, in stream order)
+        u8* planes = (u8*)z->dev_movie();
+        RIRB_CUDA_OK(cudaMemcpy2DAsync(planes, 2 * npx, z->dev_lo(), npx, npx, (size_t)m, cudaMemcpyDeviceToDevice, st));
+        RIRB_CUDA_OK(cudaMemcpy2DAsync(planes + npx, 2 * npx, z->dev_hi(), npx, npx, (size_t)m, cudaMemcpyDeviceToDevice, st));
+        const int rc = z_encode_records(z, planes, m, 2 * (long long)npx, (long long)npx, timestamps);
+        ph.mark("write: pre-code + device zstd", m);
+        return rc;
+    }
     // per frame [lo | hi], so that a record's payload is one contiguous run for zstd
     RIRB_CUDA_OK(cudaMemcpy2DAsync(z->host_planes, 2 * npx, z->dev_lo(), npx, npx, (size_t)m, cudaMemcpyDeviceToHost, st));
     RIRB_CUDA_OK(cudaMemcpy2DAsync(z->host_planes + npx, 2 * npx, z->dev_hi(), npx, npx, (size_t)m, cudaMemcpyDeviceToHost, st));
@@ -926,6 +1063,13 @@ static int z_flush_gops(ZMovie* z, const u16* dev_frames, long long m, long long
     const int rc = z_write_records(z, z->host_planes, m, timestamps, threads);
     ph.mark("write: zstd + records", m);
     return rc;
+}
+
+// one device frame into the pending GOP (host): on the caller's stream, so that it sees the work queued there
+static cudaError_t z_download_frame(void* dst, const void* src, size_t bytes, cudaStream_t st)
+{
+    const cudaError_t e = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, st);
+    return e == cudaSuccess ? cudaStreamSynchronize(st) : e;
 }
 
 // methods 2 / 3.  Whole GOPs go through the GPU pre-coder as they come; what does not fill a GOP waits in z->pending
@@ -945,7 +1089,7 @@ static int z_write_precoded(ZMovie* z, const unsigned short* frames, long long n
         const size_t have = z->pending_times.size();
         z->pending.resize((have + 1) * npx);
         if (on_device)
-            RIRB_CUDA_OK(cudaMemcpy(z->pending.data() + have * npx, frames + (size_t)done * npx, npx * 2, cudaMemcpyDeviceToHost));
+            RIRB_CUDA_OK(z_download_frame(z->pending.data() + have * npx, frames + (size_t)done * npx, npx * 2, st));
         else
             memcpy(z->pending.data() + have * npx, frames + (size_t)done * npx, npx * 2);
         z->pending_times.push_back(timestamps[done]);
@@ -975,7 +1119,7 @@ static int z_write_precoded(ZMovie* z, const unsigned short* frames, long long n
         const size_t have = z->pending_times.size();
         z->pending.resize((have + 1) * npx);
         if (on_device)
-            RIRB_CUDA_OK(cudaMemcpy(z->pending.data() + have * npx, frames + (size_t)done * npx, npx * 2, cudaMemcpyDeviceToHost));
+            RIRB_CUDA_OK(z_download_frame(z->pending.data() + have * npx, frames + (size_t)done * npx, npx * 2, st));
         else
             memcpy(z->pending.data() + have * npx, frames + (size_t)done * npx, npx * 2);
         z->pending_times.push_back(timestamps[done]);
@@ -995,6 +1139,26 @@ static int z_flush_pending(ZMovie* z)
     z->pending.clear();
     z->pending_times.clear();
     return rc;
+}
+
+int rirb_z_set_coder(int handle, int coder)
+{
+    auto z = g_zfiles.get(handle);
+    if (!z || !z->writing) {
+        set_error("z_set_coder: not a handle open for writing");
+        return -1;
+    }
+    if (coder != 0 && coder != 1) {
+        set_error("z_set_coder: coder must be 0 (host zstd) or 1 (device coder), not %d", coder);
+        return -1;
+    }
+    if (coder == 1 && rirb_device_count() <= 0) {
+        set_error("z_set_coder: the device coder needs a CUDA device (no CPU fallback)");
+        return -1;
+    }
+    std::lock_guard<std::mutex> lock(z->mu);
+    z->coder = coder;
+    return 0;
 }
 
 int rirb_z_write_image(int handle, const unsigned short* img, long long timestamp)

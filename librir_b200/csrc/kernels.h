@@ -78,6 +78,15 @@ int launch_precode_movie_stats(const u16* mov, long long nframes, int w, int h, 
 int launch_decode_movie(const u8* lo, const u8* hi, long long nframes, int w, int h, int gop, int delta, long long first_frame,
                         u16* mov, cudaStream_t st);
 
+// zcoder.cu: n payloads of bytes_each bytes at src -> one zstd frame each (blocks cut at multiples of `segment` bytes, 0 = none).
+// dst_stride > 0: frame i at dst + i * dst_stride.  dst_stride == 0: records packed back to back, frame i at
+// foff[i] + rec_head with foff[n] = the total; rec_head bytes before each frame are left for the caller.  sizes (may be null):
+// frame bytes.  *frame_offsets (may be null) receives the device array foff (inside scratch).
+size_t zcoder_scratch_bytes(long long n, long long bytes_each, long long segment);
+long long zcoder_frame_bound(long long bytes_each, long long segment);  // the largest frame: raw blocks plus headers
+int launch_zstd_encode(const u8* src, long long n, long long bytes_each, long long segment, u8* dst, long long dst_stride,
+                       int rec_head, long long* sizes, long long** frame_offsets, void* scratch, cudaStream_t st);
+
 // lossy.cu (H264_Saver::addImageLossyNoCamera, h264.cpp:2253-2424)
 size_t lossy_scalars_bytes();
 int launch_lossy_first(const u16* tmp, u16* out, u16* lastDL, u16* refT, u16* prevT, int n, int ns, int subtract_min, void* scalars,
