@@ -93,8 +93,11 @@ RIRB_API const char* rirb_version(void);
  * "ecc_queue" (default 1): rirb_ecc_track solves runs of up to 16 device-resident frames in ONE cooperative launch (the
  *   warm start stays on the device, a frame that fails or triggers the replacement of the reference image ends the
  *   run) instead of one launch + copy back + synchronisation per frame.
+ * "zstd_decoder" (default 1): a method-1 zstd movie file read into device memory whose first record has no LZ sequences
+ *   (what the device coder writes) uploads the records and decodes them with rirb_zstd_decode_batch; 2: every read that
+ *   ends on the device does (methods 2/3 too); 0: host libzstd for every read.  2 and 0 are for A/B runs.
  * Initial values can also come from RIRB_TRANSLATE_TMA / RIRB_GAUSS_TMA / RIRB_LOADER_FUSED / RIRB_ECC_FUSED /
- * RIRB_LOSSY_RUN / RIRB_TRANSLATE_ROWS / RIRB_ECC_QUEUE.  -1: unknown key. */
+ * RIRB_LOSSY_RUN / RIRB_TRANSLATE_ROWS / RIRB_ECC_QUEUE / RIRB_ZSTD_DECODER.  -1: unknown key. */
 RIRB_API int rirb_set_parameter(const char* key, const char* value);
 
 /* ---- batches of frames (nframes dense frames back to back) ---- */
@@ -298,6 +301,13 @@ RIRB_API int rirb_z_set_coder(int handle, int coder);
  * stream.  dst_stride must be at least 9 + 3 * blocks + bytes_each (the frame when every block is raw). */
 RIRB_API int rirb_zstd_encode_batch(const unsigned char* src, long long n, long long bytes_each, long long segment,
                                     unsigned char* dst, long long dst_stride, long long* sizes);
+
+/* Device zstd decoder: n zstd frames, frame i at src + offsets[i] (sizes[i] bytes) -> its content at dst + i * dst_stride,
+ * at most dst_capacity bytes.  status[i] = bytes written, -1 = malformed frame, -2 = a frame this decoder does not take
+ * (dictionary ID, content checksum, skippable frame, bytes after the frame's last block).  All pointers are DEVICE
+ * pointers; asynchronous on the current stream.  Returns -1 (and sets the last error) for bad arguments or no device. */
+RIRB_API int rirb_zstd_decode_batch(const unsigned char* src, const long long* offsets, const unsigned* sizes, long long n,
+                                    unsigned char* dst, long long dst_stride, long long dst_capacity, long long* status);
 
 /* ===================== Part 4: the registration front end (SURVEY.md 8f-4) ==================
  * MaskedRegistratorECC.compute, librir/registration/masked_registration_ecc.py:105-191: quantile clamp,

@@ -66,9 +66,9 @@ void set_error(const char* fmt, ...)
 cudaStream_t current_stream() { return tls.stream; }
 
 // ---- run-time switches ---------------------------------------------------------------------------
-static const char* const k_opt_names[OPT_COUNT] = {"translate_tma", "gauss_tma", "loader_fused", "ecc_fused", "lossy_run", "translate_rows", "ecc_queue"};
-static const char* const k_opt_env[OPT_COUNT] = {"RIRB_TRANSLATE_TMA", "RIRB_GAUSS_TMA", "RIRB_LOADER_FUSED", "RIRB_ECC_FUSED", "RIRB_LOSSY_RUN", "RIRB_TRANSLATE_ROWS", "RIRB_ECC_QUEUE"};
-static const int k_opt_default[OPT_COUNT] = {1, 1, 0, 1, 1, 1, 1};
+static const char* const k_opt_names[OPT_COUNT] = {"translate_tma", "gauss_tma", "loader_fused", "ecc_fused", "lossy_run", "translate_rows", "ecc_queue", "zstd_decoder"};
+static const char* const k_opt_env[OPT_COUNT] = {"RIRB_TRANSLATE_TMA", "RIRB_GAUSS_TMA", "RIRB_LOADER_FUSED", "RIRB_ECC_FUSED", "RIRB_LOSSY_RUN", "RIRB_TRANSLATE_ROWS", "RIRB_ECC_QUEUE", "RIRB_ZSTD_DECODER"};
+static const int k_opt_default[OPT_COUNT] = {1, 1, 0, 1, 1, 1, 1, 1};
 static std::atomic<int> g_opts[OPT_COUNT];
 static std::once_flag g_opts_once;
 static void init_options()

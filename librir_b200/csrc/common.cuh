@@ -26,7 +26,7 @@ cudaStream_t current_stream();
 extern std::atomic<long long> g_launches;
 int sm_count();
 // run-time switches (rirb_set_parameter; initial values from the environment): kernel variants for A/B runs
-enum { OPT_TRANSLATE_TMA = 0, OPT_GAUSS_TMA = 1, OPT_LOADER_FUSED = 2, OPT_ECC_FUSED = 3, OPT_LOSSY_RUN = 4, OPT_TRANSLATE_ROWS = 5, OPT_ECC_QUEUE = 6, OPT_COUNT = 7 };
+enum { OPT_TRANSLATE_TMA = 0, OPT_GAUSS_TMA = 1, OPT_LOADER_FUSED = 2, OPT_ECC_FUSED = 3, OPT_LOSSY_RUN = 4, OPT_TRANSLATE_ROWS = 5, OPT_ECC_QUEUE = 6, OPT_ZSTD_DECODER = 7, OPT_COUNT = 8 };
 bool option_enabled(int which);
 int option_value(int which);  // the switch's integer value (option_enabled: != 0)
 

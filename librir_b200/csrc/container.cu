@@ -1,6 +1,6 @@
 // librir_b200/csrc/container.cu -- the on-disk formats either side of the path (SURVEY.md 8f-3).
 //
-// Host code only (no kernels): what the per-frame path reads from and writes to when it runs inside
+// Host code (the zstd kernels are zcoder.cu / zdecoder.cu): what the per-frame path reads from and writes to when it runs inside
 // librir's own file tooling.
 //   attribute trailer   rir::FileAttributes, FileAttributes.cpp:51-165 (strings, maps), :250-372
 //                       (open / openReadOnly), :454-514 (writeIfDirty); C interface tools.cpp:87-350
@@ -29,6 +29,12 @@
 // decompressed by a pool of host threads while the records keep their order, that frames may be handed over as device
 // pointers (downloaded / uploaded in one copy per call), and that a writer may switch to the device coder (zcoder.cu,
 // rirb_z_set_coder): the payloads are then encoded in HBM and one copy per pass brings back the packed records.
+// A method-1 read into device memory of records without LZ sequences (the device coder's) goes the other way through
+// the device decoder (zdecoder.cu): a pass's records are one span of the file, read into pinned memory, uploaded in one
+// copy and decoded in HBM; a record it refuses (checksum, dictionary, ...) or finds malformed is decoded by host zstd
+// instead.  Records with sequences stay on the host pool, which decodes them faster (DESIGN.md 7 f-3, r4), and so does
+// method 1 into host memory, so a host-only caller never initialises CUDA.  The "zstd_decoder" switch: 2 sends every
+// read that ends on the device (methods 2/3 too) through the device decoder, 0 none; both for A/B runs.
 #include <dlfcn.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -832,6 +838,7 @@ int rirb_z_open_file_write_gop(const char* filename, int width, int height, int 
 static int z_write_records(ZMovie* z, const void* frames, long long nframes, const long long* timestamps, int threads);
 static int z_read_records(ZMovie* z, int pos, int count, void* out, long long* timestamps, int threads, bool to_pinned_planes);
 static int z_read_precoded(ZMovie* z, int pos, int count, unsigned short* out, int threads);
+static int z_read_records_device(ZMovie* z, int pos, int count, u8* out, int threads);
 static int z_write_precoded(ZMovie* z, const unsigned short* frames, long long nframes, const long long* timestamps, int threads);
 
 // frames[nframes][h][w] host or device; timestamps host.  Records are appended in order; the frames
@@ -859,7 +866,7 @@ static bool z_grow(char** p, size_t* have, size_t need, bool pinned)
     if ((pinned ? cudaMallocHost((void**)p, need) : cudaMalloc((void**)p, need)) != cudaSuccess) {
         cudaGetLastError();
         *p = nullptr;
-        set_error("zstd movie file: out of %s memory for the device coder (%zu bytes)", pinned ? "pinned host" : "device", need);
+        set_error("zstd movie file: out of %s memory for the device zstd buffers (%zu bytes)", pinned ? "pinned host" : "device", need);
         return false;
     }
     *have = need;
@@ -1310,6 +1317,44 @@ int rirb_z_get_timestamps(int handle, long long* times)
 }
 
 // frames [pos, pos + count) -> out[count][h][w] (host or device), timestamps (host, may be NULL)
+// Whether record i is a zstd frame with LZ sequences in some block (or cannot be walked).  The device decoder runs the
+// sequences of a frame on one warp, which is slower than the host pool (DESIGN.md 7 f-3, r4); frames without sequences --
+// what the device coder writes -- it decodes faster.  A read takes the decoder by its first record.
+static bool z_record_has_sequences(ZMovie* z, long long i)
+{
+    std::vector<u8> f(z->sizes[i]);
+    if (pread(fileno(z->f), f.data(), f.size(), (off_t)(z->positions[i] + 12)) != (ssize_t)f.size() || f.size() < 6) return true;
+    const size_t n = f.size();
+    const unsigned fhd = f[4];
+    const int single = (fhd >> 5) & 1, fcs_flag = fhd >> 6;
+    size_t p = 5 + (single ? 0 : 1) + (size_t)((fhd & 3) == 3 ? 4 : (fhd & 3)) + (size_t)(fcs_flag ? 1 << fcs_flag : single);
+    for (;;) {
+        if (p + 3 > n) return true;
+        const unsigned h = f[p] | (f[p + 1] << 8) | (f[p + 2] << 16), type = (h >> 1) & 3, size = h >> 3;
+        p += 3;
+        if (type == 2) {
+            if (p + size > n || size < 3) return true;
+            const unsigned b0 = f[p], lt = b0 & 3, sf = (b0 >> 2) & 3;
+            size_t hs, cs;
+            if (lt < 2) {
+                hs = (sf & 1) == 0 ? 1 : sf == 1 ? 2 : 3;
+                const size_t regen = hs == 1 ? b0 >> 3 : hs == 2 ? (b0 >> 4) + (f[p + 1] << 4) : (b0 >> 4) + (f[p + 1] << 4) + (f[p + 2] << 12);
+                cs = lt == 0 ? regen : 1;
+            } else {
+                hs = sf < 2 ? 3 : sf + 2;
+                uint64_t v = 0;
+                for (size_t k = 0; k < hs && p + k < n; ++k) v |= (uint64_t)f[p + k] << (8 * k);
+                const int bits = sf < 2 ? 10 : sf == 2 ? 14 : 18;
+                cs = (size_t)((v >> (4 + bits)) & ((1u << bits) - 1));
+            }
+            if (p + hs + cs >= p + size || f[p + hs + cs] != 0) return true;
+        }
+        if (type == 3) return true;
+        p += type == 1 ? 1 : size;
+        if (h & 1) return false;
+    }
+}
+
 int rirb_z_read_images(int handle, int pos, int count, unsigned short* out, long long* timestamps, int threads)
 {
     auto z = g_zfiles.get(handle);
@@ -1319,8 +1364,9 @@ int rirb_z_read_images(int handle, int pos, int count, unsigned short* out, long
     }
     if (count == 0) return 0;
     std::lock_guard<std::mutex> lock(z->mu);
-    if (z->method != 1) {
-        const int rc = z_read_precoded(z.get(), pos, count, out, threads);
+    if (z->method != 1 || (option_enabled(OPT_ZSTD_DECODER) && device_pointer(out) &&
+                           (option_value(OPT_ZSTD_DECODER) == 2 || !z_record_has_sequences(z.get(), pos)))) {
+        const int rc = z->method != 1 ? z_read_precoded(z.get(), pos, count, out, threads) : z_read_records_device(z.get(), pos, count, (u8*)out, threads);
         if (rc == 0 && timestamps)
             for (int i = 0; i < count; ++i) timestamps[i] = z->times[pos + i];
         return rc;
@@ -1395,7 +1441,104 @@ static int z_read_records(ZMovie* z, int pos, int count, void* out, long long* t
     return 0;
 }
 
-// methods 2 / 3: records -> planes (host) -> device -> merge (+ undo the temporal delta from the GOP's key frame on).
+// Records [pos, pos + count) -> their payloads (w*h*2 bytes each) back to back at `out` in DEVICE memory, decoded by the
+// device decoder: per pass of ~64 MB of payloads, the records' span of the file is read into pinned memory (by the host
+// pool when it is large), goes up in one copy with its offset / size table, and is decoded in place.  A record the decoder
+// refuses or finds malformed is decoded by host libzstd from the bytes already read; if that fails too, the read fails.
+static int z_read_records_device(ZMovie* z, int pos, int count, u8* out, int threads)
+{
+    const size_t fbytes = (size_t)z->w * z->h * 2;
+    const long long chunk = std::max<long long>(1, (64ll << 20) / (long long)fbytes);
+    cudaStream_t st = current_stream();
+    ZcBuffers& b = z->zc;
+    int dev = 0;
+    cudaGetDevice(&dev);
+    if (b.device != dev) {
+        zc_free(b);
+        zc_unpark(b, dev);
+        b.device = dev;
+    }
+    const int fd = fileno(z->f);
+    long long fallbacks = 0;
+    for (long long p0 = pos; p0 < (long long)pos + count;) {
+        const long long m = std::min<long long>(chunk, (long long)pos + count - p0);
+        ZPhase ph;
+        const long long a = z->positions[p0];
+        const size_t span = (size_t)(z->positions[p0 + m - 1] + 12 + (long long)z->sizes[p0 + m - 1] - a);
+        const size_t table = ((span + 63) & ~(size_t)63);  // pinned: the span, then offsets | statuses | sizes
+        const size_t bytes = table + (size_t)m * (8 + 8 + 4);
+        if (!z_grow(&b.scratch, &b.scratch_bytes, zdecoder_scratch_bytes(m, (long long)fbytes), false) ||
+            !z_grow(&b.dev, &b.dev_bytes, bytes, false) || !z_grow(&b.host, &b.host_bytes, bytes, true))
+            return -1;
+        char* h = b.host;
+        long long* off = (long long*)(h + table);
+        long long* status = off + m;
+        unsigned* len = (unsigned*)(status + m);
+        for (long long i = 0; i < m; ++i) {
+            off[i] = z->positions[p0 + i] + 12 - a;  // past the record's timestamp and size
+            len[i] = z->sizes[p0 + i];
+        }
+        const size_t piece = 4u << 20;
+        const long long npieces = (long long)((span + piece - 1) / piece);
+        std::atomic<bool> failed{false};
+        parallel_for(npieces, pool_size(threads, npieces), [&](long long k, int) {
+            const size_t lo = (size_t)k * piece, n = std::min(piece, span - lo);
+            for (size_t have = 0; have < n && !failed;) {
+                const ssize_t r = pread(fd, h + lo + have, n - have, (off_t)(a + (long long)(lo + have)));
+                if (r <= 0) failed = true;
+                have += r > 0 ? (size_t)r : 0;
+            }
+        });
+        if (failed) {
+            set_error("z_read_images: a record cannot be read or does not decompress to a %d x %d image", z->w, z->h);
+            return -1;
+        }
+        ph.mark("read: pread span", m);
+        const u8* d = (const u8*)b.dev;
+        long long* dstatus = (long long*)(b.dev + ((char*)status - h));
+        u8* to = out + (size_t)(p0 - pos) * fbytes;
+        RIRB_CUDA_OK(cudaMemcpyAsync(b.dev, h, bytes, cudaMemcpyHostToDevice, st));
+        if (launch_zstd_decode(d, (const long long*)(d + table), (const unsigned*)(d + ((char*)len - h)), m, to, (long long)fbytes,
+                               (long long)fbytes, dstatus, b.scratch, st) != 0)
+            return -1;
+        RIRB_CUDA_OK(cudaMemcpyAsync(status, dstatus, (size_t)m * 8, cudaMemcpyDeviceToHost, st));
+        RIRB_CUDA_OK(cudaStreamSynchronize(st));
+        ph.mark("read: upload + device zstd", m);
+        std::vector<long long> redo;
+        for (long long i = 0; i < m; ++i) {
+            if (status[i] == -1 || status[i] == -2)
+                redo.push_back(i);
+            else if (status[i] != (long long)fbytes) {
+                set_error("z_read_images: a record cannot be read or does not decompress to a %d x %d image", z->w, z->h);
+                return -1;
+            }
+        }
+        if (!redo.empty()) {
+            const int workers = pool_size(threads, (long long)redo.size());
+            if (!z->ctx || (int)z->ctx->c.size() < workers) z->ctx.reset(new Contexts(workers, false));
+            std::vector<char> host((size_t)redo.size() * fbytes);
+            parallel_for((long long)redo.size(), workers, [&](long long j, int t) {
+                const long long i = redo[j];
+                const size_t got = z_decompress(z->ctx->get(t), host.data() + (size_t)j * fbytes, fbytes, h + off[i], len[i]);
+                if (zstd().isError(got) || got != fbytes) failed = true;
+            });
+            if (failed) {
+                set_error("z_read_images: a record cannot be read or does not decompress to a %d x %d image", z->w, z->h);
+                return -1;
+            }
+            for (size_t j = 0; j < redo.size(); ++j)
+                RIRB_CUDA_OK(cudaMemcpyAsync(to + (size_t)redo[j] * fbytes, host.data() + j * fbytes, fbytes, cudaMemcpyHostToDevice, st));
+            RIRB_CUDA_OK(cudaStreamSynchronize(st));
+            fallbacks += (long long)redo.size();
+            ph.mark("read: host zstd fallback", (long long)redo.size());
+        }
+        p0 += m;
+    }
+    if (z_trace() && fallbacks) fprintf(stderr, "[rirb z] %-28s %6lld frames\n", "read: records on host zstd", fallbacks);
+    return 0;
+}
+
+// methods 2 / 3: records -> planes (host, or the device decoder when "zstd_decoder" is 2) -> device -> merge (+ undo the temporal delta from the GOP's key frame on).
 // The decoded frames of the last pass stay in z->dev_buf: a reader that asks for one frame at a time decodes a GOP once.
 static int z_read_precoded(ZMovie* z, int pos, int count, unsigned short* out, int threads)
 {
@@ -1419,10 +1562,18 @@ static int z_read_precoded(ZMovie* z, int pos, int count, unsigned short* out, i
             if (!z->reserve((size_t)chunk)) return -1;
             ph.mark("read: reserve", m);
             z->cache_first = -1;
-            if (z_read_records(z, (int)k0, (int)m, z->host_planes, nullptr, threads, true) != 0) return -1;
-            ph.mark("read: records + zstd", m);
-            RIRB_CUDA_OK(cudaMemcpy2DAsync(z->dev_lo(), npx, z->host_planes, 2 * npx, npx, (size_t)m, cudaMemcpyHostToDevice, st));
-            RIRB_CUDA_OK(cudaMemcpy2DAsync(z->dev_hi(), npx, z->host_planes + npx, 2 * npx, npx, (size_t)m, cudaMemcpyHostToDevice, st));
+            if (option_value(OPT_ZSTD_DECODER) == 2) {
+                // [frame][lo | hi] into the frames' part of dev_buf, then apart into the two plane buffers
+                u8* planes = (u8*)z->dev_movie();
+                if (z_read_records_device(z, (int)k0, (int)m, planes, threads) != 0) return -1;
+                RIRB_CUDA_OK(cudaMemcpy2DAsync(z->dev_lo(), npx, planes, 2 * npx, npx, (size_t)m, cudaMemcpyDeviceToDevice, st));
+                RIRB_CUDA_OK(cudaMemcpy2DAsync(z->dev_hi(), npx, planes + npx, 2 * npx, npx, (size_t)m, cudaMemcpyDeviceToDevice, st));
+            } else {
+                if (z_read_records(z, (int)k0, (int)m, z->host_planes, nullptr, threads, true) != 0) return -1;
+                ph.mark("read: records + zstd", m);
+                RIRB_CUDA_OK(cudaMemcpy2DAsync(z->dev_lo(), npx, z->host_planes, 2 * npx, npx, (size_t)m, cudaMemcpyHostToDevice, st));
+                RIRB_CUDA_OK(cudaMemcpy2DAsync(z->dev_hi(), npx, z->host_planes + npx, 2 * npx, npx, (size_t)m, cudaMemcpyHostToDevice, st));
+            }
             if (rirb_decode_movie(z->dev_lo(), z->dev_hi(), m, z->w, z->h, z->gop, z->method == 3, k0, z->dev_movie()) != 0) return -1;
             z->cache_first = k0;
             z->cache_count = m;

@@ -86,6 +86,11 @@ size_t zcoder_scratch_bytes(long long n, long long bytes_each, long long segment
 long long zcoder_frame_bound(long long bytes_each, long long segment);  // the largest frame: raw blocks plus headers
 int launch_zstd_encode(const u8* src, long long n, long long bytes_each, long long segment, u8* dst, long long dst_stride,
                        int rec_head, long long* sizes, long long** frame_offsets, void* scratch, cudaStream_t st);
+// zdecoder.cu: n zstd frames (frame i at src + offsets[i], sizes[i] bytes) -> content at dst + i * dst_stride, at most cap
+// bytes; status[i] = bytes, -1 malformed, -2 refused (rirb_zstd_decode_batch).  scratch: zdecoder_scratch_bytes(n, cap).
+size_t zdecoder_scratch_bytes(long long n, long long cap);
+int launch_zstd_decode(const u8* src, const long long* offsets, const unsigned* sizes, long long n, u8* dst, long long dst_stride,
+                       long long cap, long long* status, void* scratch, cudaStream_t st);
 
 // lossy.cu (H264_Saver::addImageLossyNoCamera, h264.cpp:2253-2424)
 size_t lossy_scalars_bytes();

@@ -4,11 +4,17 @@ thread-pooled container (rirb_z_write_images / rirb_z_read_images) next to the c
 (oracle/_ref, one frame per call on one thread -- what z_write_image / z_read_image do).  Host work; the GPU
 only appears in the `device` rows, where the frames start / end in HBM.  Evidence for profiles/.
 
-    python scripts/zfile_bench.py [--frames 400] [--coder host|gpu|both] > zfile_bench.jsonl
+    python scripts/zfile_bench.py [--frames 400] [--coder host|gpu|both] [--decoder host|gpu|auto|both] > zfile_bench.jsonl
 
 --coder picks the entropy coder of the method 1/2/3 rows: host zstd at --clevel (the default), the device coder
 (rirb_z_set_coder 1), or both.  With the device coder the first row gives its device time per frame (CUDA events around
 rirb_zstd_encode_batch on method-3 planes larger than L2), next to the card's name and power limit.
+
+--decoder sets the "zstd_decoder" switch around the read rows: host libzstd (0), the device decoder wherever a read ends
+on the device (2), the library's default selection (auto, 1), or all three, run alternately --reps times in the same call
+(each row then reports the best time and all of them).  With the
+device decoder, rows give its device time per frame on 600 frames of 640x512 (output larger than L2) for three inputs:
+device-coder method-3 planes, host zstd level-2 method-3 planes and host zstd level-2 method-1 frames.
 """
 import argparse
 import json
@@ -28,9 +34,13 @@ def main():
     ap.add_argument("--frames", type=int, default=400)
     ap.add_argument("--clevel", type=int, default=2)
     ap.add_argument("--coder", choices=("host", "gpu", "both"), default="host")
+    ap.add_argument("--decoder", choices=("host", "gpu", "auto", "both"), default="auto")
+    ap.add_argument("--reps", type=int, default=3)
     args = ap.parse_args()
     coders = ("host", "gpu") if args.coder == "both" else (args.coder,)
-    from librir_b200 import tools
+    decoders = ("host", "gpu", "auto") if args.decoder == "both" else (args.decoder,)
+    switch = {"host": 0, "auto": 1, "gpu": 2}
+    from librir_b200 import _lib, tools
     from oracle import container as oc  # checker / baseline only
     from tests.conftest import ir_movie
 
@@ -48,8 +58,23 @@ def main():
         rows.append(row)
         print(json.dumps(row), flush=True)
 
+    def timed_reads(name, impl, threads, read, extra=None):
+        """read(): one read of the whole file; alternates the decoders, args.reps times each."""
+        times = {dec: [] for dec in decoders}
+        for _ in range(args.reps):
+            for dec in decoders:
+                _lib.set_parameter("zstd_decoder", switch[dec])
+                t0 = time.perf_counter()
+                read()
+                times[dec].append(time.perf_counter() - t0)
+        _lib.set_parameter("zstd_decoder", 1)
+        for dec in decoders:
+            rec(name, impl, threads, min(times[dec]), dict(extra or {}, decoder=dec, all_seconds=[round(t, 4) for t in times[dec]]))
+
     if "gpu" in coders:
         coder_device_time(mov)
+    if "host" not in decoders or len(decoders) > 1:
+        decoder_device_time(mov)
     have_ref = oc.have_ref()
     if have_ref:
         p = os.path.join(tmp, "ref.bin")
@@ -85,12 +110,14 @@ def main():
                 wr.add_images(d, ts)
             rec("write", "product, frames in HBM", cores, time.perf_counter() - t0)
             out = torch.empty_like(d)
-            t0 = time.perf_counter()
-            with tools.ZFileReader(p, threads=0) as rd:
-                rd.read_images(0, n, out=out)
-            torch.cuda.synchronize()
-            rec("read", "product, frames to HBM", cores, time.perf_counter() - t0)
-            assert torch.equal(out.view(torch.int16), d.view(torch.int16))
+
+            def read_hbm(p=p):
+                with tools.ZFileReader(p, threads=0) as rd:
+                    rd.read_images(0, n, out=out)
+                torch.cuda.synchronize()
+                assert torch.equal(out.view(torch.int16), d.view(torch.int16))
+
+            timed_reads("read", "product, frames to HBM", cores, read_hbm)
             # methods 2 / 3 (video_io.h:298-305): the GPU pre-coder in front of zstd; host frames and frames in HBM
             for method, coder in [(m, c) for c in coders for m in (1, 2, 3)]:
                 for where, src in (("host", mov), ("HBM", d)):
@@ -102,18 +129,19 @@ def main():
                     rec("write", f"product, method {method}, frames in {where}", cores, time.perf_counter() - t0,
                         {"file_MB": round(os.path.getsize(p) / 1e6, 1), "coder": coder,
                          "ratio": round(mov.nbytes / (os.path.getsize(p) - 256), 3)})
-                    t0 = time.perf_counter()
-                    with tools.ZFileReader(p, threads=0) as rd:
+                    def read(p=p, where=where):
+                        with tools.ZFileReader(p, threads=0) as rd:
+                            if where == "host":
+                                back = rd.read_images()
+                            else:
+                                rd.read_images(0, n, out=out)
+                        torch.cuda.synchronize()
                         if where == "host":
-                            back = rd.read_images()
+                            assert np.array_equal(back, mov)
                         else:
-                            rd.read_images(0, n, out=out)
-                    torch.cuda.synchronize()
-                    rec("read", f"product, method {method}, frames to {where}", cores, time.perf_counter() - t0, {"coder": coder})
-                    if where == "host":
-                        assert np.array_equal(back, mov)
-                    else:
-                        assert torch.equal(out.view(torch.int16), d.view(torch.int16))
+                            assert torch.equal(out.view(torch.int16), d.view(torch.int16))
+
+                    timed_reads("read", f"product, method {method}, frames to {where}", cores, read, {"coder": coder})
     except ImportError:
         pass
     for f in os.listdir(tmp):
@@ -162,6 +190,73 @@ def coder_device_time(mov, frames=600, reps=5):
            "us_per_frame": round(1000 * best / frames, 2), "input_GB_per_s": round(src.numel() / best / 1e6, 1),
            "ratio": round(src.numel() / float(sizes.sum()), 3)}
     print(json.dumps(row), flush=True)
+
+
+def card():
+    import subprocess
+
+    try:
+        return subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                              capture_output=True, text=True, timeout=30).stdout.strip().splitlines()[0]
+    except (OSError, IndexError, subprocess.SubprocessError):
+        return "unknown"
+
+
+def decoder_device_time(mov, frames=600, reps=5):
+    """Device time of rirb_zstd_decode_batch per frame over `frames` records of 640x512 (output > L2), CUDA events, best of
+    reps after a warm-up: device-coder method-3 planes, host zstd level-2 method-3 planes, host zstd level-2 method-1."""
+    import torch
+
+    from librir_b200 import _lib
+    from librir_b200 import entropy as E
+    from tests import zcoder_cases as K
+
+    n, h, w = len(mov), mov.shape[1], mov.shape[2]
+    fbytes = 2 * h * w
+    lib = _lib.load()
+    _lib.use_torch_stream()
+    planes = K.planes(mov, 3)
+    dplanes = torch.from_numpy(planes).cuda()
+    stride = 9 + 3 * 2 * ((h * w + 131071) // 131072) + fbytes
+    enc = torch.empty((n, stride), dtype=torch.uint8, device="cuda")
+    sizes = torch.empty(n, dtype=torch.int64, device="cuda")
+    assert lib.rirb_zstd_encode_batch(dplanes.data_ptr(), n, fbytes, h * w, enc.data_ptr(), stride, sizes.data_ptr()) == 0
+    e, sz = enc.cpu().numpy(), sizes.cpu().numpy()
+    inputs = {
+        "device-coder method-3 planes": [e[i, :sz[i]].tobytes() for i in range(n)],
+        "host zstd level-2 method-3 planes": [E.zstd_compress(planes[i], 2) for i in range(n)],
+        "host zstd level-2 method-1 frames": [E.zstd_compress(mov[i].reshape(-1).view(np.uint8), 2) for i in range(n)],
+    }
+    q = card()
+    for name, recs in inputs.items():
+        pick = [recs[i % n] for i in range(frames)]
+        offs = np.cumsum([0] + [len(r) for r in pick[:-1]]).astype(np.int64)
+        src = torch.from_numpy(np.frombuffer(b"".join(pick), np.uint8).copy()).cuda()
+        off = torch.from_numpy(offs).cuda()
+        size = torch.from_numpy(np.array([len(r) for r in pick], np.uint32).view(np.int32)).cuda()
+        dst = torch.empty((frames, fbytes), dtype=torch.uint8, device="cuda")
+        status = torch.empty(frames, dtype=torch.int64, device="cuda")
+
+        def run():
+            assert lib.rirb_zstd_decode_batch(src.data_ptr(), off.data_ptr(), size.data_ptr(), frames, dst.data_ptr(), fbytes,
+                                              fbytes, status.data_ptr()) == 0, _lib.last_error()
+
+        run()
+        torch.cuda.synchronize()
+        assert bool((status == fbytes).all()), name
+        best = None
+        for _ in range(reps):
+            a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            a.record()
+            run()
+            b.record()
+            b.synchronize()
+            best = a.elapsed_time(b) if best is None else min(best, a.elapsed_time(b))
+        row = {"op": "device decoder, " + name, "gpu": torch.cuda.get_device_name(), "nvidia_smi": q, "frames": frames,
+               "frame": [w, h], "input_MB": round(src.numel() / 1e6, 1), "output_MB": round(frames * fbytes / 1e6, 1),
+               "ms_best_of_%d" % reps: round(best, 3), "us_per_frame": round(1000 * best / frames, 2),
+               "output_GB_per_s": round(frames * fbytes / best / 1e6, 1)}
+        print(json.dumps(row), flush=True)
 
 
 if __name__ == "__main__":
