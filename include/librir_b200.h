@@ -293,6 +293,11 @@ RIRB_API int rirb_z_read_images(int handle, int pos, int count, unsigned short* 
  * coder (rirb_zstd_encode_batch; clevel is ignored).  Every record is a standalone zstd frame, so a file may mix them.
  * Returns -1 for an unknown coder, a read handle, or coder 1 without a CUDA device (no CPU fallback). */
 RIRB_API int rirb_z_set_coder(int handle, int coder);
+/* LZ matches in the device coder ("coder 2"): on = 1 makes the records the device coder writes after the call
+ * rirb_zstd_encode_batch_lz's frames, 0 (the default) rirb_zstd_encode_batch's.  It applies while rirb_z_set_coder selects
+ * the device coder (1), for methods 1, 2 and 3.  Returns -1 for a value other than 0 / 1, a read handle, or on = 1 without
+ * a CUDA device. */
+RIRB_API int rirb_z_set_lz(int handle, int on);
 
 /* Device zstd coder: n payloads of bytes_each bytes back to back at src -> one zstd frame each (RFC 8878: Huffman-coded
  * literals, no sequences; RLE / raw blocks where they are smaller), frame i at dst + i * dst_stride, its size in sizes[i].
@@ -301,6 +306,14 @@ RIRB_API int rirb_z_set_coder(int handle, int coder);
  * stream.  dst_stride must be at least 9 + 3 * blocks + bytes_each (the frame when every block is raw). */
 RIRB_API int rirb_zstd_encode_batch(const unsigned char* src, long long n, long long bytes_each, long long segment,
                                     unsigned char* dst, long long dst_stride, long long* sizes);
+
+/* Device zstd coder with LZ matches ("coder 2"): the same arguments and contract as rirb_zstd_encode_batch.  Each block is
+ * coder 1's block, or an LZ form when that is smaller: a greedy parse of matches of at least 8 bytes inside the block
+ * (the latest earlier position with the same 8 bytes), literals coded as coder 1 codes a block, sequences with the
+ * predefined or RLE FSE tables.  A frame where no block takes the LZ form is byte for byte coder 1's frame.  It needs
+ * about 30 bytes of device memory per input byte while it runs. */
+RIRB_API int rirb_zstd_encode_batch_lz(const unsigned char* src, long long n, long long bytes_each, long long segment,
+                                       unsigned char* dst, long long dst_stride, long long* sizes);
 
 /* Device zstd decoder: n zstd frames, frame i at src + offsets[i] (sizes[i] bytes) -> its content at dst + i * dst_stride,
  * at most dst_capacity bytes.  status[i] = bytes written, -1 = malformed frame, -2 = a frame this decoder does not take

@@ -33,8 +33,9 @@ extern "C" {
  * pre-coder in front; "zstd1" / "zstd2" / "zstd3" pick the container method), GOP, threads (host zstd threads, 0 = all),
  * slices (ignored), stdFactor, inputCamera (must stay 0: the camera calibration is outside this library), removeBadPixels,
  * subtractMin, subtractLocalMin (ignored), runningAverage, and this library's entropyCoder ("host": host zstd at
- * compressionLevel, the default; "gpu": the device coder, Huffman-literal zstd frames that any zstd decoder reads; it needs a
- * CUDA device, and applies to the images added after the call); -1 for an unknown key or value.
+ * compressionLevel, the default; "gpu": the device coder, Huffman-literal zstd frames that any zstd decoder reads; "gpu-lz":
+ * the device coder with LZ matches in the blocks where they make the frame smaller; the device coders need a CUDA device,
+ * and the value applies to the images added after the call); -1 for an unknown key or value.
  * h264_add_image_lossy = addImageLossyNoCamera (h264.cpp:2253-2424) in front of the lossless stage, with the
  * BackgroundError / ForegroundError frame attributes and the MIN_T / MIN_T_HEIGHT / Global*Error global ones;
  * h264_add_loss = addLoss (:2426-2607), in place on the caller's image, nothing is stored;

@@ -115,7 +115,9 @@ SIGNATURES = {
     "rirb_z_read_image": (_i, [_i, _i, _vp, _vp]),
     "rirb_z_read_images": (_i, [_i, _i, _i, _vp, _vp, _i]),
     "rirb_z_set_coder": (_i, [_i, _i]),
+    "rirb_z_set_lz": (_i, [_i, _i]),
     "rirb_zstd_encode_batch": (_i, [_vp, _ll, _ll, _ll, _vp, _ll, _vp]),
+    "rirb_zstd_encode_batch_lz": (_i, [_vp, _ll, _ll, _ll, _vp, _ll, _vp]),
     "rirb_zstd_decode_batch": (_i, [_vp, _vp, _vp, _ll, _vp, _ll, _ll, _vp]),
     # Part 4: registration front end
     "rirb_ecc_open": (_i, [_i, _i]),

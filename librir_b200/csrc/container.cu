@@ -522,6 +522,7 @@ struct ZMovie {
     size_t host_bytes = 0, dev_bytes = 0;  // what the two buffers really hold (a pair taken over may be larger than asked)
     // writing with the device coder (coder 1): its scratch, the packed records of a pass on the device and their pinned copy
     int coder = 0;
+    bool lz = false;  // the device coder with LZ matches (rirb_z_set_lz): rirb_zstd_encode_batch_lz's frames
     ZcBuffers zc;
     ~ZMovie()
     {
@@ -887,11 +888,14 @@ static int z_encode_records(ZMovie* z, const u8* src, long long m, long long byt
         zc_unpark(b, dev);
         b.device = dev;
     }
-    if (!z_grow(&b.scratch, &b.scratch_bytes, zcoder_scratch_bytes(m, bytes_each, segment), false) ||
-        !z_grow(&b.dev, &b.dev_bytes, records, false) || !z_grow(&b.host, &b.host_bytes, head + records, true))
+    const bool lz = z->lz;
+    const size_t scratch = lz ? zcoder_lz_scratch_bytes(m, bytes_each, segment) : zcoder_scratch_bytes(m, bytes_each, segment);
+    if (!z_grow(&b.scratch, &b.scratch_bytes, scratch, false) || !z_grow(&b.dev, &b.dev_bytes, records, false) ||
+        !z_grow(&b.host, &b.host_bytes, head + records, true))
         return -1;
     long long* dev_off = nullptr;
-    if (launch_zstd_encode(src, m, bytes_each, segment, (u8*)b.dev, 0, 12, nullptr, &dev_off, b.scratch, st) != 0) return -1;
+    if ((lz ? launch_zstd_encode_lz : launch_zstd_encode)(src, m, bytes_each, segment, (u8*)b.dev, 0, 12, nullptr, &dev_off, b.scratch, st) != 0)
+        return -1;
     long long* off = (long long*)b.host;
     char* rec = b.host + head;
     RIRB_CUDA_OK(cudaMemcpyAsync(off, dev_off, (size_t)(m + 1) * 8, cudaMemcpyDeviceToHost, st));
@@ -1165,6 +1169,26 @@ int rirb_z_set_coder(int handle, int coder)
     }
     std::lock_guard<std::mutex> lock(z->mu);
     z->coder = coder;
+    return 0;
+}
+
+int rirb_z_set_lz(int handle, int on)
+{
+    auto z = g_zfiles.get(handle);
+    if (!z || !z->writing) {
+        set_error("z_set_lz: not a handle open for writing");
+        return -1;
+    }
+    if (on != 0 && on != 1) {
+        set_error("z_set_lz: on must be 0 or 1, not %d", on);
+        return -1;
+    }
+    if (on && rirb_device_count() <= 0) {
+        set_error("z_set_lz: the device coder needs a CUDA device (no CPU fallback)");
+        return -1;
+    }
+    std::lock_guard<std::mutex> lock(z->mu);
+    z->lz = on != 0;
     return 0;
 }
 

@@ -86,6 +86,11 @@ size_t zcoder_scratch_bytes(long long n, long long bytes_each, long long segment
 long long zcoder_frame_bound(long long bytes_each, long long segment);  // the largest frame: raw blocks plus headers
 int launch_zstd_encode(const u8* src, long long n, long long bytes_each, long long segment, u8* dst, long long dst_stride,
                        int rec_head, long long* sizes, long long** frame_offsets, void* scratch, cudaStream_t st);
+// coder 2 (rirb_zstd_encode_batch_lz): the same arguments, coder 1's frame with an LZ form wherever it is smaller; its scratch
+// (zcoder_lz_scratch_bytes) holds coder 1's and a candidate sort of at most 512 blocks at a time (about 1.6 GB)
+size_t zcoder_lz_scratch_bytes(long long n, long long bytes_each, long long segment);
+int launch_zstd_encode_lz(const u8* src, long long n, long long bytes_each, long long segment, u8* dst, long long dst_stride,
+                          int rec_head, long long* sizes, long long** frame_offsets, void* scratch, cudaStream_t st);
 // zdecoder.cu: n zstd frames (frame i at src + offsets[i], sizes[i] bytes) -> content at dst + i * dst_stride, at most cap
 // bytes; status[i] = bytes, -1 malformed, -2 refused (rirb_zstd_decode_batch).  scratch: zdecoder_scratch_bytes(n, cap).
 size_t zdecoder_scratch_bytes(long long n, long long cap);

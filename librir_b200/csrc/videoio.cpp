@@ -125,6 +125,13 @@ std::string frame_attr_string(int (*get)(int, int, int, char*, int*), int handle
 // ---------------------------------------------------------------------------------------------------------------------
 // saver
 // ---------------------------------------------------------------------------------------------------------------------
+// the saver's coder 0 / 1 / 2 on a container handle: the device coder (1) with LZ matches off / on
+static int set_coder(int zfile, int coder)
+{
+    if (rirb_z_set_coder(zfile, coder == 0 ? 0 : 1) != 0) return -1;
+    return coder == 0 ? 0 : rirb_z_set_lz(zfile, coder == 2 ? 1 : 0);
+}
+
 struct Saver {
     std::string filename;
     int w = 0, h = 0, lossy_height = 0;
@@ -134,7 +141,8 @@ struct Saver {
     double std_factor = 5.0;
     std::string codec = "h264";
     int method = 3;  // container method: 3 = delta + byte planes + zstd; "codec" = "zstd1" / "zstd2" / "zstd3" selects it
-    int coder = 0;   // entropy coder of the records: 0 = host zstd, 1 = the device coder ("entropyCoder" = "host" / "gpu")
+    int coder = 0;   // entropy coder of the records: 0 = host zstd, 1 / 2 = the device coder without / with LZ matches
+                     // ("entropyCoder" = "host" / "gpu" / "gpu-lz")
     AttrMap global;
     // open state
     int zfile = 0;        // rirb_z_* handle, 0 until the first image
@@ -156,7 +164,7 @@ struct Saver {
         const int lv = level_of[clevel < 0 ? 0 : (clevel > 8 ? 8 : clevel)];
         zfile = rirb_z_open_file_write_gop(filename.c_str(), w, h, 50, method, lv, gop);  // 50: the fps h264_* hands H264_Saver::open
         if (!zfile) fail(std::string("cannot create the movie file: ") + rirb_last_error());
-        else if (coder != 0 && rirb_z_set_coder(zfile, coder) != 0) fail(std::string("entropyCoder: ") + rirb_last_error());
+        else if (coder != 0 && set_coder(zfile, coder) != 0) fail(std::string("entropyCoder: ") + rirb_last_error());
         return zfile != 0;
     }
     bool open_lossy(int variant)
@@ -503,15 +511,16 @@ int h264_set_parameter(int file, const char* param, const char* value)
     else if (k == "runningAverage") s->running_average = atoi(value) > 64 ? 64 : atoi(value);
     else if (k == "entropyCoder") {
         // "host": zstd on the host threads at compressionLevel (the default); "gpu": the device coder, Huffman-coded zstd frames
-        // that any zstd decoder reads (compressionLevel does not apply).  Applies to the images added after the call.
+        // that any zstd decoder reads (compressionLevel does not apply); "gpu-lz": the device coder with LZ matches in the
+        // blocks where they make the frame smaller.  Applies to the images added after the call.
         const std::string v(value);
-        if (v != "host" && v != "gpu") return -1;
-        const int c = v == "gpu" ? 1 : 0;
-        if (c == 1 && rirb_device_count() <= 0) {
-            fail("h264_set_parameter: entropyCoder gpu needs a CUDA device (no CPU fallback)");
+        if (v != "host" && v != "gpu" && v != "gpu-lz") return -1;
+        const int c = v == "gpu" ? 1 : v == "gpu-lz" ? 2 : 0;
+        if (c != 0 && rirb_device_count() <= 0) {
+            fail("h264_set_parameter: entropyCoder " + v + " needs a CUDA device (no CPU fallback)");
             return -1;
         }
-        if (s->zfile && rirb_z_set_coder(s->zfile, c) != 0) {
+        if (s->zfile && set_coder(s->zfile, c) != 0) {
             fail(std::string("h264_set_parameter: ") + rirb_last_error());
             return -1;
         }

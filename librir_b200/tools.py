@@ -278,15 +278,16 @@ class ZFileWriter:
         """``method`` 1 = zstd of the raw image (the reference's files), 2 = byte planes + zstd, 3 = temporal delta with
         key frames every ``gop`` images + byte planes + zstd (video_io.h:298-305); 2 and 3 pre-code on the GPU.
         ``coder`` "host" = zstd on host threads at ``clevel``; "gpu" = the device coder (Huffman-literal zstd frames that any
-        zstd decoder reads; ``clevel`` does not apply; needs a CUDA device)."""
-        if coder not in ("host", "gpu"):
-            raise ValueError(f"coder must be 'host' or 'gpu', not {coder!r}")
+        zstd decoder reads; ``clevel`` does not apply; needs a CUDA device); "gpu-lz" = the device coder with LZ matches in
+        the blocks where they make the frame smaller (the high-byte planes of methods 2/3 above all)."""
+        if coder not in ("host", "gpu", "gpu-lz"):
+            raise ValueError(f"coder must be 'host', 'gpu' or 'gpu-lz', not {coder!r}")
         lib = _lib.load()
         self.handle = lib.rirb_z_open_file_write_gop(str(filename).encode(), int(width), int(height), int(rate), int(method),
                                                      int(clevel), int(gop))
         if self.handle <= 0:
             raise RuntimeError(f"cannot open '{filename}' for writing: {_lib.last_error()}")
-        if coder == "gpu" and lib.rirb_z_set_coder(self.handle, 1) != 0:
+        if coder != "host" and (lib.rirb_z_set_coder(self.handle, 1) != 0 or lib.rirb_z_set_lz(self.handle, int(coder == "gpu-lz")) != 0):
             err = _lib.last_error()
             lib.rirb_z_close_file(self.handle)
             self.handle = 0

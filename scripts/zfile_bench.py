@@ -4,11 +4,13 @@ thread-pooled container (rirb_z_write_images / rirb_z_read_images) next to the c
 (oracle/_ref, one frame per call on one thread -- what z_write_image / z_read_image do).  Host work; the GPU
 only appears in the `device` rows, where the frames start / end in HBM.  Evidence for profiles/.
 
-    python scripts/zfile_bench.py [--frames 400] [--coder host|gpu|both] [--decoder host|gpu|auto|both] > zfile_bench.jsonl
+    python scripts/zfile_bench.py [--frames 400] [--coder host|gpu|gpu-lz|both|all] [--decoder host|gpu|auto|both] > zfile_bench.jsonl
 
 --coder picks the entropy coder of the method 1/2/3 rows: host zstd at --clevel (the default), the device coder
-(rirb_z_set_coder 1), or both.  With the device coder the first row gives its device time per frame (CUDA events around
-rirb_zstd_encode_batch on method-3 planes larger than L2), next to the card's name and power limit.
+(rirb_z_set_coder 1), the device coder with LZ matches (gpu-lz, rirb_z_set_coder 1 and rirb_z_set_lz 1), host and gpu (both), or all three.
+With a device coder the first rows give its device time per frame (CUDA events around rirb_zstd_encode_batch and, with
+gpu-lz, rirb_zstd_encode_batch_lz, alternated in one call on 600 frames of method-2 and method-3 planes, larger than L2),
+next to the card's name and power limit.
 
 --decoder sets the "zstd_decoder" switch around the read rows: host libzstd (0), the device decoder wherever a read ends
 on the device (2), the library's default selection (auto, 1), or all three, run alternately --reps times in the same call
@@ -33,11 +35,11 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--frames", type=int, default=400)
     ap.add_argument("--clevel", type=int, default=2)
-    ap.add_argument("--coder", choices=("host", "gpu", "both"), default="host")
+    ap.add_argument("--coder", choices=("host", "gpu", "gpu-lz", "both", "all"), default="host")
     ap.add_argument("--decoder", choices=("host", "gpu", "auto", "both"), default="auto")
     ap.add_argument("--reps", type=int, default=3)
     args = ap.parse_args()
-    coders = ("host", "gpu") if args.coder == "both" else (args.coder,)
+    coders = {"both": ("host", "gpu"), "all": ("host", "gpu", "gpu-lz")}.get(args.coder, (args.coder,))
     decoders = ("host", "gpu", "auto") if args.decoder == "both" else (args.decoder,)
     switch = {"host": 0, "auto": 1, "gpu": 2}
     from librir_b200 import _lib, tools
@@ -71,8 +73,8 @@ def main():
         for dec in decoders:
             rec(name, impl, threads, min(times[dec]), dict(extra or {}, decoder=dec, all_seconds=[round(t, 4) for t in times[dec]]))
 
-    if "gpu" in coders:
-        coder_device_time(mov)
+    if "gpu" in coders or "gpu-lz" in coders:
+        coder_device_time(mov, ("gpu", "gpu-lz") if "gpu-lz" in coders else ("gpu",))
     if "host" not in decoders or len(decoders) > 1:
         decoder_device_time(mov)
     have_ref = oc.have_ref()
@@ -149,47 +151,51 @@ def main():
     os.rmdir(tmp)
 
 
-def coder_device_time(mov, frames=600, reps=5):
-    """Device time of rirb_zstd_encode_batch per frame: method-3 planes of `frames` frames (> L2), CUDA events, best of reps."""
-    import subprocess
-
+def coder_device_time(mov, coders, frames=600, reps=5):
+    """Device time per frame of the device coders (gpu: rirb_zstd_encode_batch, gpu-lz: rirb_zstd_encode_batch_lz) on the
+    method-2 and method-3 planes of `frames` frames (> L2): CUDA events, the coders alternated, best of reps each."""
     import torch
 
     from librir_b200 import _lib
     from tests import zcoder_cases as K
 
     n, h, w = len(mov), mov.shape[1], mov.shape[2]
-    planes = torch.from_numpy(K.planes(mov, 3)).cuda()
-    src = planes[torch.arange(frames) % n].contiguous()  # [frames, 2*h*w]
     stride = 9 + 3 * 2 * ((h * w + 131071) // 131072) + 2 * h * w
     dst = torch.empty((frames, stride), dtype=torch.uint8, device="cuda")
     sizes = torch.empty(frames, dtype=torch.int64, device="cuda")
     _lib.use_torch_stream()
     lib = _lib.load()
+    entry = {"gpu": lib.rirb_zstd_encode_batch, "gpu-lz": lib.rirb_zstd_encode_batch_lz}
+    q = card()
+    for method in (2, 3):
+        planes = torch.from_numpy(K.planes(mov, method)).cuda()
+        src = planes[torch.arange(frames) % n].contiguous()  # [frames, 2*h*w]
 
-    def run():
-        assert lib.rirb_zstd_encode_batch(src.data_ptr(), frames, 2 * h * w, h * w, dst.data_ptr(), stride, sizes.data_ptr()) == 0, _lib.last_error()
+        def run(coder):
+            assert entry[coder](src.data_ptr(), frames, 2 * h * w, h * w, dst.data_ptr(), stride, sizes.data_ptr()) == 0, _lib.last_error()
 
-    run()
-    torch.cuda.synchronize()
-    best = None
-    for _ in range(reps):
-        a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        a.record()
-        run()
-        b.record()
-        b.synchronize()
-        best = a.elapsed_time(b) if best is None else min(best, a.elapsed_time(b))
-    try:
-        q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
-                           capture_output=True, text=True, timeout=30).stdout.strip().splitlines()[0]
-    except (OSError, IndexError, subprocess.SubprocessError):
-        q = "unknown"
-    row = {"op": "device coder, method-3 planes", "gpu": torch.cuda.get_device_name(), "nvidia_smi": q, "frames": frames,
-           "frame": [w, h], "input_MB": round(src.numel() / 1e6, 1), "ms_best_of_%d" % reps: round(best, 3),
-           "us_per_frame": round(1000 * best / frames, 2), "input_GB_per_s": round(src.numel() / best / 1e6, 1),
-           "ratio": round(src.numel() / float(sizes.sum()), 3)}
-    print(json.dumps(row), flush=True)
+        ratio = {}
+        for coder in coders:
+            run(coder)
+            torch.cuda.synchronize()
+            ratio[coder] = src.numel() / float(sizes.sum())
+        best = {}
+        for _ in range(reps):
+            for coder in coders:
+                a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                a.record()
+                run(coder)
+                b.record()
+                b.synchronize()
+                best[coder] = min(best.get(coder, 1e30), a.elapsed_time(b))
+        for coder in coders:
+            row = {"op": f"device coder, method-{method} planes", "coder": coder, "gpu": torch.cuda.get_device_name(),
+                   "nvidia_smi": q, "frames": frames, "frame": [w, h], "input_MB": round(src.numel() / 1e6, 1),
+                   "ms_best_of_%d" % reps: round(best[coder], 3), "us_per_frame": round(1000 * best[coder] / frames, 2),
+                   "input_GB_per_s": round(src.numel() / best[coder] / 1e6, 1), "ratio": round(ratio[coder], 3)}
+            print(json.dumps(row), flush=True)
+        del planes, src
+        torch.cuda.empty_cache()
 
 
 def card():
