@@ -221,6 +221,8 @@ __global__ void delta_merge_scalar_kernel(const u8* __restrict__ lo, const u8* _
     }
 }
 
+constexpr long long MAX_GOPS_PER_LAUNCH = 65535;  // the delta kernels put the GOP index in gridDim.y
+
 static bool movie_vectorizable(const void* mov, const void* lo, const void* hi, size_t npx)
 {
     return (npx % 16 == 0) && aligned32(mov) && aligned16(lo) && aligned16(hi);
@@ -328,18 +330,22 @@ int launch_precode_movie(const u16* mov, long long nframes, int w, int h, int go
         set_error("precode: with delta on, a shard must start on a key frame (first_frame %lld, GOP %d)", first_frame, gop);
         return -1;
     }
-    const long long ngop = ceil_div(nframes, gop);
-    if (ngop > 65535) {
-        set_error("precode: too many GOPs in one call (%lld)", ngop);
-        return -1;
-    }
-    if (movie_vectorizable(mov, lo, hi, npx)) {
-        const size_t vpf = npx / 16;
-        dim3 grid((unsigned)ceil_div((long long)vpf, PC_THREADS), (unsigned)ngop);
-        RIRB_LAUNCH(delta_split_kernel, grid, PC_THREADS, 0, st, mov, lo, hi, vpf, nframes, gop);
-    } else {
-        dim3 grid((unsigned)ceil_div((long long)npx, 256), (unsigned)ngop);
-        RIRB_LAUNCH(delta_split_scalar_kernel, grid, 256, 0, st, mov, lo, hi, npx, nframes, gop);
+    // grid = (pixel block, GOP); gridDim.y <= 65535, so long movies go in several launches of whole GOPs (whole frames
+    // keep the vector alignment, as npx % 16 == 0 on that path) -- the fused split_stats_kernel has no such limit
+    const bool vec = movie_vectorizable(mov, lo, hi, npx);
+    const long long span = (long long)MAX_GOPS_PER_LAUNCH * gop;
+    for (long long f0 = 0; f0 < nframes; f0 += span) {
+        const long long n = min(nframes - f0, span);
+        const size_t off = (size_t)f0 * npx;
+        const unsigned ngop = (unsigned)ceil_div(n, gop);
+        if (vec) {
+            const size_t vpf = npx / 16;
+            dim3 grid((unsigned)ceil_div((long long)vpf, PC_THREADS), ngop);
+            RIRB_LAUNCH(delta_split_kernel, grid, PC_THREADS, 0, st, mov + off, lo + off, hi + off, vpf, n, gop);
+        } else {
+            dim3 grid((unsigned)ceil_div((long long)npx, 256), ngop);
+            RIRB_LAUNCH(delta_split_scalar_kernel, grid, 256, 0, st, mov + off, lo + off, hi + off, npx, n, gop);
+        }
     }
     return 0;
 }
@@ -367,18 +373,20 @@ int launch_decode_movie(const u8* lo, const u8* hi, long long nframes, int w, in
         set_error("decode: with delta on, a shard must start on a key frame (first_frame %lld, GOP %d)", first_frame, gop);
         return -1;
     }
-    const long long ngop = ceil_div(nframes, gop);
-    if (ngop > 65535) {
-        set_error("decode: too many GOPs in one call (%lld)", ngop);
-        return -1;
-    }
-    if (movie_vectorizable(mov, lo, hi, npx)) {
-        const size_t vpf = npx / 16;
-        dim3 grid((unsigned)ceil_div((long long)vpf, PC_THREADS), (unsigned)ngop);
-        RIRB_LAUNCH(delta_merge_kernel, grid, PC_THREADS, 0, st, lo, hi, mov, vpf, nframes, gop);
-    } else {
-        dim3 grid((unsigned)ceil_div((long long)npx, 256), (unsigned)ngop);
-        RIRB_LAUNCH(delta_merge_scalar_kernel, grid, 256, 0, st, lo, hi, mov, npx, nframes, gop);
+    const bool vec = movie_vectorizable(mov, lo, hi, npx);
+    const long long span = (long long)MAX_GOPS_PER_LAUNCH * gop;  // as in launch_precode_movie
+    for (long long f0 = 0; f0 < nframes; f0 += span) {
+        const long long n = min(nframes - f0, span);
+        const size_t off = (size_t)f0 * npx;
+        const unsigned ngop = (unsigned)ceil_div(n, gop);
+        if (vec) {
+            const size_t vpf = npx / 16;
+            dim3 grid((unsigned)ceil_div((long long)vpf, PC_THREADS), ngop);
+            RIRB_LAUNCH(delta_merge_kernel, grid, PC_THREADS, 0, st, lo + off, hi + off, mov + off, vpf, n, gop);
+        } else {
+            dim3 grid((unsigned)ceil_div((long long)npx, 256), ngop);
+            RIRB_LAUNCH(delta_merge_scalar_kernel, grid, 256, 0, st, lo + off, hi + off, mov + off, npx, n, gop);
+        }
     }
     return 0;
 }
