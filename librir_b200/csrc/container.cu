@@ -420,78 +420,63 @@ static size_t z_decompress(void* dctx, void* dst, size_t cap, const void* src, s
     return dctx ? zstd().decompressDCtx(dctx, dst, cap, src, n) : zstd().decompress(dst, cap, src, n);
 }
 
-// Work space of the pre-coded methods (a pinned plane buffer + a device buffer, ~64 MB of frames each way).  Pinning and
-// unpinning cost 10-800 ms a time on the measured host (a VM), more than reading a 400-frame file, so a closed file PARKS
-// its pair here and the next file of the process takes it over; one pair is kept, a second one is freed.
-static std::mutex g_park_mu;
-static char* g_park_host = nullptr;
-static char* g_park_dev = nullptr;
-static size_t g_park_host_bytes = 0, g_park_dev_bytes = 0;
-static int g_park_device = -1;
-static void z_park_buffers(char* host, size_t host_bytes, char* dev, size_t dev_bytes, int device)
-{
-    if (!host && !dev) return;
+// A grow-only buffer in device memory or pinned host memory.
+struct ZBuf {
+    bool pinned;
+    char* p = nullptr;
+    size_t bytes = 0;
+    explicit ZBuf(bool pin) : pinned(pin) {}
+    // false + set_error when memory runs out
+    bool grow(size_t need)
     {
-        std::lock_guard<std::mutex> lock(g_park_mu);
-        if (host && dev && host_bytes + dev_bytes > g_park_host_bytes + g_park_dev_bytes) {
-            std::swap(host, g_park_host);
-            std::swap(dev, g_park_dev);
-            g_park_host_bytes = host_bytes;
-            g_park_dev_bytes = dev_bytes;
-            g_park_device = device;
+        if (bytes >= need) return true;
+        release();
+        if ((pinned ? cudaMallocHost((void**)&p, need) : cudaMalloc((void**)&p, need)) != cudaSuccess) {
+            cudaGetLastError();
+            p = nullptr;
+            set_error("zstd movie file: out of %s memory (%zu bytes)", pinned ? "pinned host" : "device", need);
+            return false;
         }
+        bytes = need;
+        return true;
     }
-    if (host) (void)cudaFreeHost(host);
-    if (dev) (void)cudaFree(dev);
-    (void)cudaGetLastError();
-}
-static bool z_unpark_buffers(size_t host_bytes, size_t dev_bytes, int device, char** host, size_t* host_has, char** dev, size_t* dev_has)
-{
-    std::lock_guard<std::mutex> lock(g_park_mu);
-    if (!g_park_host || g_park_device != device || g_park_host_bytes < host_bytes || g_park_dev_bytes < dev_bytes) return false;
-    *host = g_park_host;
-    *dev = g_park_dev;
-    *host_has = g_park_host_bytes;
-    *dev_has = g_park_dev_bytes;
-    g_park_host = g_park_dev = nullptr;
-    g_park_host_bytes = g_park_dev_bytes = 0;
-    return true;
-}
-
-// The device coder's buffers: its scratch, the packed records of a pass on the device and their pinned copy.  Parked like the
-// pair above when a file closes (pinning is the expensive part), so that the next file of the process starts warm.
-struct ZcBuffers {
-    char* scratch = nullptr;
-    char* dev = nullptr;
-    char* host = nullptr;
-    size_t scratch_bytes = 0, dev_bytes = 0, host_bytes = 0;
-    int device = -1;
-};
-static std::mutex g_zc_mu;
-static ZcBuffers g_zc_parked;
-static void zc_free(ZcBuffers& b)
-{
-    if (b.scratch) cudaFree(b.scratch);
-    if (b.dev) cudaFree(b.dev);
-    if (b.host) cudaFreeHost(b.host);
-    (void)cudaGetLastError();
-    b = ZcBuffers();
-}
-static void zc_park(ZcBuffers& b)
-{
-    if (!b.scratch && !b.dev && !b.host) return;
+    void release()
     {
-        std::lock_guard<std::mutex> lock(g_zc_mu);
-        std::swap(b, g_zc_parked);  // the newer set is kept, the older one freed
+        if (p) (void)(pinned ? cudaFreeHost(p) : cudaFree(p));
+        p = nullptr;
+        bytes = 0;
     }
-    zc_free(b);
-}
-static void zc_unpark(ZcBuffers& b, int device)
+};
+
+// Every work buffer of an open file, all on one device: the pinned planes of methods 2 / 3 ([frame][lo plane | hi plane]), the
+// device frames | lo planes | hi planes of a pass, the device coder's or decoder's scratch, and a pass's records on the device
+// and their pinned copy.
+struct ZBuffers {
+    ZBuf host_planes{true}, frames{false}, scratch{false}, records{false}, host_records{true};
+    int device = -1;
+    bool empty() const { return !host_planes.p && !frames.p && !scratch.p && !records.p && !host_records.p; }
+    void release()
+    {
+        for (ZBuf* b : {&host_planes, &frames, &scratch, &records, &host_records}) b->release();
+        (void)cudaGetLastError();
+        device = -1;
+    }
+};
+
+// Pinning and unpinning cost 10-800 ms a time on the measured host (a VM), more than reading a 400-frame file, so a closed file
+// PARKS its buffers here and the next file of the process that needs buffers on that device takes them over.  One set is kept,
+// the newer: files opened one after another then hand on one set that has grown to what each of them needed, and of two files
+// open at once the one closed last is the likelier to resemble the next.  The older set is freed.
+static std::mutex g_parked_mu;
+static ZBuffers g_parked;
+static void z_park(ZBuffers& b)
 {
-    std::lock_guard<std::mutex> lock(g_zc_mu);
-    if (g_zc_parked.device != device) return;
-    b = g_zc_parked;
-    g_zc_parked = ZcBuffers();
+    if (b.empty()) return;
+    {
+        std::lock_guard<std::mutex> lock(g_parked_mu);
+        std::swap(b, g_parked);
+    }
+    b.release();
 }
 
 struct ZMovie {
@@ -512,61 +497,43 @@ struct ZMovie {
     int gop = 50;
     std::vector<u16> pending;            // writing: frames that do not fill a GOP yet (host)
     std::vector<int64_t> pending_times;
-    char* host_planes = nullptr;         // pinned: [frame][lo plane | hi plane]
-    size_t host_planes_frames = 0;
-    char* dev_buf = nullptr;             // device: frames | lo planes | hi planes for dev_frames frames
-    size_t dev_frames = 0;
-    int dev_device = -1;
-    long long cache_first = -1, cache_count = 0;  // reading: decoded frames [cache_first, +cache_count) still in dev_buf
+    ZBuffers buf;                        // use through buffers()
+    size_t dev_frames = 0;               // the frames | lo planes | hi planes layout of buf.frames is for this many frames
+    long long cache_first = -1, cache_count = 0;  // reading: decoded frames [cache_first, +cache_count) still in buf.frames
     std::mutex mu;
-    size_t host_bytes = 0, dev_bytes = 0;  // what the two buffers really hold (a pair taken over may be larger than asked)
-    // writing with the device coder (coder 1): its scratch, the packed records of a pass on the device and their pinned copy
+    // writing with the device coder (coder 1)
     int coder = 0;
     bool lz = false;  // the device coder with LZ matches (rirb_z_set_lz): rirb_zstd_encode_batch_lz's frames
-    ZcBuffers zc;
     ~ZMovie()
     {
         if (f) fclose(f);
-        z_park_buffers(host_planes, host_bytes, dev_buf, dev_bytes, dev_device);
-        zc_park(zc);
+        z_park(buf);
     }
-    // grow-only work space for m frames; false + set_error when memory runs out
+    // the work buffers on the current device: a change of device frees them and takes over a set parked on the new one
+    ZBuffers& buffers()
+    {
+        int dev = 0;
+        cudaGetDevice(&dev);
+        if (buf.device != dev) {
+            buf.release();
+            cache_first = -1;
+            std::lock_guard<std::mutex> lock(g_parked_mu);
+            if (g_parked.device == dev) std::swap(buf, g_parked);
+            buf.device = dev;
+        }
+        return buf;
+    }
+    // frames and planes for m frames; false + set_error when memory runs out
     bool reserve(size_t m)
     {
         const size_t npx = (size_t)w * h;
-        int dev = 0;
-        cudaGetDevice(&dev);
-        if (m <= dev_frames && m <= host_planes_frames && dev == dev_device) return true;
-        // both at once, so that the pair a closed file parked can be taken over as it is
-        m = std::max(m, std::max(dev_frames, host_planes_frames));
-        z_park_buffers(host_planes, host_bytes, dev_buf, dev_bytes, dev_device);
-        host_planes = dev_buf = nullptr;
-        host_planes_frames = dev_frames = 0;
-        host_bytes = dev_bytes = 0;
-        cache_first = -1;
-        if (!z_unpark_buffers(m * npx * 2, m * npx * 4, dev, &host_planes, &host_bytes, &dev_buf, &dev_bytes)) {
-            if (cudaMalloc((void**)&dev_buf, m * npx * 4) != cudaSuccess) {
-                cudaGetLastError();
-                dev_buf = nullptr;
-                set_error("zstd movie file: out of device memory for %zu frames", m);
-                return false;
-            }
-            if (cudaMallocHost((void**)&host_planes, m * npx * 2) != cudaSuccess) {
-                cudaGetLastError();
-                cudaFree(dev_buf);
-                host_planes = dev_buf = nullptr;
-                set_error("zstd movie file: out of pinned host memory for %zu frames", m);
-                return false;
-            }
-            host_bytes = m * npx * 2;
-            dev_bytes = m * npx * 4;
-        }
-        dev_frames = host_planes_frames = m;
-        dev_device = dev;
-        return true;
+        ZBuffers& b = buffers();
+        dev_frames = std::max(dev_frames, m);  // the layout only grows
+        return b.frames.grow(dev_frames * npx * 4) && b.host_planes.grow(dev_frames * npx * 2);
     }
-    u16* dev_movie() const { return (u16*)dev_buf; }
-    u8* dev_lo() const { return (u8*)dev_buf + dev_frames * (size_t)w * h * 2; }
+    char* host_planes() const { return buf.host_planes.p; }
+    u16* dev_movie() const { return (u16*)buf.frames.p; }
+    u8* dev_lo() const { return (u8*)buf.frames.p + dev_frames * (size_t)w * h * 2; }
     u8* dev_hi() const { return dev_lo() + dev_frames * (size_t)w * h; }
 };
 static Table<ZMovie> g_zfiles;
@@ -625,6 +592,54 @@ static bool device_pointer(const void* p)
         return false;
     }
     return a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged;
+}
+
+// all n bytes at file offset `at` (one pread / pwrite may move fewer); false on an error or the end of the file
+static bool pread_all(int fd, void* p, size_t n, long long at)
+{
+    for (size_t done = 0; done < n;) {
+        const ssize_t r = pread(fd, (char*)p + done, n - done, (off_t)(at + (long long)done));
+        if (r <= 0) return false;
+        done += (size_t)r;
+    }
+    return true;
+}
+static bool pwrite_all(int fd, const void* p, size_t n, long long at)
+{
+    for (size_t done = 0; done < n;) {
+        const ssize_t r = pwrite(fd, (const char*)p + done, n - done, (off_t)(at + (long long)done));
+        if (r <= 0) return false;
+        done += (size_t)r;
+    }
+    return true;
+}
+
+// frames in one pass of the GPU paths: about 64 MB of pixels, in whole GOPs of `gop` frames
+static long long z_pass_frames(const ZMovie* z, long long gop)
+{
+    const long long chunk = std::max<long long>(1, (64ll << 20) / ((long long)z->w * z->h * 2));
+    return std::max(gop, chunk / gop * gop);
+}
+
+// m frames' planes from dev_lo / dev_hi into `planes`, per frame [lo | hi], so that a record's payload is one contiguous run
+static cudaError_t interleave_planes(const ZMovie* z, void* planes, long long m, cudaMemcpyKind kind, cudaStream_t st)
+{
+    const size_t npx = (size_t)z->w * z->h;
+    const cudaError_t e = cudaMemcpy2DAsync(planes, 2 * npx, z->dev_lo(), npx, npx, (size_t)m, kind, st);
+    return e == cudaSuccess ? cudaMemcpy2DAsync((char*)planes + npx, 2 * npx, z->dev_hi(), npx, npx, (size_t)m, kind, st) : e;
+}
+// the other way: per frame [lo | hi] at `planes` apart into dev_lo / dev_hi
+static cudaError_t split_planes(const ZMovie* z, const void* planes, long long m, cudaMemcpyKind kind, cudaStream_t st)
+{
+    const size_t npx = (size_t)z->w * z->h;
+    const cudaError_t e = cudaMemcpy2DAsync(z->dev_lo(), npx, planes, 2 * npx, npx, (size_t)m, kind, st);
+    return e == cudaSuccess ? cudaMemcpy2DAsync(z->dev_hi(), npx, (const char*)planes + npx, 2 * npx, npx, (size_t)m, kind, st) : e;
+}
+
+static int z_unreadable(const ZMovie* z)
+{
+    set_error("z_read_images: a record cannot be read or does not decompress to a %d x %d image", z->w, z->h);
+    return -1;
 }
 
 }  // namespace rirb
@@ -836,101 +851,72 @@ int rirb_z_open_file_write_gop(const char* filename, int width, int height, int 
     return g_zfiles.add(z);
 }
 
-static int z_write_records(ZMovie* z, const void* frames, long long nframes, const long long* timestamps, int threads);
-static int z_read_records(ZMovie* z, int pos, int count, void* out, long long* timestamps, int threads, bool to_pinned_planes);
-static int z_read_precoded(ZMovie* z, int pos, int count, unsigned short* out, int threads);
-static int z_read_records_device(ZMovie* z, int pos, int count, u8* out, int threads);
-static int z_write_precoded(ZMovie* z, const unsigned short* frames, long long nframes, const long long* timestamps, int threads);
-
-// frames[nframes][h][w] host or device; timestamps host.  Records are appended in order; the frames
-// are compressed `threads` at a time (0: all host cores).
-int rirb_z_write_images(int handle, const unsigned short* frames, long long nframes, const long long* timestamps, int threads)
+// Appends m records (i64 timestamp, u32 size, payload) at z->pos and adds them to the index.  Record i is 12 + sizes[i] bytes at
+// rec[i], its payload from rec[i] + 12 on; the heads are written here.  Records that follow one another in memory go out in one
+// pwrite (the device coder's packed pass), the others one each, `workers` at a time.
+static int z_append_records(ZMovie* z, char* const* rec, const size_t* sizes, const long long* timestamps, long long m, int workers)
 {
-    auto z = g_zfiles.get(handle);
-    if (!z || !z->writing || !frames || nframes < 0 || (nframes > 0 && !timestamps)) {
-        set_error("z_write_images: bad handle or arguments");
+    std::vector<long long> at((size_t)m + 1, z->pos);  // where each record goes, then the end
+    std::vector<long long> runs;                        // the first record of each run that is contiguous in memory, then m
+    for (long long i = 0; i < m; ++i) {
+        const int64_t ts = timestamps[i];
+        const uint32_t c32 = (uint32_t)sizes[i];
+        memcpy(rec[i], &ts, 8);
+        memcpy(rec[i] + 8, &c32, 4);
+        at[i + 1] = at[i] + 12 + (long long)sizes[i];
+        if (i == 0 || rec[i] != rec[i - 1] + 12 + sizes[i - 1]) runs.push_back(i);
+    }
+    runs.push_back(m);
+    const int fd = fileno(z->f);
+    std::atomic<bool> failed{false};
+    parallel_for((long long)runs.size() - 1, workers, [&](long long r, int) {
+        const long long i = runs[r], j = runs[r + 1];
+        if (!pwrite_all(fd, rec[i], (size_t)(at[j] - at[i]), at[i])) failed = true;
+    });
+    if (failed) {
+        set_error("z_write_images: write failed");
         return -1;
     }
-    if (nframes == 0) return 0;
-    std::lock_guard<std::mutex> lock(z->mu);
-    return z->method == 1 ? z_write_records(z.get(), frames, nframes, timestamps, threads)
-                          : z_write_precoded(z.get(), frames, nframes, timestamps, threads);
+    z->times.insert(z->times.end(), timestamps, timestamps + m);
+    z->positions.insert(z->positions.end(), at.begin(), at.end() - 1);
+    z->pos = at[m];
+    return 0;
 }
 
-// grow-only buffers of the device coder; false + set_error when memory runs out
-static bool z_grow(char** p, size_t* have, size_t need, bool pinned)
-{
-    if (*have >= need) return true;
-    if (*p) (void)(pinned ? cudaFreeHost(*p) : cudaFree(*p));
-    *p = nullptr;
-    *have = 0;
-    if ((pinned ? cudaMallocHost((void**)p, need) : cudaMalloc((void**)p, need)) != cudaSuccess) {
-        cudaGetLastError();
-        *p = nullptr;
-        set_error("zstd movie file: out of %s memory for the device zstd buffers (%zu bytes)", pinned ? "pinned host" : "device", need);
-        return false;
-    }
-    *have = need;
-    return true;
-}
-
-// m payloads of bytes_each bytes on the DEVICE -> device coder -> records packed back to back -> host -> one pwrite
+// m payloads of bytes_each bytes on the DEVICE -> device coder -> records packed back to back -> host -> file
 static int z_encode_records(ZMovie* z, const u8* src, long long m, long long bytes_each, long long segment, const long long* timestamps)
 {
     cudaStream_t st = current_stream();
     const size_t records = (size_t)m * (size_t)(12 + zcoder_frame_bound(bytes_each, segment));
     const size_t head = ((size_t)(m + 1) * 8 + 63) & ~(size_t)63;  // pinned: the record offsets, then the records
-    ZcBuffers& b = z->zc;
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (b.device != dev) {
-        zc_free(b);
-        zc_unpark(b, dev);
-        b.device = dev;
-    }
+    ZBuffers& b = z->buffers();
     const bool lz = z->lz;
     const size_t scratch = lz ? zcoder_lz_scratch_bytes(m, bytes_each, segment) : zcoder_scratch_bytes(m, bytes_each, segment);
-    if (!z_grow(&b.scratch, &b.scratch_bytes, scratch, false) || !z_grow(&b.dev, &b.dev_bytes, records, false) ||
-        !z_grow(&b.host, &b.host_bytes, head + records, true))
-        return -1;
+    if (!b.scratch.grow(scratch) || !b.records.grow(records) || !b.host_records.grow(head + records)) return -1;
     long long* dev_off = nullptr;
-    if ((lz ? launch_zstd_encode_lz : launch_zstd_encode)(src, m, bytes_each, segment, (u8*)b.dev, 0, 12, nullptr, &dev_off, b.scratch, st) != 0)
+    if ((lz ? launch_zstd_encode_lz : launch_zstd_encode)(src, m, bytes_each, segment, (u8*)b.records.p, 0, 12, nullptr, &dev_off,
+                                                          b.scratch.p, st) != 0)
         return -1;
-    long long* off = (long long*)b.host;
-    char* rec = b.host + head;
+    long long* off = (long long*)b.host_records.p;
+    char* rec = b.host_records.p + head;
     RIRB_CUDA_OK(cudaMemcpyAsync(off, dev_off, (size_t)(m + 1) * 8, cudaMemcpyDeviceToHost, st));
     RIRB_CUDA_OK(cudaStreamSynchronize(st));
-    const long long total = off[m];
-    RIRB_CUDA_OK(cudaMemcpyAsync(rec, b.dev, (size_t)total, cudaMemcpyDeviceToHost, st));
+    RIRB_CUDA_OK(cudaMemcpyAsync(rec, b.records.p, (size_t)off[m], cudaMemcpyDeviceToHost, st));
     RIRB_CUDA_OK(cudaStreamSynchronize(st));
-    for (long long i = 0; i < m; ++i) {  // record = i64 timestamp, u32 size, payload
-        const int64_t ts = timestamps[i];
-        const uint32_t c32 = (uint32_t)((i + 1 < m ? off[i + 1] : total) - off[i] - 12);
-        memcpy(rec + off[i], &ts, 8);
-        memcpy(rec + off[i] + 8, &c32, 4);
-    }
-    const int fd = fileno(z->f);
-    for (long long done = 0; done < total;) {
-        const ssize_t w = pwrite(fd, rec + done, (size_t)(total - done), (off_t)(z->pos + done));
-        if (w <= 0) {
-            set_error("z_write_images: write failed");
-            return -1;
-        }
-        done += w;
-    }
+    std::vector<char*> recs((size_t)m);
+    std::vector<size_t> sizes((size_t)m);
     for (long long i = 0; i < m; ++i) {
-        z->times.push_back(timestamps[i]);
-        z->positions.push_back(z->pos + off[i]);
+        recs[i] = rec + off[i];
+        sizes[i] = (size_t)(off[i + 1] - off[i] - 12);
     }
-    z->pos += total;
-    return 0;
+    return z_append_records(z, recs.data(), sizes.data(), timestamps, m, 1);
 }
 
 // method 1 with the device coder: device frames are encoded where they are, host frames go up in passes of ~64 MB
 static int z_write_records_device(ZMovie* z, const void* frames, long long nframes, const long long* timestamps)
 {
     const size_t fbytes = (size_t)z->w * z->h * 2;
-    const long long chunk = std::max<long long>(1, (64ll << 20) / (long long)fbytes);
+    const long long chunk = z_pass_frames(z, 1);
     const bool on_device = device_pointer(frames);
     cudaStream_t st = current_stream();
     for (long long done = 0; done < nframes;) {
@@ -959,8 +945,8 @@ static int z_write_records(ZMovie* z, const void* frames, long long nframes, con
     const long long batch = std::min<long long>(nframes, std::max<long long>(2LL * workers, 8));
     auto& out = z->slots;
     while ((long long)out.size() < batch) out.emplace_back(new char[bound + 12]);
-    std::vector<long long> at((size_t)batch);
-    const int fd = fileno(z->f);
+    std::vector<char*> rec((size_t)batch);
+    for (long long i = 0; i < batch; ++i) rec[i] = out[i].get();
     std::vector<size_t> csize((size_t)batch);
     if (!z->ctx || (int)z->ctx->c.size() < workers) z->ctx.reset(new Contexts(workers, true));
     Contexts& ctx = *z->ctx;
@@ -990,7 +976,7 @@ static int z_write_records(ZMovie* z, const void* frames, long long nframes, con
         }
         std::atomic<bool> failed{false};
         parallel_for(m, workers, [&](long long i, int t) {
-            const size_t c = z_compress(ctx.get(t), out[i].get() + 12, bound, src + (size_t)i * fbytes, fbytes, z->clevel);
+            const size_t c = z_compress(ctx.get(t), rec[i] + 12, bound, src + (size_t)i * fbytes, fbytes, z->clevel);
             if (zstd().isError(c)) failed = true;
             csize[i] = c;
         });
@@ -998,37 +984,7 @@ static int z_write_records(ZMovie* z, const void* frames, long long nframes, con
             set_error("z_write_images: zstd failed");
             return -1;
         }
-        // record = i64 timestamp, u32 size, payload; positions are a prefix sum, so the workers can write their own
-        long long pos = z->pos;
-        for (long long i = 0; i < m; ++i) {
-            const int64_t ts = timestamps[b0 + i];
-            const uint32_t c32 = (uint32_t)csize[i];
-            memcpy(out[i].get(), &ts, 8);
-            memcpy(out[i].get() + 8, &c32, 4);
-            at[i] = pos;
-            pos += 12 + (long long)csize[i];
-        }
-        parallel_for(m, workers, [&](long long i, int) {
-            const size_t len = 12 + csize[i];
-            size_t done = 0;
-            while (done < len) {
-                const ssize_t w = pwrite(fd, out[i].get() + done, len - done, (off_t)(at[i] + (long long)done));
-                if (w <= 0) {
-                    failed = true;
-                    return;
-                }
-                done += (size_t)w;
-            }
-        });
-        if (failed) {
-            set_error("z_write_images: write failed");
-            return -1;
-        }
-        for (long long i = 0; i < m; ++i) {
-            z->times.push_back(timestamps[b0 + i]);
-            z->positions.push_back(at[i]);
-        }
-        z->pos = pos;
+        if (z_append_records(z, rec.data(), csize.data(), timestamps + b0, m, workers) != 0) return -1;
     }
     return 0;
 }
@@ -1053,34 +1009,52 @@ struct ZPhase {
 // m frames on the DEVICE, the first of them a key frame (frame number `first`): pre-coder -> pinned planes -> zstd -> records
 static int z_flush_gops(ZMovie* z, const u16* dev_frames, long long m, long long first, const long long* timestamps, int threads)
 {
-    const size_t npx = (size_t)z->w * z->h;
     cudaStream_t st = current_stream();
     ZPhase ph;
     if (rirb_precode_movie(dev_frames, m, z->w, z->h, z->gop, z->method == 3, first, z->dev_lo(), z->dev_hi()) != 0) return -1;
     if (z->coder == 1) {
-        // per frame [lo | hi] into the frames' part of dev_buf (the pre-coder has read them by now, in stream order)
+        // into the frames' part of the device buffer (the pre-coder has read them by now, in stream order)
         u8* planes = (u8*)z->dev_movie();
-        RIRB_CUDA_OK(cudaMemcpy2DAsync(planes, 2 * npx, z->dev_lo(), npx, npx, (size_t)m, cudaMemcpyDeviceToDevice, st));
-        RIRB_CUDA_OK(cudaMemcpy2DAsync(planes + npx, 2 * npx, z->dev_hi(), npx, npx, (size_t)m, cudaMemcpyDeviceToDevice, st));
-        const int rc = z_encode_records(z, planes, m, 2 * (long long)npx, (long long)npx, timestamps);
+        RIRB_CUDA_OK(interleave_planes(z, planes, m, cudaMemcpyDeviceToDevice, st));
+        const int rc = z_encode_records(z, planes, m, 2 * (long long)z->w * z->h, (long long)z->w * z->h, timestamps);
         ph.mark("write: pre-code + device zstd", m);
         return rc;
     }
-    // per frame [lo | hi], so that a record's payload is one contiguous run for zstd
-    RIRB_CUDA_OK(cudaMemcpy2DAsync(z->host_planes, 2 * npx, z->dev_lo(), npx, npx, (size_t)m, cudaMemcpyDeviceToHost, st));
-    RIRB_CUDA_OK(cudaMemcpy2DAsync(z->host_planes + npx, 2 * npx, z->dev_hi(), npx, npx, (size_t)m, cudaMemcpyDeviceToHost, st));
+    RIRB_CUDA_OK(interleave_planes(z, z->host_planes(), m, cudaMemcpyDeviceToHost, st));
     RIRB_CUDA_OK(cudaStreamSynchronize(st));
     ph.mark("write: pre-code + download", m);
-    const int rc = z_write_records(z, z->host_planes, m, timestamps, threads);
+    const int rc = z_write_records(z, z->host_planes(), m, timestamps, threads);
     ph.mark("write: zstd + records", m);
     return rc;
 }
 
-// one device frame into the pending GOP (host): on the caller's stream, so that it sees the work queued there
-static cudaError_t z_download_frame(void* dst, const void* src, size_t bytes, cudaStream_t st)
+// the frames of an unfinished GOP (it starts on a key frame, so it stands on its own)
+static int z_flush_pending(ZMovie* z, int threads)
 {
-    const cudaError_t e = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, st);
-    return e == cudaSuccess ? cudaStreamSynchronize(st) : e;
+    const long long m = (long long)z->pending_times.size();
+    if (m == 0) return 0;
+    const size_t npx = (size_t)z->w * z->h;
+    if (!z->reserve((size_t)m)) return -1;
+    RIRB_CUDA_OK(cudaMemcpyAsync(z->dev_movie(), z->pending.data(), (size_t)m * npx * 2, cudaMemcpyHostToDevice, current_stream()));
+    const int rc = z_flush_gops(z, z->dev_movie(), m, (long long)z->times.size(), (const long long*)z->pending_times.data(), threads);
+    z->pending.clear();
+    z->pending_times.clear();
+    return rc;
+}
+
+// n frames (host or device) onto the pending GOP (host); device frames on the caller's stream, so that the copy sees the work
+// queued there
+static cudaError_t z_pend(ZMovie* z, const u16* frames, long long n, const long long* timestamps, bool on_device, cudaStream_t st)
+{
+    const size_t npx = (size_t)z->w * z->h, have = z->pending_times.size();
+    z->pending.resize((have + (size_t)n) * npx);
+    cudaError_t e = cudaSuccess;
+    if (!on_device)
+        memcpy(z->pending.data() + have * npx, frames, (size_t)n * npx * 2);
+    else if ((e = cudaMemcpyAsync(z->pending.data() + have * npx, frames, (size_t)n * npx * 2, cudaMemcpyDeviceToHost, st)) == cudaSuccess)
+        e = cudaStreamSynchronize(st);
+    if (e == cudaSuccess) z->pending_times.insert(z->pending_times.end(), timestamps, timestamps + n);
+    return e;
 }
 
 // methods 2 / 3.  Whole GOPs go through the GPU pre-coder as they come; what does not fill a GOP waits in z->pending
@@ -1089,29 +1063,15 @@ static int z_write_precoded(ZMovie* z, const unsigned short* frames, long long n
 {
     const size_t npx = (size_t)z->w * z->h;
     const long long gop = z->method == 3 ? z->gop : 1;
-    // how many frames one pass takes: whole GOPs, about 64 MB of pixels
-    long long chunk = std::max<long long>(1, (64ll << 20) / (long long)(npx * 2));
-    chunk = std::max(gop, chunk / gop * gop);
+    const long long chunk = z_pass_frames(z, gop);
     const bool on_device = device_pointer(frames);
     cudaStream_t st = current_stream();
     long long done = 0;
     // 1. top up a GOP that is already waiting
-    while (!z->pending_times.empty() && done < nframes) {
-        const size_t have = z->pending_times.size();
-        z->pending.resize((have + 1) * npx);
-        if (on_device)
-            RIRB_CUDA_OK(z_download_frame(z->pending.data() + have * npx, frames + (size_t)done * npx, npx * 2, st));
-        else
-            memcpy(z->pending.data() + have * npx, frames + (size_t)done * npx, npx * 2);
-        z->pending_times.push_back(timestamps[done]);
-        ++done;
-        if ((long long)z->pending_times.size() == gop) {
-            if (!z->reserve((size_t)chunk)) return -1;
-            RIRB_CUDA_OK(cudaMemcpyAsync(z->dev_movie(), z->pending.data(), (size_t)gop * npx * 2, cudaMemcpyHostToDevice, st));
-            if (z_flush_gops(z, z->dev_movie(), gop, (long long)z->times.size(), (const long long*)z->pending_times.data(), threads) != 0) return -1;
-            z->pending.clear();
-            z->pending_times.clear();
-        }
+    if (!z->pending_times.empty()) {
+        done = std::min(nframes, gop - (long long)z->pending_times.size());
+        RIRB_CUDA_OK(z_pend(z, frames, done, timestamps, on_device, st));
+        if ((long long)z->pending_times.size() == gop && (!z->reserve((size_t)chunk) || z_flush_pending(z, threads) != 0)) return -1;
     }
     // 2. whole GOPs straight from the caller's buffer
     while (nframes - done >= gop) {
@@ -1126,30 +1086,23 @@ static int z_write_precoded(ZMovie* z, const unsigned short* frames, long long n
         done += m;
     }
     // 3. the rest waits
-    for (; done < nframes; ++done) {
-        const size_t have = z->pending_times.size();
-        z->pending.resize((have + 1) * npx);
-        if (on_device)
-            RIRB_CUDA_OK(z_download_frame(z->pending.data() + have * npx, frames + (size_t)done * npx, npx * 2, st));
-        else
-            memcpy(z->pending.data() + have * npx, frames + (size_t)done * npx, npx * 2);
-        z->pending_times.push_back(timestamps[done]);
-    }
+    if (done < nframes) RIRB_CUDA_OK(z_pend(z, frames + (size_t)done * npx, nframes - done, timestamps + done, on_device, st));
     return 0;
 }
 
-// the frames of an unfinished GOP (it starts on a key frame, so it stands on its own)
-static int z_flush_pending(ZMovie* z)
+// frames[nframes][h][w] host or device; timestamps host.  Records are appended in order; the frames
+// are compressed `threads` at a time (0: all host cores).
+int rirb_z_write_images(int handle, const unsigned short* frames, long long nframes, const long long* timestamps, int threads)
 {
-    const long long m = (long long)z->pending_times.size();
-    if (m == 0) return 0;
-    const size_t npx = (size_t)z->w * z->h;
-    if (!z->reserve((size_t)std::max<long long>(m, 1))) return -1;
-    RIRB_CUDA_OK(cudaMemcpyAsync(z->dev_movie(), z->pending.data(), (size_t)m * npx * 2, cudaMemcpyHostToDevice, current_stream()));
-    const int rc = z_flush_gops(z, z->dev_movie(), m, (long long)z->times.size(), (const long long*)z->pending_times.data(), 0);
-    z->pending.clear();
-    z->pending_times.clear();
-    return rc;
+    auto z = g_zfiles.get(handle);
+    if (!z || !z->writing || !frames || nframes < 0 || (nframes > 0 && !timestamps)) {
+        set_error("z_write_images: bad handle or arguments");
+        return -1;
+    }
+    if (nframes == 0) return 0;
+    std::lock_guard<std::mutex> lock(z->mu);
+    return z->method == 1 ? z_write_records(z.get(), frames, nframes, timestamps, threads)
+                          : z_write_precoded(z.get(), frames, nframes, timestamps, threads);
 }
 
 int rirb_z_set_coder(int handle, int coder)
@@ -1205,7 +1158,7 @@ long long rirb_z_close_file(int handle)
     long long res = 0;
     if (z->writing) {
         std::lock_guard<std::mutex> lock(z->mu);
-        if (z->method != 1 && z_flush_pending(z.get()) != 0) set_error("z_close_file: the last frames could not be written");
+        if (z->method != 1 && z_flush_pending(z.get(), 0) != 0) set_error("z_close_file: the last frames could not be written");
         z->hdr.trig[T_SAMPLES] = (uint64_t)z->times.size();
         if (pwrite(fileno(z->f), z->hdr.trig, 128, 128) != 128) set_error("z_close_file: cannot update the sample count");
         fclose(z->f);
@@ -1340,67 +1293,9 @@ int rirb_z_get_timestamps(int handle, long long* times)
     return 0;
 }
 
-// frames [pos, pos + count) -> out[count][h][w] (host or device), timestamps (host, may be NULL)
-// Whether record i is a zstd frame with LZ sequences in some block (or cannot be walked).  The device decoder runs the
-// sequences of a frame on one warp, which is slower than the host pool (DESIGN.md 7 f-3, r4); frames without sequences --
-// what the device coder writes -- it decodes faster.  A read takes the decoder by its first record.
-static bool z_record_has_sequences(ZMovie* z, long long i)
-{
-    std::vector<u8> f(z->sizes[i]);
-    if (pread(fileno(z->f), f.data(), f.size(), (off_t)(z->positions[i] + 12)) != (ssize_t)f.size() || f.size() < 6) return true;
-    const size_t n = f.size();
-    const unsigned fhd = f[4];
-    const int single = (fhd >> 5) & 1, fcs_flag = fhd >> 6;
-    size_t p = 5 + (single ? 0 : 1) + (size_t)((fhd & 3) == 3 ? 4 : (fhd & 3)) + (size_t)(fcs_flag ? 1 << fcs_flag : single);
-    for (;;) {
-        if (p + 3 > n) return true;
-        const unsigned h = f[p] | (f[p + 1] << 8) | (f[p + 2] << 16), type = (h >> 1) & 3, size = h >> 3;
-        p += 3;
-        if (type == 2) {
-            if (p + size > n || size < 3) return true;
-            const unsigned b0 = f[p], lt = b0 & 3, sf = (b0 >> 2) & 3;
-            size_t hs, cs;
-            if (lt < 2) {
-                hs = (sf & 1) == 0 ? 1 : sf == 1 ? 2 : 3;
-                const size_t regen = hs == 1 ? b0 >> 3 : hs == 2 ? (b0 >> 4) + (f[p + 1] << 4) : (b0 >> 4) + (f[p + 1] << 4) + (f[p + 2] << 12);
-                cs = lt == 0 ? regen : 1;
-            } else {
-                hs = sf < 2 ? 3 : sf + 2;
-                uint64_t v = 0;
-                for (size_t k = 0; k < hs && p + k < n; ++k) v |= (uint64_t)f[p + k] << (8 * k);
-                const int bits = sf < 2 ? 10 : sf == 2 ? 14 : 18;
-                cs = (size_t)((v >> (4 + bits)) & ((1u << bits) - 1));
-            }
-            if (p + hs + cs >= p + size || f[p + hs + cs] != 0) return true;
-        }
-        if (type == 3) return true;
-        p += type == 1 ? 1 : size;
-        if (h & 1) return false;
-    }
-}
-
-int rirb_z_read_images(int handle, int pos, int count, unsigned short* out, long long* timestamps, int threads)
-{
-    auto z = g_zfiles.get(handle);
-    if (!z || z->writing || !out || pos < 0 || count < 0 || (size_t)pos + (size_t)count > z->times.size()) {
-        set_error("z_read_images: bad handle or range");
-        return -1;
-    }
-    if (count == 0) return 0;
-    std::lock_guard<std::mutex> lock(z->mu);
-    if (z->method != 1 || (option_enabled(OPT_ZSTD_DECODER) && device_pointer(out) &&
-                           (option_value(OPT_ZSTD_DECODER) == 2 || !z_record_has_sequences(z.get(), pos)))) {
-        const int rc = z->method != 1 ? z_read_precoded(z.get(), pos, count, out, threads) : z_read_records_device(z.get(), pos, count, (u8*)out, threads);
-        if (rc == 0 && timestamps)
-            for (int i = 0; i < count; ++i) timestamps[i] = z->times[pos + i];
-        return rc;
-    }
-    return z_read_records(z.get(), pos, count, out, timestamps, threads, false);
-}
-
 // records [pos, pos + count) -> decompressed payloads (w*h*2 bytes each) back to back at `out`; to_pinned_planes: `out` is
-// z->host_planes (host memory, whatever cudaPointerGetAttributes says about pinned buffers)
-static int z_read_records(ZMovie* z, int pos, int count, void* out, long long* timestamps, int threads, bool to_pinned_planes)
+// the pinned planes (host memory, whatever cudaPointerGetAttributes says about pinned buffers)
+static int z_read_records(ZMovie* z, int pos, int count, void* out, int threads, bool to_pinned_planes)
 {
     const size_t fbytes = (size_t)z->w * z->h * 2;
     const int workers = pool_size(threads, count);
@@ -1435,32 +1330,23 @@ static int z_read_records(ZMovie* z, int pos, int count, void* out, long long* t
         }
         std::atomic<bool> failed{false};
         parallel_for(m, workers, [&](long long i, int t) {
-            char* rec = raw.get() + (z->positions[pos + b0 + i] - a) + 12;
+            const long long at = z->positions[pos + b0 + i] + 12;
             const size_t len = z->sizes[pos + b0 + i];
-            size_t have = 0;
-            while (have < len) {
-                const ssize_t r = pread(fd, rec + have, len - have, (off_t)(z->positions[pos + b0 + i] + 12 + (long long)have));
-                if (r <= 0) {
-                    failed = true;
-                    return;
-                }
-                have += (size_t)r;
+            char* rec = raw.get() + (at - a);
+            if (!pread_all(fd, rec, len, at)) {
+                failed = true;
+                return;
             }
-            const size_t got = z_decompress(ctx.get(t), dst + (size_t)i * fbytes, fbytes, rec, z->sizes[pos + b0 + i]);
+            const size_t got = z_decompress(ctx.get(t), dst + (size_t)i * fbytes, fbytes, rec, len);
             if (zstd().isError(got) || got != fbytes) failed = true;
         });
-        if (failed) {
-            set_error("z_read_images: a record cannot be read or does not decompress to a %d x %d image", z->w, z->h);
-            return -1;
-        }
+        if (failed) return z_unreadable(z);
         if (to_device) {
             RIRB_CUDA_OK(cudaMemcpyAsync((char*)out + (size_t)b0 * fbytes, dst, fbytes * m, cudaMemcpyHostToDevice, st));
             RIRB_CUDA_OK(cudaEventRecord(pin.ev[slot], st));
             used[slot] = true;
         }
     }
-    if (timestamps)
-        for (int i = 0; i < count; ++i) timestamps[i] = z->times[pos + i];
     if (to_device) RIRB_CUDA_OK(cudaStreamSynchronize(st));
     return 0;
 }
@@ -1472,16 +1358,9 @@ static int z_read_records(ZMovie* z, int pos, int count, void* out, long long* t
 static int z_read_records_device(ZMovie* z, int pos, int count, u8* out, int threads)
 {
     const size_t fbytes = (size_t)z->w * z->h * 2;
-    const long long chunk = std::max<long long>(1, (64ll << 20) / (long long)fbytes);
+    const long long chunk = z_pass_frames(z, 1);
     cudaStream_t st = current_stream();
-    ZcBuffers& b = z->zc;
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (b.device != dev) {
-        zc_free(b);
-        zc_unpark(b, dev);
-        b.device = dev;
-    }
+    ZBuffers& b = z->buffers();
     const int fd = fileno(z->f);
     long long fallbacks = 0;
     for (long long p0 = pos; p0 < (long long)pos + count;) {
@@ -1491,10 +1370,9 @@ static int z_read_records_device(ZMovie* z, int pos, int count, u8* out, int thr
         const size_t span = (size_t)(z->positions[p0 + m - 1] + 12 + (long long)z->sizes[p0 + m - 1] - a);
         const size_t table = ((span + 63) & ~(size_t)63);  // pinned: the span, then offsets | statuses | sizes
         const size_t bytes = table + (size_t)m * (8 + 8 + 4);
-        if (!z_grow(&b.scratch, &b.scratch_bytes, zdecoder_scratch_bytes(m, (long long)fbytes), false) ||
-            !z_grow(&b.dev, &b.dev_bytes, bytes, false) || !z_grow(&b.host, &b.host_bytes, bytes, true))
+        if (!b.scratch.grow(zdecoder_scratch_bytes(m, (long long)fbytes)) || !b.records.grow(bytes) || !b.host_records.grow(bytes))
             return -1;
-        char* h = b.host;
+        char* h = b.host_records.p;
         long long* off = (long long*)(h + table);
         long long* status = off + m;
         unsigned* len = (unsigned*)(status + m);
@@ -1506,24 +1384,17 @@ static int z_read_records_device(ZMovie* z, int pos, int count, u8* out, int thr
         const long long npieces = (long long)((span + piece - 1) / piece);
         std::atomic<bool> failed{false};
         parallel_for(npieces, pool_size(threads, npieces), [&](long long k, int) {
-            const size_t lo = (size_t)k * piece, n = std::min(piece, span - lo);
-            for (size_t have = 0; have < n && !failed;) {
-                const ssize_t r = pread(fd, h + lo + have, n - have, (off_t)(a + (long long)(lo + have)));
-                if (r <= 0) failed = true;
-                have += r > 0 ? (size_t)r : 0;
-            }
+            const size_t lo = (size_t)k * piece;
+            if (!pread_all(fd, h + lo, std::min(piece, span - lo), a + (long long)lo)) failed = true;
         });
-        if (failed) {
-            set_error("z_read_images: a record cannot be read or does not decompress to a %d x %d image", z->w, z->h);
-            return -1;
-        }
+        if (failed) return z_unreadable(z);
         ph.mark("read: pread span", m);
-        const u8* d = (const u8*)b.dev;
-        long long* dstatus = (long long*)(b.dev + ((char*)status - h));
+        const u8* d = (const u8*)b.records.p;
+        long long* dstatus = (long long*)(b.records.p + ((char*)status - h));
         u8* to = out + (size_t)(p0 - pos) * fbytes;
-        RIRB_CUDA_OK(cudaMemcpyAsync(b.dev, h, bytes, cudaMemcpyHostToDevice, st));
+        RIRB_CUDA_OK(cudaMemcpyAsync(b.records.p, h, bytes, cudaMemcpyHostToDevice, st));
         if (launch_zstd_decode(d, (const long long*)(d + table), (const unsigned*)(d + ((char*)len - h)), m, to, (long long)fbytes,
-                               (long long)fbytes, dstatus, b.scratch, st) != 0)
+                               (long long)fbytes, dstatus, b.scratch.p, st) != 0)
             return -1;
         RIRB_CUDA_OK(cudaMemcpyAsync(status, dstatus, (size_t)m * 8, cudaMemcpyDeviceToHost, st));
         RIRB_CUDA_OK(cudaStreamSynchronize(st));
@@ -1532,10 +1403,8 @@ static int z_read_records_device(ZMovie* z, int pos, int count, u8* out, int thr
         for (long long i = 0; i < m; ++i) {
             if (status[i] == -1 || status[i] == -2)
                 redo.push_back(i);
-            else if (status[i] != (long long)fbytes) {
-                set_error("z_read_images: a record cannot be read or does not decompress to a %d x %d image", z->w, z->h);
-                return -1;
-            }
+            else if (status[i] != (long long)fbytes)
+                return z_unreadable(z);
         }
         if (!redo.empty()) {
             const int workers = pool_size(threads, (long long)redo.size());
@@ -1546,10 +1415,7 @@ static int z_read_records_device(ZMovie* z, int pos, int count, u8* out, int thr
                 const size_t got = z_decompress(z->ctx->get(t), host.data() + (size_t)j * fbytes, fbytes, h + off[i], len[i]);
                 if (zstd().isError(got) || got != fbytes) failed = true;
             });
-            if (failed) {
-                set_error("z_read_images: a record cannot be read or does not decompress to a %d x %d image", z->w, z->h);
-                return -1;
-            }
+            if (failed) return z_unreadable(z);
             for (size_t j = 0; j < redo.size(); ++j)
                 RIRB_CUDA_OK(cudaMemcpyAsync(to + (size_t)redo[j] * fbytes, host.data() + j * fbytes, fbytes, cudaMemcpyHostToDevice, st));
             RIRB_CUDA_OK(cudaStreamSynchronize(st));
@@ -1562,19 +1428,19 @@ static int z_read_records_device(ZMovie* z, int pos, int count, u8* out, int thr
     return 0;
 }
 
-// methods 2 / 3: records -> planes (host, or the device decoder when "zstd_decoder" is 2) -> device -> merge (+ undo the temporal delta from the GOP's key frame on).
-// The decoded frames of the last pass stay in z->dev_buf: a reader that asks for one frame at a time decodes a GOP once.
-static int z_read_precoded(ZMovie* z, int pos, int count, unsigned short* out, int threads)
+// methods 2 / 3: records -> planes (host zstd, or the device decoder) -> device -> merge (+ undo the temporal delta from the GOP's
+// key frame on).  The decoded frames of the last pass stay on the device: a reader that asks for one frame at a time decodes a
+// GOP once.
+static int z_read_precoded(ZMovie* z, int pos, int count, unsigned short* out, int threads, bool device_decoder)
 {
     const size_t npx = (size_t)z->w * z->h;
     const long long gop = z->method == 3 ? z->gop : 1;
-    long long chunk = std::max<long long>(1, (64ll << 20) / (long long)(npx * 2));
-    chunk = std::max(gop, chunk / gop * gop);
+    const long long chunk = z_pass_frames(z, gop);
     cudaStream_t st = current_stream();
     const bool to_device = device_pointer(out);
     long long p = pos;
     const long long end = (long long)pos + count;
-    bool in_flight = false;  // the stream may still be reading host_planes / dev_buf for the previous chunk
+    bool in_flight = false;  // the stream may still be reading the pinned planes / device frames for the previous chunk
     while (p < end) {
         if (!(z->cache_first >= 0 && p >= z->cache_first && p < z->cache_first + z->cache_count)) {
             const long long k0 = p - p % gop;                                            // the GOP's key frame
@@ -1586,17 +1452,15 @@ static int z_read_precoded(ZMovie* z, int pos, int count, unsigned short* out, i
             if (!z->reserve((size_t)chunk)) return -1;
             ph.mark("read: reserve", m);
             z->cache_first = -1;
-            if (option_value(OPT_ZSTD_DECODER) == 2) {
-                // [frame][lo | hi] into the frames' part of dev_buf, then apart into the two plane buffers
+            if (device_decoder) {
+                // [frame][lo | hi] into the frames' part of the device buffer, then apart into the two plane buffers
                 u8* planes = (u8*)z->dev_movie();
                 if (z_read_records_device(z, (int)k0, (int)m, planes, threads) != 0) return -1;
-                RIRB_CUDA_OK(cudaMemcpy2DAsync(z->dev_lo(), npx, planes, 2 * npx, npx, (size_t)m, cudaMemcpyDeviceToDevice, st));
-                RIRB_CUDA_OK(cudaMemcpy2DAsync(z->dev_hi(), npx, planes + npx, 2 * npx, npx, (size_t)m, cudaMemcpyDeviceToDevice, st));
+                RIRB_CUDA_OK(split_planes(z, planes, m, cudaMemcpyDeviceToDevice, st));
             } else {
-                if (z_read_records(z, (int)k0, (int)m, z->host_planes, nullptr, threads, true) != 0) return -1;
+                if (z_read_records(z, (int)k0, (int)m, z->host_planes(), threads, true) != 0) return -1;
                 ph.mark("read: records + zstd", m);
-                RIRB_CUDA_OK(cudaMemcpy2DAsync(z->dev_lo(), npx, z->host_planes, 2 * npx, npx, (size_t)m, cudaMemcpyHostToDevice, st));
-                RIRB_CUDA_OK(cudaMemcpy2DAsync(z->dev_hi(), npx, z->host_planes + npx, 2 * npx, npx, (size_t)m, cudaMemcpyHostToDevice, st));
+                RIRB_CUDA_OK(split_planes(z, z->host_planes(), m, cudaMemcpyHostToDevice, st));
             }
             if (rirb_decode_movie(z->dev_lo(), z->dev_hi(), m, z->w, z->h, z->gop, z->method == 3, k0, z->dev_movie()) != 0) return -1;
             z->cache_first = k0;
@@ -1612,9 +1476,9 @@ static int z_read_precoded(ZMovie* z, int pos, int count, unsigned short* out, i
             // a run of frames for a host caller: down into the pinned buffer (the planes in it are consumed by now, it holds
             // exactly a chunk of frames), then into the caller's pageable memory by the host pool -- the driver's own pageable
             // download is one thread faulting the destination in page by page (0.3 GB/s measured on a fresh numpy array)
-            RIRB_CUDA_OK(cudaMemcpyAsync(z->host_planes, from, (size_t)n * npx * 2, cudaMemcpyDeviceToHost, st));
+            const char* hp = z->host_planes();
+            RIRB_CUDA_OK(cudaMemcpyAsync(z->host_planes(), from, (size_t)n * npx * 2, cudaMemcpyDeviceToHost, st));
             RIRB_CUDA_OK(cudaStreamSynchronize(st));
-            const char* hp = z->host_planes;
             parallel_for(n, pool_size(threads, (int)n), [&](long long i, int) { memcpy(to + (size_t)i * npx, hp + (size_t)i * npx * 2, npx * 2); });
         } else {
             RIRB_CUDA_OK(cudaMemcpyAsync(to, from, (size_t)n * npx * 2, cudaMemcpyDeviceToHost, st));
@@ -1624,6 +1488,40 @@ static int z_read_precoded(ZMovie* z, int pos, int count, unsigned short* out, i
     }
     RIRB_CUDA_OK(cudaStreamSynchronize(st));
     return 0;
+}
+
+// Which decoder a read takes.  The "zstd_decoder" switch: 0 host zstd, 2 the device decoder for every read that ends on the
+// device (methods 2 / 3 always do), 1 (the default) the device decoder only for a method-1 read into device memory whose first
+// record is a frame without LZ sequences -- what the device coder writes.  The device decoder runs the sequences of a frame
+// on one warp, which is slower than the host pool (DESIGN.md 7 f-3, r4); frames without sequences it decodes faster.
+static bool z_use_device_decoder(ZMovie* z, int pos, const void* out)
+{
+    const int mode = option_value(OPT_ZSTD_DECODER);
+    if (z->method != 1) return mode == 2;
+    if (mode == 0 || !device_pointer(out)) return false;
+    if (mode == 2) return true;
+    std::vector<u8> f(z->sizes[pos]);
+    return pread_all(fileno(z->f), f.data(), f.size(), z->positions[pos] + 12) &&
+           zdecoder_frame_plain(f.data(), (long long)f.size(), (long long)z->w * z->h * 2);
+}
+
+// frames [pos, pos + count) -> out[count][h][w] (host or device), timestamps (host, may be NULL)
+int rirb_z_read_images(int handle, int pos, int count, unsigned short* out, long long* timestamps, int threads)
+{
+    auto z = g_zfiles.get(handle);
+    if (!z || z->writing || !out || pos < 0 || count < 0 || (size_t)pos + (size_t)count > z->times.size()) {
+        set_error("z_read_images: bad handle or range");
+        return -1;
+    }
+    if (count == 0) return 0;
+    std::lock_guard<std::mutex> lock(z->mu);
+    const bool device_decoder = z_use_device_decoder(z.get(), pos, out);
+    const int rc = z->method != 1 ? z_read_precoded(z.get(), pos, count, out, threads, device_decoder)
+                   : device_decoder ? z_read_records_device(z.get(), pos, count, (u8*)out, threads)
+                                    : z_read_records(z.get(), pos, count, out, threads, false);
+    if (rc == 0 && timestamps)
+        for (int i = 0; i < count; ++i) timestamps[i] = z->times[pos + i];
+    return rc;
 }
 
 int rirb_z_read_image(int handle, int pos, unsigned short* img, long long* timestamp)

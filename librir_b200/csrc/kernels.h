@@ -94,6 +94,8 @@ int launch_zstd_encode_lz(const u8* src, long long n, long long bytes_each, long
 // zdecoder.cu: n zstd frames (frame i at src + offsets[i], sizes[i] bytes) -> content at dst + i * dst_stride, at most cap
 // bytes; status[i] = bytes, -1 malformed, -2 refused (rirb_zstd_decode_batch).  scratch: zdecoder_scratch_bytes(n, cap).
 size_t zdecoder_scratch_bytes(long long n, long long cap);
+// Host: 1 when the frame at f (host memory) is one the decoder takes, with content of at most cap bytes and no LZ sequences.
+int zdecoder_frame_plain(const u8* f, long long size, long long cap);
 int launch_zstd_decode(const u8* src, const long long* offsets, const unsigned* sizes, long long n, u8* dst, long long dst_stride,
                        long long cap, long long* status, void* scratch, cudaStream_t st);
 

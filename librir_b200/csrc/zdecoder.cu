@@ -854,6 +854,13 @@ size_t zdecoder_scratch_bytes(long long n, long long cap)
     return (size_t)n * (((size_t)cap + 255) / 256 * 256) + (size_t)n * sizeof(ZdFrame) + 256;
 }
 
+int zdecoder_frame_plain(const u8* f, long long size, long long cap)
+{
+    ZdFrame fr;
+    zd_scan_frame(f, size, cap, fr);
+    return fr.err == 0 && !fr.has_seq;
+}
+
 int launch_zstd_decode(const u8* src, const long long* offsets, const unsigned* sizes, long long n, u8* dst, long long dst_stride,
                        long long cap, long long* status, void* scratch, cudaStream_t st)
 {
