@@ -71,6 +71,8 @@ def test_corpus_covers_every_feature():
                 seen.add("ml_code_52")
             if any(ll == 0 for ll, _, _ in seqs):
                 seen.add("ll_0")
+            if any(ll >= 65536 for ll, _, _ in seqs):
+                seen.add("ll_code_35")
             if len(seqs) == 1:
                 seen.add("one_sequence")  # every table in mode RLE
             if len(seqs) >= 128:
@@ -87,7 +89,7 @@ def test_corpus_covers_every_feature():
             seen.add(("raw", "rle", "huffman", "?")[lit_kind] + "_literals")
     # RLE literals cannot occur in a block that takes the LZ form: every byte value of a block is a literal once, so
     # literals of one value mean a block of one value, and that block is coder 1's RLE block
-    assert seen >= {"lz_block", "overlap", "run", "ml_code_52", "ll_0", "one_sequence", "two_byte_count",
+    assert seen >= {"lz_block", "overlap", "run", "ml_code_52", "ll_0", "ll_code_35", "one_sequence", "two_byte_count",
                     "no_trailing_literals", "offset_w", "segments", "predefined", "all_rle", "raw_literals",
                     "huffman_literals"}, seen
 

@@ -40,6 +40,8 @@ def cases():
     for n in (7, 8, 9, 15, 16, 17, 300):
         out.append((f"short{n}", np.tile(np.array([1, 2, 3], np.uint8), n)[:n], 0))
     out.append(("random_with_copies", np.concatenate([rng.integers(0, 256, 20000).astype(np.uint8)] * 3), 0))
+    tail = rng.integers(0, 256, 100000).astype(np.uint8)
+    out.append(("ll_code_35", np.concatenate([tail, tail[:20]]), 0))  # the one sequence (LL 100 000, ML 20, offset 100 000)
     mov = C.movie(3, 120, 160, seed=4)
     for method in (1, 2):
         p = mov.reshape(3, -1).view(np.uint8) if method == 1 else K.planes(mov, method)
