@@ -5,7 +5,8 @@ the Gaussian radius and the grid limits.  Freshly allocated buffers are 256-byte
 defaults, so without this file several instantiations that ship in the library would never run under test.  Every
 case here names the kernel it expects (``kernels_run`` reads the launched kernels back from ``torch.profiler``),
 checks that the kernel of the other path did NOT run, and compares the result with the oracle and with the default
-route.  The last test checks that the cases together reached every instantiation in ``ALL_KERNELS``.
+route (Gaussian: with the float64 operation of tests/gauss_exact.py, within its rounding bound on every pixel).  The
+last test checks that the cases together reached every instantiation in ``ALL_KERNELS``.
 """
 import contextlib
 import re
@@ -14,7 +15,8 @@ import numpy as np
 import pytest
 
 from tests.conftest import ir_movie
-from tests.test_gpu_parity import assert_gauss_close, reference_reads_past_the_buffer, to_dev, to_host
+from tests.gauss_exact import assert_gauss_exact
+from tests.test_gpu_parity import reference_reads_past_the_buffer, to_dev, to_host
 
 pytestmark = pytest.mark.gpu
 
@@ -197,7 +199,7 @@ GAUSS_SHAPES = [(3, 130, 264), (2, 65, 136), (2, 1, 8), (2, 5, 12), (2, 3, 16), 
 @pytest.mark.parametrize("dt", [np.uint16, np.float32], ids=["u16", "f32"])
 @pytest.mark.parametrize("sigma", [0.5, 1.0, 1.5, 2.0, 2.6])
 @pytest.mark.parametrize("shape", GAUSS_SHAPES, ids=lambda s: "x".join(map(str, s)))
-def test_gaussian_every_kernel(best, dt, sigma, shape):
+def test_gaussian_every_kernel(dt, sigma, shape):
     """R = max(1, int(2 sigma)) = 1..5 on tile seams, below one tile and below 2R+1 rows; every kernel the launcher
     can pick for the shape: tile, wide, sep (gauss_tma = 0, and uint16 rows that are 8 but not 16 bytes), the first-
     generation tile kernel at R = 3, 4 (gauss_tma = 2) and the generic kernel (misaligned input or output, R > 4)."""
@@ -205,19 +207,14 @@ def test_gaussian_every_kernel(best, dt, sigma, shape):
     r = max(1, int(2 * sigma))
     rng = np.random.default_rng(h * w + r)
     mov = (rng.integers(0, 16384, shape) if dt == np.uint16 else rng.random(shape) * 5000 - 1000).astype(dt)
-    want = [best.gaussian_filter(f.astype(np.float32), sigma) for f in mov]
     d = to_dev(mov)
     esz = np.dtype(dt).itemsize
     default, names = kernels_run(lambda: sp.gaussian_filter_batch(d, sigma))
     expect(names, gauss_route(dt, r, w, d, default, "default"), GAUSS, "default")
-    default = default.cpu().numpy()
-    for t in range(n):
-        assert_gauss_close(default[t], want[t])
+    assert_gauss_exact(default.cpu().numpy(), mov, sigma, "default")
 
     def check(got, what):
-        for t in range(n):
-            assert_gauss_close(got[t], want[t])
-            assert_gauss_close(got[t], default[t])
+        assert_gauss_exact(got, mov, sigma, what)
 
     for name, value, route in [("gauss_tma", 0, "sep"), ("gauss_tma", 2, "tile")]:
         _lib.set_parameter(name, value)
@@ -265,6 +262,7 @@ def test_bad_pixels_correct_gaussian_every_radius(shape, sigma):
     want_g = sp.gaussian_filter_batch(want_c, sigma)
     assert torch.equal(fc.view(torch.int16), want_c.view(torch.int16))
     assert torch.equal(fg, want_g)
+    assert_gauss_exact(fg.cpu().numpy(), to_host(want_c), sigma, "fused")
     for c_off, g_off in [(2, 0), (0, 4), (16 + 2, 8)]:
         cor, sm = Placed(shape, np.uint16, c_off), Placed(shape, np.float32, g_off)
         _, names = kernels_run(lambda: bp.correct_gaussian_batch(d, sigma, out=cor.t, smoothed=sm.t))
@@ -277,8 +275,7 @@ def test_bad_pixels_correct_gaussian_every_radius(shape, sigma):
         assert torch.equal(cor.t.view(torch.int16), sep_c.t.view(torch.int16))
         assert torch.equal(sm.t, sep_g.t)
         assert torch.equal(cor.t.view(torch.int16), want_c.view(torch.int16))
-        for t in range(n):
-            assert_gauss_close(sm.t[t].cpu().numpy(), fg[t].cpu().numpy())
+        assert_gauss_exact(sm.t.cpu().numpy(), to_host(want_c), sigma, f"fallback corrected+{c_off} smoothed+{g_off}")
         assert cor.untouched_outside() and sm.untouched_outside(), "a fallback kernel wrote outside its view"
 
 
@@ -395,9 +392,9 @@ def pid(o):
 
 
 @pytest.mark.parametrize("shape", ALIGN_SHAPES, ids=SHAPE_IDS)
-def test_bad_pixels_and_gaussian_alignment(port, best, shape):
+def test_bad_pixels_and_gaussian_alignment(port, shape):
     """correct_batch, correct_gaussian_batch, gaussian_filter_batch on inputs and outputs misaligned independently:
-    bit-identical to the aligned call (Gaussian: within the bar of it and of the oracle), the vector kernel exactly
+    bit-identical to the aligned call (Gaussian: within the bound of the float64 operation), the vector kernel exactly
     when the layout allows it, and nothing written outside the output views."""
     n, h, w = shape
     mov = bp_movie(n, h, w, 3 * h + w)
@@ -407,9 +404,6 @@ def test_bad_pixels_and_gaussian_alignment(port, best, shape):
     d = to_dev(mov)
     ref_c = to_host(bp.correct_batch(d))
     np.testing.assert_array_equal(ref_c, want_c)
-    want_g = [best.gaussian_filter(f.astype(np.float32), 1.0) for f in want_c]
-    ref_g = sp.gaussian_filter_batch(to_dev(want_c), 1.0).cpu().numpy()
-    ref_cg = [x for x in bp.correct_gaussian_batch(d, 1.0)]
     for io, oo in U16_OFFSETS:
         src = Placed(shape, np.uint16, io, fill=mov)
         what = f"in+{io} out+{oo}"
@@ -424,10 +418,7 @@ def test_bad_pixels_and_gaussian_alignment(port, best, shape):
         gout = Placed(shape, np.float32, oo * 2)
         _, names = kernels_run(lambda: sp.gaussian_filter_batch(csrc.t, 1.0, out=gout.t))
         expect(names, gauss_route(np.uint16, 2, w, csrc.t, gout.t, "default"), GAUSS, f"gaussian {what}")
-        g = gout.t.cpu().numpy()
-        for t in range(n):
-            assert_gauss_close(g[t], want_g[t])
-            assert_gauss_close(g[t], ref_g[t])
+        assert_gauss_exact(gout.t.cpu().numpy(), want_c, 1.0, f"gaussian {what}")
         assert gout.untouched_outside(), f"gaussian {what}"
 
         cor, sm = Placed(shape, np.uint16, oo), Placed(shape, np.float32, 2 * io + (4 if oo else 0))
@@ -440,10 +431,7 @@ def test_bad_pixels_and_gaussian_alignment(port, best, shape):
                     gauss_route(np.uint16, 2, w, cor.t, sm.t, "default")}
         expect(names, kern, GAUSS + ("bp_correct_kernel",), f"correct_gaussian {what}")
         np.testing.assert_array_equal(cor.host(), ref_c, err_msg=f"correct_gaussian {what}")
-        g = sm.t.cpu().numpy()
-        for t in range(n):
-            assert_gauss_close(g[t], ref_cg[1][t].cpu().numpy())
-            assert_gauss_close(g[t], want_g[t])
+        assert_gauss_exact(sm.t.cpu().numpy(), want_c, 1.0, f"correct_gaussian {what}")
         assert cor.untouched_outside() and sm.untouched_outside(), f"correct_gaussian {what}"
 
 

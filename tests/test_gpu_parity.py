@@ -3,7 +3,8 @@ numpy out for the per-frame entries; torch CUDA tensors for the batched ones).
 
 Bars (BASELINE.json north_star): bit-exact for bad pixels, pre-coder, statistics -- and, since
 the blend is evaluated in the reference's fp64 order, for integer translate as well (the
-allowed +-1 LSB is not used); 1e-5 relative (+1e-6*max floor) for float32 Gaussian output.
+allowed +-1 LSB is not used); float32 Gaussian output within the rounding bound of the float64 operation on every
+pixel (tests/gauss_exact.py).
 """
 import os
 
@@ -11,6 +12,7 @@ import numpy as np
 import pytest
 
 from tests.conftest import ir_frame, ir_movie
+from tests.gauss_exact import assert_gauss_exact, assert_reference_exact
 from tests.golden.make_golden import DTYPES, STRATEGIES, typed_image
 
 pytestmark = pytest.mark.gpu
@@ -54,12 +56,6 @@ def to_host(t):
     if t.dtype == torch.uint16:
         return t.cpu().view(torch.int16).numpy().view(np.uint16)
     return t.cpu().numpy()
-
-
-def assert_gauss_close(got, want):
-    tol = 1e-5 * np.abs(want) + 1e-6 * float(np.abs(want).max())
-    bad = np.abs(got.astype(np.float64) - want.astype(np.float64)) > tol
-    assert not bad.any(), f"{bad.sum()} pixels out of tolerance, max abs err {np.abs(got - want).max()}"
 
 
 # ---------------------------------------------------------------------------------------------
@@ -115,15 +111,15 @@ def test_translate_u16_odd_shapes(best, shape):
 
 def test_kernel_variant_switches():
     """rirb_set_parameter: the register-only kernels behind "translate_tma" / "gauss_tma" = 0 give the same
-    results as the TMA-tiled ones (bit-exact translate; Gaussian within tolerance of each other)."""
+    results as the TMA-tiled ones (bit-exact translate; Gaussian within the bound of the float64 operation)."""
     f = ir_frame(96, 128, 5)
     want_t = sp.translate(f, 1.3, -2.7, "nearest", 0)
-    want_g = sp.gaussian_filter(f, 1.0)
+    assert_gauss_exact(sp.gaussian_filter(f, 1.0), f, 1.0, "default")
     try:
         _lib.set_parameter("translate_tma", 0)
         _lib.set_parameter("gauss_tma", 0)
         np.testing.assert_array_equal(sp.translate(f, 1.3, -2.7, "nearest", 0), want_t)
-        assert_gauss_close(sp.gaussian_filter(f, 1.0), want_g)
+        assert_gauss_exact(sp.gaussian_filter(f, 1.0), f, 1.0, "gauss_tma = 0")
     finally:
         _lib.set_parameter("translate_tma", 1)
         _lib.set_parameter("gauss_tma", 1)
@@ -290,46 +286,47 @@ def test_translate_identity_and_integer_shift_properties():
 # gaussian
 # ---------------------------------------------------------------------------------------------
 def test_gaussian_golden(golden):
+    """The compiled reference's outputs (the goldens) are within the reference's own rounding bound of the float64
+    operation -- that pins the operation to the reference -- and the kernel is within the kernel's bound of it."""
     g = golden["ga_in"]
     for k, s in enumerate(golden["ga_sigmas"]):
-        assert_gauss_close(sp.gaussian_filter(g, float(s)), golden[f"ga_{k}"])
+        assert_reference_exact(golden[f"ga_{k}"], g, float(s), f"golden sigma {s}")
+        assert_gauss_exact(sp.gaussian_filter(g, float(s)), g, float(s), f"sigma {s}")
 
 
 @pytest.mark.parametrize("sigma", [0.5, 1.0, 2.0])
-def test_gaussian_full_frame(best, sigma):
+def test_gaussian_full_frame(sigma):
     f = ir_frame(512, 640, 41)
-    want = best.gaussian_filter(f, sigma)
-    assert_gauss_close(sp.gaussian_filter(f, sigma), want)
-    d = to_dev(np.stack([f, f[::-1].copy()]))
+    assert_gauss_exact(sp.gaussian_filter(f, sigma), f, sigma)
+    pair = np.stack([f, f[::-1].copy()])
+    d = to_dev(pair)
     got = sp.gaussian_filter_batch(d, sigma).cpu().numpy()  # fused uint16 -> float32 path
-    assert_gauss_close(got[0], want)
-    assert_gauss_close(got[1], best.gaussian_filter(f[::-1].copy(), sigma))
+    assert_gauss_exact(got, pair, sigma)
     gotf = sp.gaussian_filter_batch(d.view(torch.int16).to(torch.float32), sigma).cpu().numpy()
     np.testing.assert_array_equal(gotf, got)
 
 
 @pytest.mark.parametrize("shape,sigma", [((37, 53), 1.0), ((5, 7), 1.0), ((3, 3), 2.0), ((40, 56), 4.2), ((64, 128), 3.0),
                                          ((33, 132), 0.5), ((16, 260), 1.5)])
-def test_gaussian_odd_shapes_and_large_sigma(best, shape, sigma):
+def test_gaussian_odd_shapes_and_large_sigma(shape, sigma):
     rng = np.random.default_rng(6)
     img = (rng.random(shape) * 4000).astype(np.float32)
-    assert_gauss_close(sp.gaussian_filter(img, sigma), best.gaussian_filter(img, sigma))
+    assert_gauss_exact(sp.gaussian_filter(img, sigma), img, sigma)
 
 
 @pytest.mark.parametrize("shape", [(8, 8), (1, 8), (64, 128), (65, 136), (130, 264), (63, 120), (200, 320)])
 @pytest.mark.parametrize("sigma", [0.5, 1.0, 1.7, 2.4])
-def test_gaussian_tiled_shapes_u16_and_f32(best, shape, sigma):
+def test_gaussian_tiled_shapes_u16_and_f32(shape, sigma):
     """TMA-tiled kernel (16-byte aligned rows), radius 1..4, uint16 and float32 input, tile edges."""
     rng = np.random.default_rng(61)
     f = rng.integers(0, 16384, shape, dtype=np.uint16)
-    want = best.gaussian_filter(f.astype(np.float32), sigma)
-    assert_gauss_close(sp.gaussian_filter(f, sigma), want)
+    assert_gauss_exact(sp.gaussian_filter(f, sigma), f, sigma)
+    assert_gauss_exact(sp.gaussian_filter(f.astype(np.float32), sigma), f, sigma, "float32 input")
     got = sp.gaussian_filter_batch(to_dev(np.stack([f, f])), sigma).cpu().numpy()
-    assert_gauss_close(got[0], want)
-    assert_gauss_close(got[1], want)
+    assert_gauss_exact(got, np.stack([f, f]), sigma, "batch")
 
 
-def test_gaussian_randomized(best):
+def test_gaussian_randomized():
     """60 random (shape, sigma, dtype) cases through both input types."""
     rng = np.random.default_rng(77 + FUZZ_SEED)
     for case in range(60 * FUZZ_SCALE):
@@ -338,14 +335,9 @@ def test_gaussian_randomized(best):
         sigma = float(rng.choice([0.3, 0.5, 0.8, 1.0, 1.3, 1.7, 2.0, 2.49, 3.1]))
         if case % 2:
             img = rng.integers(0, 16384, (h, w), dtype=np.uint16)
-            want = best.gaussian_filter(img.astype(np.float32), sigma)
         else:
             img = (rng.random((h, w)) * 5000 - 1000).astype(np.float32)
-            want = best.gaussian_filter(img, sigma)
-        got = sp.gaussian_filter(img, sigma)
-        tol = 1e-5 * np.abs(want) + 1e-6 * float(np.abs(want).max() + 1e-30)
-        bad = np.abs(got.astype(np.float64) - want.astype(np.float64)) > tol
-        assert not bad.any(), f"case {case}: {h}x{w} sigma {sigma}: {bad.sum()} pixels out of tolerance"
+        assert_gauss_exact(sp.gaussian_filter(img, sigma), img, sigma, f"case {case}: {h}x{w} {img.dtype}")
 
 
 def test_gaussian_constant_image_stays_constant():
@@ -757,7 +749,7 @@ def test_more_frames_than_one_grid_dimension(port, best):
     np.testing.assert_array_equal(back, mov)
     for t in [0, 1, 65534, 65535, 65536, 65537, n - 1]:
         np.testing.assert_array_equal(reg[t], best.translate(mov[t], dx[t], dy[t], "nearest", 0), err_msg=f"translate frame {t}")
-        assert_gauss_close(sm[t], best.gaussian_filter(mov[t].astype(np.float32), 1.0))
+        assert_gauss_exact(sm[t], mov[t], 1.0, f"gaussian frame {t}")
         np.testing.assert_array_equal(cor[t], port.bad_pixels_correct_with(xy, clamp, mov[t]), err_msg=f"bad pixels frame {t}")
 
 
@@ -887,7 +879,7 @@ def test_full_size_pipeline_matches_oracle_on_sampled_frames(port):
     for t in (0, 1, 49, 50, 59):
         oc = port.bad_pixels_correct_with(oxy, oclamp, mov[t])
         np.testing.assert_array_equal(to_host(c[t]), oc)
-        assert_gauss_close(s[t].cpu().numpy(), port.gaussian_filter(oc.astype(np.float32), 1.0))
+        assert_gauss_exact(s[t].cpu().numpy(), oc, 1.0, f"smoothed frame {t}")
         np.testing.assert_array_equal(to_host(r[t]), port.translate(oc, dx[t], dy[t], "nearest", 0))
     reg = to_host(r)
     olo, ohi = port.precode_movie(reg, 50, True)
