@@ -158,7 +158,11 @@ __global__ void ecc_u16_to_f32_kernel(const u16* __restrict__ src, float* __rest
 __global__ void ecc_cast_u16_kernel(const float* __restrict__ src, u16* __restrict__ dst, int n)
 {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) dst[i] = (u16)__float2int_rz(src[i]);  // numpy astype(uint16) on in-range values
+    if (i >= n) return;
+    // numpy's astype(uint16) on x86-64: cvttss2si to int32, low 16 bits kept.  NaN and values beyond int range give
+    // INT_MIN, i.e. 0 -- where __float2int_rz would saturate +inf and values >= 2^31 to 65,535
+    const float v = src[i];
+    dst[i] = (v >= -2147483648.0f && v < 2147483648.0f) ? (u16)__float2int_rz(v) : (u16)0;
 }
 
 // ---- one ECC iteration (ecc.cpp, the body of the for loop), in pieces shared by the two drivers below -----------

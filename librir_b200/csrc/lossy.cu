@@ -15,8 +15,9 @@
 // Time is sequential (every frame needs the previous frame's state and two global reductions of its
 // own), pixels are parallel: three small launches per frame on one stream (the two scalar steps run in the
 // last CTA of the reduction that feeds them).  All sums are exact integers
-// (the reference adds int products into doubles, exact below 2^53), the scalar decision is evaluated in
-// non-contracted fp64 by one thread, so the outputs are bit-identical to the COMPILED reference (oracle/_ref/libs/
+// (the reference adds int products into doubles, exact below 2^53; its products wrap, see lossy_wrapped_square), the
+// scalar decision is evaluated in non-contracted fp64 by one thread with x86's float -> int conversion (lossy_sub_rounded),
+// so the outputs are bit-identical to the COMPILED reference (oracle/_ref/libs/
 // libvideo_io.so; tests/golden/vio_golden.npz) -- including what its overlapping memcpy at :2347 does to the window of
 // spreads (see lossy_window_quirk below).
 // State per pixel: sums u32, const (value u16, count i16), refT, prevT, lastDL u16 and a ring of
@@ -60,6 +61,16 @@ struct LossyScalars {
 __device__ __forceinline__ void lossy_window_quirk(double (*win)[2], int nstds, int quirk)
 {
     if (quirk && nstds == 40) win[38][1] = win[39][1];
+}
+
+// stdDev's `sum_diff2 += diff * diff` (:1993-2036) multiplies ints: for |diff| >= 46341 the product wraps modulo
+// 2^32 (undefined in C++, a wrap as x86-64 builds it), and the wrapped, possibly negative value is what the reference adds
+// into its double sum.  Here the wrapped products are added in signed 64-bit two's complement (carried in the unsigned long
+// long sums and slots) and converted to double once.  That equals the reference's sequential double sum as long as every
+// partial sum stays exact in a double: |product| <= 2^31, so up to 2^22 lossy pixels (DESIGN.md section 4).
+__device__ __forceinline__ unsigned long long lossy_wrapped_square(int d)
+{
+    return (unsigned long long)(long long)(int)((unsigned)d * (unsigned)d);
 }
 
 __global__ void lossy_min_kernel(const u16* __restrict__ tmp, int ns, LossyScalars* sc)
@@ -172,6 +183,16 @@ __global__ void __launch_bounds__(1024) lossy_prep_kernel(const u16* __restrict_
 // memory pays a full round trip per entry: 40 us per frame in the first version of this kernel).
 // nstds: size of the stdDevs window BEFORE this frame (0..40); head: slot of its oldest entry when full;
 // first: this is the first non-initial frame.
+// `error -= (int)round(x)` (:2367-2368, :2559-2563) as the reference's x86-64 build evaluates it: cvttsd2si gives INT_MIN
+// for NaN -- an empty background / foreground split makes a spread 0 / 0 -- and for values beyond int range, and the int
+// subtraction wraps.  A plain (int) here would be cvt.rzi, which saturates and turns NaN into 0.
+__device__ __forceinline__ int lossy_sub_rounded(int error, double x)
+{
+    const double r = round(x);
+    const int k = (r >= -2147483648.0 && r <= 2147483647.0) ? (int)r : INT_MIN;
+    return (int)((unsigned)error - (unsigned)k);
+}
+
 __device__ __forceinline__ void lossy_bounds(double sd0, double sd1, double m0, double m1, double std_factor, int variant, int low0,
                                              int high0, int* low_out, int* high_out)
 {
@@ -183,8 +204,8 @@ __device__ __forceinline__ void lossy_bounds(double sd0, double sd1, double m0, 
         dh = sd1 < m1 ? 0.0 : __dsub_rn(sd1, m1);
         dl = sd0 < m0 ? 0.0 : __dsub_rn(sd0, m0);
     }
-    int high = high0 - (int)round(__dmul_rn(dh, std_factor));
-    int low = low0 - (int)round(__dmul_rn(dl, std_factor));
+    int high = lossy_sub_rounded(high0, __dmul_rn(dh, std_factor));
+    int low = lossy_sub_rounded(low0, __dmul_rn(dl, std_factor));
     if (high < 0) high = 0;
     if (low < high) low = high;
     *low_out = low;
@@ -213,10 +234,10 @@ __device__ __forceinline__ void lossy_decide_body(LossyScalars* sc, int ns, int 
     if (quirk && nstds == 40) sc->stds[(head + 38) % 40][1] = win[38][1];
     double sd0, sd1;
     if (nstds < 40) {
-        const double s = (double)(sums[0] + sums[2]), s2 = (double)(sums[1] + sums[3]);
+        const double s = (double)(sums[0] + sums[2]), s2 = (double)(long long)(sums[1] + sums[3]);
         sd0 = sd1 = __ddiv_rn(__dsqrt_rn(__dsub_rn(__dmul_rn(s, s), s2)), (double)ns);
     } else {
-        const double s = (double)sums[0], s2 = (double)sums[1], b = (double)sums[2], b2 = (double)sums[3];
+        const double s = (double)sums[0], s2 = (double)(long long)sums[1], b = (double)sums[2], b2 = (double)(long long)sums[3];
         sd0 = __ddiv_rn(__dsqrt_rn(__dsub_rn(__dmul_rn(b, b), b2)), (double)(int)cnts[1]);
         sd1 = __ddiv_rn(__dsqrt_rn(__dsub_rn(__dmul_rn(s, s), s2)), (double)(int)cnts[0]);
     }
@@ -266,7 +287,7 @@ lossy_sums_kernel(const u16* __restrict__ prevT, const u16* __restrict__ tmpT, c
     unsigned nf = 0, nb = 0;
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < ns; i += gridDim.x * blockDim.x) {
         const int d = abs((int)tmpT[i] - (int)prevT[i]);
-        const unsigned long long d2 = (unsigned long long)d * (unsigned long long)d;
+        const unsigned long long d2 = lossy_wrapped_square(d);
         if ((unsigned)img[i] > back) {
             sd += d; sd2 += d2; ++nf;
         } else {
@@ -528,7 +549,7 @@ __global__ void __launch_bounds__(1024) lossy_run_kernel(const __grid_constant__
     unsigned nf = 0, nb = 0;
     auto add_pixel = [&](unsigned tv1, unsigned prev, bool fore) {
         const int d = abs((int)tv1 - (int)prev);
-        const unsigned long long d2 = (unsigned long long)d * (unsigned long long)d;
+        const unsigned long long d2 = lossy_wrapped_square(d);
         if (fore) {
             sd += d; sd2 += d2; ++nf;
         } else {
@@ -625,10 +646,10 @@ __global__ void __launch_bounds__(1024) lossy_run_kernel(const __grid_constant__
                 lossy_window_quirk(win, nstds, p.quirk);
                 double sd0, sd1;
                 if (nstds < 40) {
-                    const double s1 = (double)(su[0] + su[2]), s2 = (double)(su[1] + su[3]);
+                    const double s1 = (double)(su[0] + su[2]), s2 = (double)(long long)(su[1] + su[3]);
                     sd0 = sd1 = __ddiv_rn(__dsqrt_rn(__dsub_rn(__dmul_rn(s1, s1), s2)), (double)ns);
                 } else {
-                    const double s1 = (double)su[0], s2 = (double)su[1], b1 = (double)su[2], b2 = (double)su[3];
+                    const double s1 = (double)su[0], s2 = (double)(long long)su[1], b1 = (double)su[2], b2 = (double)(long long)su[3];
                     sd0 = __ddiv_rn(__dsqrt_rn(__dsub_rn(__dmul_rn(b1, b1), b2)), (double)(int)cn[1]);
                     sd1 = __ddiv_rn(__dsqrt_rn(__dsub_rn(__dmul_rn(s1, s1), s2)), (double)(int)cn[0]);
                 }

@@ -79,6 +79,26 @@ static int orc_clamp_value(int median, double gstd)
         return -1;
     return median - (int)v;
 }
+/* The lossy pre-conditioner's two constructs of the same class (h264.cpp:1993-2036 and :2367-2368 / :2559-2563), as
+ * g++ -O3 builds them for x86-64 (pinned by tests/test_lossy_extremes.py, which compiles the reference's statements):
+ * `diff * diff` on int wraps modulo 2^32 for |diff| >= 46341, and `lowError -= (int)round(x)` converts with cvttsd2si --
+ * the "integer indefinite" INT_MIN for NaN (an empty background / foreground split) and for values beyond int range --
+ * and then subtracts modulo 2^32. */
+static int orc_wrapped_square(int diff)
+{
+    return (int)(uint32_t)((unsigned)diff * (unsigned)diff);
+}
+static int orc_round_to_int(double x)
+{
+    double r = round(x);
+    if (!(r >= -2147483648.0 && r <= 2147483647.0))
+        return INT32_MIN;
+    return (int)r;
+}
+static int orc_wrapping_sub(int a, int b)
+{
+    return (int)((unsigned)a - (unsigned)b);
+}
 
 static void frame_median_std(const u16 *img, size_t n, int *median, double *std_out)
 {
@@ -630,6 +650,8 @@ typedef struct {
     int bp_enabled;
     int variant;                /* 0 = addImageLossyNoCamera (h264.cpp:2253-2424), 1 = addLoss (:2426-2607) */
     int memcpy_quirk;           /* 1 (default) = the compiled reference's overlapping-memcpy outcome, see orc_lossy_add_image */
+    int exact_squares;          /* 0 (default) = the reference's wrapping int product; 1 = exact squares (what it does not do) */
+    int saturating_round;       /* 0 (default) = x86's conversion; 1 = a saturating one with NaN -> 0 (what it does not do) */
     /* state */
     long frames;                /* m_data->attributes.size() */
     unsigned short minv;
@@ -665,6 +687,14 @@ ORC_API void orc_lossy_configure(orc_lossy *s, int variant, int memcpy_quirk)
     s->variant = variant;
     s->memcpy_quirk = memcpy_quirk;
 }
+/* Counterfactual arithmetic, for tests that show the reference's own makes a difference (like memcpy_quirk = 0):
+ * exact_squares = 1 adds exact squares in stdDev, saturating_round = 1 converts with saturation and NaN -> 0 in the
+ * bound update. */
+ORC_API void orc_lossy_counterfactual(orc_lossy *s, int exact_squares, int saturating_round)
+{
+    s->exact_squares = exact_squares;
+    s->saturating_round = saturating_round;
+}
 ORC_API void orc_lossy_close(orc_lossy *s)
 {
     if (!s) return;
@@ -672,14 +702,22 @@ ORC_API void orc_lossy_close(orc_lossy *s)
     free(s->sums); free(s->cvalue); free(s->ccount); free(s->bp_xy); free(s);
 }
 
-/* stdDev, h264.cpp:1993-2036: (first, second) = (background, foreground) spreads of |img - prev| */
-static void lossy_std_dev(const u16 *prev, const u16 *img, int n, const u16 *img_dl, const unsigned *back, double out[2])
+static double lossy_square(int diff, int exact)
+{
+    return exact ? (double)diff * (double)diff : (double)orc_wrapped_square(diff);
+}
+
+/* stdDev, h264.cpp:1993-2036: (first, second) = (background, foreground) spreads of |img - prev|.  Each int square is
+ * added into the double sums in pixel order, like the reference (orc_wrapped_square: the product wraps for
+ * |diff| >= 46341).  An empty side gives 0 / 0 = NaN. */
+static void lossy_std_dev(const u16 *prev, const u16 *img, int n, const u16 *img_dl, const unsigned *back, int exact,
+                          double out[2])
 {
     if (!back || !img_dl) {
         double sum_diff2 = 0, sum_diff = 0;
         for (int i = 0; i < n; ++i) {
             int diff = abs((int)img[i] - (int)prev[i]);
-            sum_diff2 += diff * diff; /* int product, like the reference (overflows for |diff| >= 46341: UB there) */
+            sum_diff2 += lossy_square(diff, exact);
             sum_diff += diff;
         }
         double res = sqrt((sum_diff * sum_diff - sum_diff2)) / n;
@@ -689,12 +727,50 @@ static void lossy_std_dev(const u16 *prev, const u16 *img, int n, const u16 *img
         int b_sum = 0, sum = 0;
         for (int i = 0; i < n; ++i) {
             int diff = abs((int)img[i] - (int)prev[i]);
-            if (img_dl[i] > *back) { sum_diff2 += diff * diff; sum_diff += diff; sum++; }
-            else { b_sum_diff2 += diff * diff; b_sum_diff += diff; b_sum++; }
+            if (img_dl[i] > *back) { sum_diff2 += lossy_square(diff, exact); sum_diff += diff; sum++; }
+            else { b_sum_diff2 += lossy_square(diff, exact); b_sum_diff += diff; b_sum++; }
         }
         out[0] = sqrt((b_sum_diff * b_sum_diff - b_sum_diff2)) / b_sum;
         out[1] = sqrt((sum_diff * sum_diff - sum_diff2)) / sum;
     }
+}
+/* stdDev as the tests call it: img_dl == NULL is the un-split form */
+ORC_API void orc_lossy_std_dev(const u16 *prev, const u16 *img, int n, const u16 *img_dl, unsigned back, double out[2])
+{
+    lossy_std_dev(prev, img, n, img_dl, img_dl ? &back : NULL, 0, out);
+}
+
+static int lossy_round(double x, int saturating)
+{
+    if (!saturating)
+        return orc_round_to_int(x);
+    double r = round(x);
+    return r != r ? 0 : r >= 2147483647.0 ? INT32_MAX : r <= -2147483648.0 ? INT32_MIN : (int)r;
+}
+
+/* The bound update of a frame (:2367-2376 in addImageLossyNoCamera, :2559-2567 in addLoss): errors = {low, high} in,
+ * the frame's {BackgroundError, ForegroundError} out. */
+static void lossy_bounds(int variant, int saturating, double sd0, double sd1, double mean0, double mean1, double std_factor,
+                         int errors[2])
+{
+    int lowError = errors[0], highError = errors[1];
+    double diff_high, diff_low;
+    if (variant == 0) { /* :2367-2368 */
+        diff_high = fabs(sd1 - mean1);
+        diff_low = fabs(sd0 - mean0);
+    } else { /* addLoss :2559-2563: only a spread ABOVE the running mean tightens the bound */
+        diff_high = sd1 < mean1 ? 0 : sd1 - mean1;
+        diff_low = sd0 < mean0 ? 0 : sd0 - mean0;
+    }
+    highError = orc_wrapping_sub(highError, lossy_round(diff_high * std_factor, saturating));
+    lowError = orc_wrapping_sub(lowError, lossy_round(diff_low * std_factor, saturating));
+    if (highError < 0) highError = 0;
+    if (lowError < highError) lowError = highError;
+    errors[0] = lowError; errors[1] = highError;
+}
+ORC_API void orc_lossy_bounds(int variant, double sd0, double sd1, double mean0, double mean1, double std_factor, int errors[2])
+{
+    lossy_bounds(variant, 0, sd0, sd1, mean0, mean1, std_factor, errors);
 }
 
 /* One frame in, one frame out (what addImageLossLess then receives).  errors[0] = BackgroundError
@@ -733,11 +809,10 @@ ORC_API void orc_lossy_add_image(orc_lossy *s, const u16 *img, u16 *out, int *er
     if (s->subtract_min)
         for (int i = 0; i < ns; ++i) s->tmpT[i] = (s->tmpT[i] < s->minv) ? 0 : (u16)(s->tmpT[i] - s->minv);
     unsigned background = orc_get_background(s->tmp, ns); /* :2331 */
-    int lowError = s->low_error, highError = s->high_error;
     double sd[2];
     const int running_average_frames = 40;
-    if (s->nstds < running_average_frames) lossy_std_dev(s->prevT, s->tmpT, ns, NULL, NULL, sd);
-    else lossy_std_dev(s->prevT, s->tmpT, ns, img, &background, sd);
+    if (s->nstds < running_average_frames) lossy_std_dev(s->prevT, s->tmpT, ns, NULL, NULL, s->exact_squares, sd);
+    else lossy_std_dev(s->prevT, s->tmpT, ns, img, &background, s->exact_squares, sd);
     if (!s->have_first) { s->first_std[0] = sd[0]; s->first_std[1] = sd[1]; s->have_first = 1; }
     if (s->nstds < running_average_frames) { s->stds[s->nstds][0] = sd[0]; s->stds[s->nstds][1] = sd[1]; s->nstds++; }
     else {
@@ -754,18 +829,9 @@ ORC_API void orc_lossy_add_image(orc_lossy *s, const u16 *img, u16 *out, int *er
     double mean0 = s->first_std[0], mean1 = s->first_std[1]; /* :2353-2365 */
     for (int i = 0; i < s->nstds; ++i) { mean0 += s->stds[i][0]; mean1 += s->stds[i][1]; }
     mean0 /= (s->nstds + 1); mean1 /= (s->nstds + 1);
-    if (s->variant == 0) { /* :2367-2368 */
-        highError -= (int)round(fabs(sd[1] - mean1) * s->std_factor);
-        lowError -= (int)round(fabs(sd[0] - mean0) * s->std_factor);
-    } else { /* addLoss :2559-2563: only a spread ABOVE the running mean tightens the bound */
-        double diff_high = sd[1] < mean1 ? 0 : sd[1] - mean1;
-        double diff_low = sd[0] < mean0 ? 0 : sd[0] - mean0;
-        highError -= (int)round(diff_high * s->std_factor);
-        lowError -= (int)round(diff_low * s->std_factor);
-    }
-    if (highError < 0) highError = 0;
-    if (lowError < highError) lowError = highError;
-    errors[0] = lowError; errors[1] = highError;
+    errors[0] = s->low_error; errors[1] = s->high_error;
+    lossy_bounds(s->variant, s->saturating_round, sd[0], sd[1], mean0, mean1, s->std_factor, errors);
+    const int lowError = errors[0], highError = errors[1];
     /* RunningAverage2::addImage :1560-1594 */
     const int ra = s->running_average;
     if (ra > 0) {

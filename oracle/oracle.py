@@ -217,9 +217,11 @@ class Port(_Base):
         return img
 
     def lossy_open(self, w, h, stop_h, low_error=6, high_error=2, std_factor=5.0, running_average=32, subtract_min=False,
-                   bp_enabled=False, variant=0, memcpy_quirk=True):
+                   bp_enabled=False, variant=0, memcpy_quirk=True, exact_squares=False, saturating_round=False):
         """H264_Saver::addImageLossyNoCamera state (h264.cpp:2253-2424; variant=1: addLoss, :2426-2607); returns an
-        opaque state for lossy_add.  memcpy_quirk: reproduce the compiled reference's overlapping memcpy (oracle.c)."""
+        opaque state for lossy_add.  memcpy_quirk: reproduce the compiled reference's overlapping memcpy (oracle.c).
+        exact_squares / saturating_round: arithmetic the reference does NOT have (exact squares in stdDev; a saturating
+        conversion with NaN -> 0 in the bound update), for tests that show its own arithmetic matters."""
         f = self.lib.orc_lossy_open
         f.restype = ct.c_void_p
         f.argtypes = [ct.c_int, ct.c_int, ct.c_int, ct.c_int, ct.c_int, ct.c_double, ct.c_int, ct.c_int, ct.c_int]
@@ -228,7 +230,31 @@ class Port(_Base):
         g.restype = None
         g.argtypes = [ct.c_void_p, ct.c_int, ct.c_int]
         g(st, int(variant), int(memcpy_quirk))
+        g = self.lib.orc_lossy_counterfactual
+        g.restype = None
+        g.argtypes = [ct.c_void_p, ct.c_int, ct.c_int]
+        g(st, int(exact_squares), int(saturating_round))
         return st
+
+    def lossy_std_dev(self, prev, img, img_dl=None, back=0):
+        """stdDev (h264.cpp:1993-2036) on flat arrays: (background, foreground) spreads; img_dl=None: un-split."""
+        prev, img = _c(prev, np.uint16).ravel(), _c(img, np.uint16).ravel()
+        dl = None if img_dl is None else _c(img_dl, np.uint16).ravel()
+        out = np.zeros(2, dtype=np.float64)
+        f = self.lib.orc_lossy_std_dev
+        f.restype = None
+        f.argtypes = [ct.c_void_p, ct.c_void_p, ct.c_int, ct.c_void_p, ct.c_uint, ct.c_void_p]
+        f(_p(prev), _p(img), img.size, None if dl is None else _p(dl), int(back), _p(out))
+        return float(out[0]), float(out[1])
+
+    def lossy_bounds(self, variant, sd0, sd1, mean0, mean1, std_factor, low_error, high_error):
+        """One frame's bound update (h264.cpp:2367-2376 / :2559-2567): returns (lowError, highError)."""
+        e = np.array([low_error, high_error], dtype=np.int32)
+        f = self.lib.orc_lossy_bounds
+        f.restype = None
+        f.argtypes = [ct.c_int, ct.c_double, ct.c_double, ct.c_double, ct.c_double, ct.c_double, ct.c_void_p]
+        f(int(variant), sd0, sd1, mean0, mean1, std_factor, _p(e))
+        return int(e[0]), int(e[1])
 
     def lossy_add(self, state, image):
         """One frame through the pre-conditioner: returns (frame handed to the lossless encoder, (lowError, highError))."""
