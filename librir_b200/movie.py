@@ -226,6 +226,10 @@ class FramePipeline:
         n = frames_host.shape[0]
         gop = self.cfg.gop
         sub = max(gop, sub_frames // gop * gop) if self.cfg.delta else sub_frames  # sub-chunks start on key frames
+        ns = len(self._e2e) if hasattr(self, "_e2e") else slots
+        if ns * sub > self.cfg.chunk_frames:  # each slot's window of the chunk buffers must hold a whole sub-chunk
+            raise RuntimeError(f"process_host: {ns} slots of {sub} frames do not fit the {self.cfg.chunk_frames}-frame chunk buffers; "
+                               "lower sub_frames or slots, or raise chunk_frames")
         if not hasattr(self, "_e2e"):
             h, w = self.cfg.height, self.cfg.width
             self._e2e = [dict(stream=torch.cuda.Stream(device=self.device),

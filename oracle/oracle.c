@@ -695,6 +695,11 @@ ORC_API void orc_lossy_counterfactual(orc_lossy *s, int exact_squares, int satur
     s->exact_squares = exact_squares;
     s->saturating_round = saturating_round;
 }
+/* MIN_T of a subtractMin state: the minimum of the first frame's lossy rows (0 before the first frame or without subtractMin) */
+ORC_API int orc_lossy_get_min(const orc_lossy *s)
+{
+    return (s->subtract_min && s->frames > 0) ? (int)s->minv : 0;
+}
 ORC_API void orc_lossy_close(orc_lossy *s)
 {
     if (!s) return;

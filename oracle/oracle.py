@@ -267,6 +267,13 @@ class Port(_Base):
         f(state, _p(img), _p(out), _p(err))
         return out, (int(err[0]), int(err[1]))
 
+    def lossy_get_min(self, state):
+        """MIN_T of a subtractMin state (what rirb_lossy_get_min reports)."""
+        f = self.lib.orc_lossy_get_min
+        f.restype = ct.c_int
+        f.argtypes = [ct.c_void_p]
+        return int(f(state))
+
     def lossy_close(self, state):
         f = self.lib.orc_lossy_close
         f.restype = None
