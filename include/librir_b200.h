@@ -101,6 +101,10 @@ RIRB_API const char* rirb_version(void);
 RIRB_API int rirb_set_parameter(const char* key, const char* value);
 
 /* ---- batches of frames (nframes dense frames back to back) ---- */
+/* Operands may be host (pageable, pinned or registered), managed or device memory.  Host operands are staged through
+ * separate device buffers; device and managed operands go to the kernels as they are, so an output that shares a byte
+ * with an input of the same call in device or managed memory is refused (-1), except where an entry documents in-place
+ * use and the two pointers are equal.  Outputs that overlap each other are refused in any memory. */
 
 /* translate on nframes frames; n_shifts == 1: one (dx[0],dy[0]) for all frames, n_shifts ==
  * nframes: per-frame shifts (registration).  dx/dy: host or device arrays of float. */
@@ -216,7 +220,8 @@ RIRB_API int rirb_lossy_get_min(int handle, int* min_value);
  * The movie is cut into sub-chunks of whole GOPs that rotate over three CUDA streams, so the upload of
  * one, the kernels of another and the download of a third overlap; pinned (page-locked) buffers make
  * the copies asynchronous, pageable ones work but serialise.  Returns when lo/hi (and smoothed) are
- * complete.  With delta != 0, first_frame must be a multiple of gop. */
+ * complete.  With delta != 0, first_frame must be a multiple of gop.  Any operand may also be device or managed memory.
+ * An output that overlaps an input or another output is refused (-1), whatever the kind of memory. */
 RIRB_API int rirb_process_movie_host(int handle, const unsigned short* frames, long long nframes, int w, int h, float sigma,
                                      const float* dx, const float* dy, const char* strategy, unsigned int background, int gop,
                                      int delta, long long first_frame, unsigned char* lo, unsigned char* hi, float* smoothed);

@@ -122,16 +122,7 @@ static int require_device()
     return 0;
 }
 
-static bool is_device_ptr(const void* p)
-{
-    if (!p) return false;
-    cudaPointerAttributes a;
-    if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
-        cudaGetLastError();
-        return false;
-    }
-    return a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged;
-}
+static bool is_device_ptr(const void* p) { return p && operand_on_device(p); }
 
 static void* scratch(int slot, size_t bytes)
 {
@@ -213,15 +204,7 @@ static bool pin_ready()
     return pin.state == 1;
 }
 
-static bool is_pageable(const void* p)
-{
-    cudaPointerAttributes a;
-    if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
-        cudaGetLastError();
-        return true;
-    }
-    return a.type == cudaMemoryTypeUnregistered;
-}
+static bool is_pageable(const void* p) { return operand_memory_type(p) == cudaMemoryTypeUnregistered; }
 
 // Uploads stay with the driver: its pageable host->device path already runs at the speed of one
 // host memcpy (~10 GB/s here), the ring was no faster at 640x512 and 20 % slower at 1280x1024.
@@ -500,12 +483,10 @@ int rirb_translate_batch(int type, const void* src, void* dst, int w, int h, lon
     }
     if (nframes == 0) return 0;
     RIRB_REQUIRE_DEVICE();
-    if (src == dst) {
-        set_error("translate: src and dst must not alias");
-        return -1;
-    }
-    cudaStream_t st = tls.stream;
     const size_t bytes = (size_t)w * h * esize * (size_t)nframes;
+    const size_t sbytes = sizeof(float) * (size_t)n_shifts;
+    if (refuse_overlap("translate", {{"src", src, bytes}, {"dx", dx, sbytes}, {"dy", dy, sbytes}}, {{"dst", dst, bytes}})) return -1;
+    cudaStream_t st = tls.stream;
     const void* d_src = stage_in(src, bytes, 0, st);
     if (!d_src) return -1;
     StagedOut out;
@@ -559,12 +540,9 @@ static int gaussian_any(const void* src, bool src_u16, float* dst, int w, int h,
     GaussTaps taps;
     if (gaussian_taps_host(sigma, &taps) != 0) return -1;
     RIRB_REQUIRE_DEVICE();
-    if ((const void*)src == (const void*)dst) {
-        set_error("gaussian_filter: src and dst must not alias");
-        return -1;
-    }
-    cudaStream_t st = tls.stream;
     const size_t npx = (size_t)w * h * (size_t)nframes;
+    if (refuse_overlap("gaussian_filter", {{"src", src, npx * (src_u16 ? 2 : 4)}}, {{"dst", dst, npx * 4}})) return -1;
+    cudaStream_t st = tls.stream;
     const void* d_src = stage_in(src, npx * (src_u16 ? 2 : 4), 0, st);
     if (!d_src) return -1;
     StagedOut out;
@@ -740,6 +718,7 @@ int rirb_bad_pixels_correct_batch(int handle, const unsigned short* in, unsigned
     cudaStream_t st = tls.stream;
     const size_t fpx = (size_t)s->w * s->h;
     const size_t bytes = fpx * 2 * (size_t)nframes;
+    if (in != out && refuse_overlap("bad_pixels_correct", {{"in", in, bytes}}, {{"out", out, bytes}})) return -1;
     if (in == out) {  // sequential in-place meaning of the reference (BadPixels.cpp:41-59)
         StagedOut io;
         if (!stage_out(io, out, bytes, 0, true, st)) return -1;
@@ -764,8 +743,8 @@ int rirb_bad_pixels_correct_gaussian_batch(int handle, const unsigned short* in,
 {
     auto s = find_handle_here(handle, "bad_pixels_correct_gaussian");
     if (!s) return -1;
-    if (!in || !corrected || !smoothed || nframes < 0 || in == corrected) {
-        set_error("bad_pixels_correct_gaussian: bad arguments (in-place correction is not supported here)");
+    if (!in || !corrected || !smoothed || nframes < 0) {
+        set_error("bad_pixels_correct_gaussian: bad arguments");
         return -1;
     }
     if (nframes == 0) return 0;
@@ -774,6 +753,11 @@ int rirb_bad_pixels_correct_gaussian_batch(int handle, const unsigned short* in,
     RIRB_REQUIRE_DEVICE();
     cudaStream_t st = tls.stream;
     const size_t fpx = (size_t)s->w * s->h;
+    // in place is not supported here: the filter reads corrected pixels of neighbouring rows that the correction of other
+    // blocks may not have written yet
+    if (refuse_overlap("bad_pixels_correct_gaussian", {{"in", in, fpx * 2 * (size_t)nframes}},
+                       {{"corrected", corrected, fpx * 2 * (size_t)nframes}, {"smoothed", smoothed, fpx * 4 * (size_t)nframes}}))
+        return -1;
     const u16* d_in = (const u16*)stage_in(in, fpx * 2 * (size_t)nframes, 0, st);
     if (!d_in) return -1;
     StagedOut o[2];
@@ -857,6 +841,8 @@ int rirb_loader_remove_motion(const unsigned short* in, unsigned short* out, int
     }
     if (nframes == 0) return 0;
     RIRB_REQUIRE_DEVICE();
+    const size_t bytes = frame_stride * 2 * (size_t)nframes;
+    if (in != out && refuse_overlap("remove_motion", {{"in", in, bytes}}, {{"out", out, bytes}})) return -1;
     cudaStream_t st = tls.stream;
     // shifts: doubles on the host (PointF), negated and narrowed to float as the reference's call does
     std::vector<double> sx((size_t)nframes), sy((size_t)nframes);
@@ -876,7 +862,6 @@ int rirb_loader_remove_motion(const unsigned short* in, unsigned short* out, int
     const float* d_dx = (const float*)stage_in(fx.data(), sizeof(float) * nframes, 2, st);
     const float* d_dy = (const float*)stage_in(fy.data(), sizeof(float) * nframes, 3, st);
     if (!d_dx || !d_dy) return -1;
-    const size_t bytes = frame_stride * 2 * (size_t)nframes;
     const bool inplace = (in == out);
     const u16* d_in;
     StagedOut o;
@@ -933,6 +918,7 @@ int rirb_loader_read_movie(int handle, const unsigned char* lo, const unsigned c
     cudaStream_t st = tls.stream;
     const size_t fpx = (size_t)w * h;
     const size_t pbytes = fpx * (size_t)nframes;
+    if (refuse_overlap("loader_read_movie", {{"lo", lo, pbytes}, {"hi", hi, pbytes}}, {{"out", out, pbytes * 2}})) return -1;
     const u8* d_lo = (const u8*)stage_in(lo, pbytes, 0, st);
     const u8* d_hi = (const u8*)stage_in(hi, pbytes, 1, st);
     if (!d_lo || !d_hi) return -1;
@@ -1047,6 +1033,9 @@ int rirb_split_yuv444(const unsigned short* img, const unsigned char* it, int w,
         return -1;
     }
     RIRB_REQUIRE_DEVICE();
+    if (refuse_overlap("split_yuv444", {{"img", img, (size_t)w * h * 2}, {"it", it, (size_t)w * h}},
+                       {{"y_plane", y_plane, (size_t)ls_y * h}, {"u_plane", u_plane, (size_t)ls_u * h}, {"v_plane", v_plane, (size_t)ls_v * h}}))
+        return -1;
     cudaStream_t st = tls.stream;
     const u16* d_img = (const u16*)stage_in(img, (size_t)w * h * 2, 0, st);
     if (!d_img) return -1;
@@ -1072,6 +1061,10 @@ int rirb_merge_yuv444(const unsigned char* y_plane, const unsigned char* u_plane
         return -1;
     }
     RIRB_REQUIRE_DEVICE();
+    if (refuse_overlap("merge_yuv444",
+                       {{"y_plane", it ? y_plane : nullptr, (size_t)ls_y * h}, {"u_plane", u_plane, (size_t)ls_u * h}, {"v_plane", v_plane, (size_t)ls_v * h}},
+                       {{"img", img, (size_t)w * h * 2}, {"it", y_plane ? it : nullptr, (size_t)w * h}}))
+        return -1;
     cudaStream_t st = tls.stream;
     const u8* d_u = (const u8*)stage_in(u_plane, (size_t)ls_u * h, 0, st);
     const u8* d_v = (const u8*)stage_in(v_plane, (size_t)ls_v * h, 1, st);
@@ -1096,10 +1089,13 @@ int rirb_split_yuv420(const unsigned short* img, const unsigned char* it, int w,
         return -1;
     }
     RIRB_REQUIRE_DEVICE();
+    const bool with_it = it && u_plane;
+    if (refuse_overlap("split_yuv420", {{"img", img, (size_t)w * h * 2}, {"it", with_it ? it : nullptr, (size_t)w * h}},
+                       {{"y_plane", y_plane, (size_t)ls_y * 2 * h}, {"u_plane", with_it ? u_plane : nullptr, (size_t)ls_u * h}}))
+        return -1;
     cudaStream_t st = tls.stream;
     const u16* d_img = (const u16*)stage_in(img, (size_t)w * h * 2, 0, st);
     if (!d_img) return -1;
-    const bool with_it = it && u_plane;
     const u8* d_it = nullptr;
     if (with_it) {
         d_it = (const u8*)stage_in(it, (size_t)w * h, 1, st);
@@ -1123,10 +1119,13 @@ int rirb_merge_yuv420(const unsigned char* y_plane, int ls_y, const unsigned cha
         return -1;
     }
     RIRB_REQUIRE_DEVICE();
+    const bool with_it = it && u_plane;
+    if (refuse_overlap("merge_yuv420", {{"y_plane", y_plane, (size_t)ls_y * 2 * h}, {"u_plane", with_it ? u_plane : nullptr, (size_t)ls_u * h}},
+                       {{"img", img, (size_t)w * h * 2}, {"it", with_it ? it : nullptr, (size_t)w * h}}))
+        return -1;
     cudaStream_t st = tls.stream;
     const u8* d_yp = (const u8*)stage_in(y_plane, (size_t)ls_y * 2 * h, 0, st);
     if (!d_yp) return -1;
-    const bool with_it = it && u_plane;
     const u8* d_up = nullptr;
     if (with_it) {
         d_up = (const u8*)stage_in(u_plane, (size_t)ls_u * h, 1, st);
@@ -1151,6 +1150,7 @@ int rirb_precode_movie(const unsigned short* movie, long long nframes, int w, in
     RIRB_REQUIRE_DEVICE();
     cudaStream_t st = tls.stream;
     const size_t n = (size_t)w * h * (size_t)nframes;
+    if (refuse_overlap("precode_movie", {{"movie", movie, n * 2}}, {{"lo", lo, n}, {"hi", hi, n}})) return -1;
     const u16* d_mov = (const u16*)stage_in(movie, n * 2, 0, st);
     if (!d_mov) return -1;
     StagedOut o[2];
@@ -1170,6 +1170,9 @@ int rirb_precode_movie_stats(const unsigned short* movie, long long nframes, int
     RIRB_REQUIRE_DEVICE();
     cudaStream_t st = tls.stream;
     const size_t n = (size_t)w * h * (size_t)nframes;
+    if (refuse_overlap("precode_movie_stats", {{"movie", movie, n * 2}},
+                       {{"lo", lo, n}, {"hi", hi, n}, {"minmax", minmax, 2 * sizeof(unsigned)}, {"hist", hist, 65536 * sizeof(unsigned long long)}}))
+        return -1;
     const u16* d_mov = (const u16*)stage_in(movie, n * 2, 0, st);
     if (!d_mov) return -1;
     StagedOut o[4];
@@ -1198,6 +1201,7 @@ int rirb_decode_movie(const unsigned char* lo, const unsigned char* hi, long lon
     RIRB_REQUIRE_DEVICE();
     cudaStream_t st = tls.stream;
     const size_t n = (size_t)w * h * (size_t)nframes;
+    if (refuse_overlap("decode_movie", {{"lo", lo, n}, {"hi", hi, n}}, {{"movie", movie, n * 2}})) return -1;
     const u8* d_lo = (const u8*)stage_in(lo, n, 0, st);
     const u8* d_hi = (const u8*)stage_in(hi, n, 1, st);
     if (!d_lo || !d_hi) return -1;
@@ -1386,6 +1390,8 @@ int rirb_lossy_add_images(int handle, const unsigned short* frames, long long nf
     cudaStream_t st = tls.stream;
     const int w = s->w, h = s->h, n = w * h, ns = w * s->stop_h;
     const size_t bytes = (size_t)n * 2 * (size_t)nframes;
+    if (refuse_overlap("lossy_add_images", {{"frames", frames, bytes}}, {{"out", out, bytes}, {"errors", errors, sizeof(int) * 2 * (size_t)nframes}}))
+        return -1;
     const u16* d_in = (const u16*)stage_in(frames, bytes, 0, st);
     if (!d_in) return -1;
     StagedOut o;
@@ -1524,6 +1530,21 @@ int rirb_process_movie_host(int handle, const unsigned short* frames, long long 
     if (gaussian_taps_host(sigma, &taps) != 0) return -1;
     RIRB_REQUIRE_DEVICE();
     const size_t fpx = (size_t)w * h;
+    // every operand is host memory read and written by copies on three streams at once: an output that overlaps an input
+    // races with the upload of a later sub-chunk whatever the kind of memory, so refuse_overlap's device-only rule for
+    // inputs does not apply
+    {
+        const size_t n = fpx * (size_t)nframes;
+        const Operand ins[] = {{"frames", frames, n * 2}, {"dx", dx, 4 * (size_t)nframes}, {"dy", dy, 4 * (size_t)nframes}};
+        const Operand outs[] = {{"lo", lo, n}, {"hi", hi, n}, {"smoothed", smoothed, n * 4}};
+        for (const Operand& o : outs)
+            for (const Operand& i : ins)
+                if (bytes_overlap(o, i)) {
+                    set_error("process_movie_host: %s and %s overlap", i.name, o.name);
+                    return -1;
+                }
+        if (refuse_overlap("process_movie_host", {}, {outs[0], outs[1], outs[2]})) return -1;
+    }
     // sub-chunk: whole GOPs, about 64 MB of input (RIRB_HOST_SUB_BYTES overrides the size: tests use it to make
     // small movies rotate through all the slots)
     long long sub_bytes = 64ll << 20;
@@ -1582,9 +1603,9 @@ int rirb_process_movie_host(int handle, const unsigned short* frames, long long 
             rc = -1;
             return false;
         };
-        if (!ok(cudaMemcpyAsync(d_in, frames + a * fpx, fpx * 2 * m, cudaMemcpyHostToDevice, st), "upload of the frames") ||
-            !ok(cudaMemcpyAsync(d_dx, dx + a, 4 * m, cudaMemcpyHostToDevice, st), "upload of the shifts") ||
-            !ok(cudaMemcpyAsync(d_dy, dy + a, 4 * m, cudaMemcpyHostToDevice, st), "upload of the shifts"))
+        if (!ok(cudaMemcpyAsync(d_in, frames + a * fpx, fpx * 2 * m, cudaMemcpyDefault, st), "upload of the frames") ||
+            !ok(cudaMemcpyAsync(d_dx, dx + a, 4 * m, cudaMemcpyDefault, st), "upload of the shifts") ||
+            !ok(cudaMemcpyAsync(d_dy, dy + a, 4 * m, cudaMemcpyDefault, st), "upload of the shifts"))
             break;
         if (launch_bp_correct(d_in, d_cor, s->xy_dev, s->span_off_dev, w, h, s->clamp_value, m, fpx, st) != 0 ||
             launch_gaussian_u16(d_cor, d_sm, w, h, m, taps, st) != 0 ||
@@ -1593,9 +1614,9 @@ int rirb_process_movie_host(int handle, const unsigned short* frames, long long 
             rc = -1;
             break;
         }
-        if (!ok(cudaMemcpyAsync(lo + a * fpx, d_lo, fpx * m, cudaMemcpyDeviceToHost, st), "download of the low-byte planes") ||
-            !ok(cudaMemcpyAsync(hi + a * fpx, d_hi, fpx * m, cudaMemcpyDeviceToHost, st), "download of the high-byte planes") ||
-            (smoothed && !ok(cudaMemcpyAsync(smoothed + a * fpx, d_sm, fpx * 4 * m, cudaMemcpyDeviceToHost, st), "download of the smoothed frames")))
+        if (!ok(cudaMemcpyAsync(lo + a * fpx, d_lo, fpx * m, cudaMemcpyDefault, st), "download of the low-byte planes") ||
+            !ok(cudaMemcpyAsync(hi + a * fpx, d_hi, fpx * m, cudaMemcpyDefault, st), "download of the high-byte planes") ||
+            (smoothed && !ok(cudaMemcpyAsync(smoothed + a * fpx, d_sm, fpx * 4 * m, cudaMemcpyDefault, st), "download of the smoothed frames")))
             break;
     }
     for (int q = 0; q < HP_SLOTS; ++q) {
@@ -1626,6 +1647,9 @@ int rirb_movie_stats(const unsigned short* pixels, size_t n, unsigned int* minma
         return -1;
     }
     RIRB_REQUIRE_DEVICE();
+    if (refuse_overlap("movie_stats", {{"pixels", pixels, n * 2}},
+                       {{"minmax", minmax, 2 * sizeof(unsigned)}, {"hist", hist, 65536 * sizeof(unsigned long long)}}))
+        return -1;
     cudaStream_t st = tls.stream;
     const u16* d_p = (const u16*)stage_in(pixels, n * 2, 0, st);
     if (!d_p) return -1;

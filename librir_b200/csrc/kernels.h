@@ -5,6 +5,8 @@
 #include <cuda_runtime.h>
 #include <stddef.h>
 
+#include <initializer_list>
+
 namespace rirb {
 
 typedef unsigned short u16;
@@ -65,6 +67,65 @@ int launch_gaussian_bp_u16(const u16* raw, u16* corrected, float* dst, int w, in
 
 // capi.cu: grow-only per-thread device work space for launchers, slots 8..11 (nullptr + set_error when out of memory)
 void* scratch_buffer(int slot, size_t bytes);
+
+// The operand checks of the entries, defined here so that every source file that has an entry carries them (the host
+// build of zdecoder.cu in the tests included).  A kernel that writes bytes it (or another kernel of the same call) also
+// reads races, so refuse_overlap fails (-1, set_error naming both operands) when an output shares a byte with an input --
+// both device or managed memory; host operands are staged into separate buffers -- or with another output, in any
+// memory.  Inputs may share bytes: they are only read.
+void set_error(const char* fmt, ...);
+struct Operand {
+    const char* name;
+    const void* p;
+    size_t bytes;
+};
+inline bool bytes_overlap(const Operand& a, const Operand& b)
+{
+    const size_t x = (size_t)a.p, y = (size_t)b.p;
+    return a.p && b.p && a.bytes && b.bytes && x < y + b.bytes && y < x + a.bytes;
+}
+// cudaMemoryTypeUnregistered (pageable host memory) when the runtime does not know the pointer
+inline cudaMemoryType operand_memory_type(const void* p)
+{
+    cudaPointerAttributes a;
+    if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
+        cudaGetLastError();
+        return cudaMemoryTypeUnregistered;
+    }
+    return a.type;
+}
+inline bool operand_on_device(const void* p)
+{
+    const cudaMemoryType t = operand_memory_type(p);
+    return t == cudaMemoryTypeDevice || t == cudaMemoryTypeManaged;
+}
+inline int refuse_overlap(const char* what, std::initializer_list<Operand> ins, std::initializer_list<Operand> outs)
+{
+    for (auto o = outs.begin(); o != outs.end(); ++o) {
+        for (const Operand& i : ins)
+            if (bytes_overlap(*o, i) && operand_on_device(o->p) && operand_on_device(i.p)) {
+                set_error("%s: %s and %s overlap in device memory", what, i.name, o->name);
+                return -1;
+            }
+        for (auto q = outs.begin(); q != o; ++q)
+            if (bytes_overlap(*o, *q)) {
+                set_error("%s: the outputs %s and %s overlap", what, q->name, o->name);
+                return -1;
+            }
+    }
+    return 0;
+}
+// -1 (set_error naming the operand) unless every non-null pointer is device, managed or page-locked host memory: what a
+// kernel may dereference directly
+inline int refuse_pageable(const char* what, std::initializer_list<Operand> ops)
+{
+    for (const Operand& o : ops)
+        if (o.p && operand_memory_type(o.p) == cudaMemoryTypeUnregistered) {
+            set_error("%s: %s is pageable host memory; pass device, managed or pinned memory", what, o.name);
+            return -1;
+        }
+    return 0;
+}
 
 // precode.cu
 int launch_split_planes(const u16* img, const u8* it, int w, int h, u8* y_plane, u8* u_plane, u8* v_plane, int ls_y, int ls_u,

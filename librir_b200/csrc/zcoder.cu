@@ -1014,6 +1014,10 @@ static int encode_batch(bool lz, const unsigned char* src, long long n, long lon
         set_error("%s: no CUDA device (the coder is a CUDA kernel; no CPU fallback)", name);
         return -1;
     }
+    if (refuse_pageable(name, {{"src", src, 0}, {"dst", dst, 0}, {"sizes", sizes, 0}}) ||
+        refuse_overlap(name, {{"src", src, (size_t)n * (size_t)bytes_each}},
+                       {{"dst", dst, (size_t)n * (size_t)dst_stride}, {"sizes", sizes, sizeof(long long) * (size_t)n}}))
+        return -1;
     cudaStream_t st = current_stream();
     void* scratch = nullptr;
     RIRB_CUDA_OK(cudaMallocAsync(&scratch, lz ? zcoder_lz_scratch_bytes(n, bytes_each, segment) : zcoder_scratch_bytes(n, bytes_each, segment), st));

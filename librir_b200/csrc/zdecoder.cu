@@ -894,6 +894,11 @@ extern "C" int rirb_zstd_decode_batch(const unsigned char* src, const long long*
         return -1;
     }
     if (n == 0) return 0;
+    // the extent of src is in the device-resident offsets / sizes, so src is not part of the overlap check
+    if (refuse_pageable("zstd_decode_batch", {{"src", src, 0}, {"offsets", offsets, 0}, {"sizes", sizes, 0}, {"dst", dst, 0}, {"status", status, 0}}) ||
+        refuse_overlap("zstd_decode_batch", {{"offsets", offsets, sizeof(long long) * (size_t)n}, {"sizes", sizes, sizeof(unsigned) * (size_t)n}},
+                       {{"dst", dst, (size_t)n * (size_t)dst_stride}, {"status", status, sizeof(long long) * (size_t)n}}))
+        return -1;
     cudaStream_t st = current_stream();
     void* scratch = nullptr;
     RIRB_CUDA_OK(cudaMallocAsync(&scratch, zdecoder_scratch_bytes(n, dst_capacity), st));

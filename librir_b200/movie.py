@@ -87,6 +87,7 @@ class MovieStats:
         """Fold a chunk of uint16 frames (torch CUDA tensor) into the statistics."""
         lib = _lib.load()
         sp._prepare_device_call(frames)
+        frames = sp._operand(frames, "movie_stats", "frames", dtype=np.uint16, copy=True)
         n = frames.numel()
         if self._fresh:
             self._sums[65536] = 0
@@ -275,24 +276,33 @@ def process_movie_host(bad_pixels, frames, dx, dy, sigma=1.0, strategy="nearest"
     """The whole per-frame path on HOST buffers through ONE C-ABI call (``rirb_process_movie_host``):
     ``frames`` uint16 ``[n, h, w]`` (numpy array or CPU torch tensor, ideally pinned) -> ``(lo, hi)`` uint8
     byte planes of the corrected, registered, pre-coded frames.  ``smoothed``: optional float32 ``[n, h, w]``
-    host buffer for the Gaussian output (otherwise it stays on the device)."""
+    host buffer for the Gaussian output (otherwise it stays on the device).  ``lo`` / ``hi``: uint8 of ``frames``' shape.
+    A strided numpy ``frames`` is copied first; strided outputs are refused."""
     lib = _lib.load()
+    what = "process_movie_host"
 
     def host_ptr(x):
-        if sp._is_torch(x):
-            if x.is_cuda or not x.is_contiguous():
-                raise RuntimeError("process_movie_host: contiguous host buffers expected")
-            return ct.c_void_p(x.data_ptr())
-        return x.ctypes.data_as(ct.c_void_p)
+        if sp._is_torch(x) and x.is_cuda:
+            raise RuntimeError("process_movie_host: contiguous host buffers expected")
+        return sp._ptr(x)
 
+    if len(frames.shape) != 3:
+        raise RuntimeError("process_movie_host: wrong input dimension")
+    frames = sp._operand(frames, what, "frames", dtype=np.uint16, copy=True)
     n, h, w = frames.shape
     if lo is None:
         lo = np.empty((n, h, w), np.uint8)
     if hi is None:
         hi = np.empty((n, h, w), np.uint8)
+    lo = sp._operand(lo, what, "lo", frames.shape, np.uint8)
+    hi = sp._operand(hi, what, "hi", frames.shape, np.uint8)
+    if smoothed is not None:
+        smoothed = sp._operand(smoothed, what, "smoothed", frames.shape, np.float32)
     if not sp._is_torch(dx):
         dx = np.ascontiguousarray(np.broadcast_to(np.asarray(dx, dtype=np.float32), (n,)))
         dy = np.ascontiguousarray(np.broadcast_to(np.asarray(dy, dtype=np.float32), (n,)))
+    dx = sp._operand(dx, what, "dx", (n,), np.float32, copy=True)
+    dy = sp._operand(dy, what, "dy", (n,), np.float32, copy=True)
     r = lib.rirb_process_movie_host(bad_pixels.handle, host_ptr(frames), n, w, h, float(sigma), host_ptr(dx), host_ptr(dy),
                                     sp.toCharP(strategy), int(background), int(gop), int(bool(delta)), int(first_frame),
                                     host_ptr(lo), host_ptr(hi), host_ptr(smoothed) if smoothed is not None else None)

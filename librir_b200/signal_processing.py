@@ -44,15 +44,20 @@ def _is_torch(x) -> bool:
     return type(x).__module__.startswith("torch")
 
 
-def _torch_np_dtype(t):
-    import torch
+_TORCH_NP_DTYPES = {}  # filled on first use: every operand check of a torch tensor looks its dtype up here
 
-    return {
-        torch.bool: np.dtype(np.bool_), torch.int8: np.dtype(np.int8), torch.uint8: np.dtype(np.uint8),
-        torch.int16: np.dtype(np.int16), torch.uint16: np.dtype(np.uint16), torch.int32: np.dtype(np.int32),
-        torch.uint32: np.dtype(np.uint32), torch.int64: np.dtype(np.int64), torch.uint64: np.dtype(np.uint64),
-        torch.float32: np.dtype(np.float32), torch.float64: np.dtype(np.float64),
-    }[t.dtype]
+
+def _torch_np_dtype(t):
+    if not _TORCH_NP_DTYPES:
+        import torch
+
+        _TORCH_NP_DTYPES.update({
+            torch.bool: np.dtype(np.bool_), torch.int8: np.dtype(np.int8), torch.uint8: np.dtype(np.uint8),
+            torch.int16: np.dtype(np.int16), torch.uint16: np.dtype(np.uint16), torch.int32: np.dtype(np.int32),
+            torch.uint32: np.dtype(np.uint32), torch.int64: np.dtype(np.int64), torch.uint64: np.dtype(np.uint64),
+            torch.float32: np.dtype(np.float32), torch.float64: np.dtype(np.float64),
+        })
+    return _TORCH_NP_DTYPES[t.dtype]
 
 
 def _ptr(x):
@@ -60,11 +65,41 @@ def _ptr(x):
         if not x.is_contiguous():
             raise RuntimeError("librir_b200: tensors must be contiguous")
         return ct.c_void_p(x.data_ptr())
+    if not x.flags.c_contiguous:  # the library reads and writes dense buffers from the first element's address
+        raise RuntimeError("librir_b200: arrays must be contiguous")
     return x.ctypes.data_as(ct.c_void_p)
 
 
 def _dtype_of(x):
     return _torch_np_dtype(x) if _is_torch(x) else x.dtype
+
+
+def _operand(x, what, name, shape=None, dtype=None, copy=False):
+    """Check an array operand of ``what`` before its pointer goes to the library, which trusts the pointer for the whole
+    extent the call implies: ``dtype`` and ``shape`` (None: any) must match exactly, and the buffer must be dense.  A
+    strided numpy input is copied when ``copy`` (operands the library only reads); otherwise -- outputs, in-place
+    operands, torch tensors -- it is refused, as is a read-only numpy output.  ``dtype`` may be a tuple of the dtypes
+    accepted.  Returns the operand to hand to ``_ptr``."""
+    try:
+        dt = _dtype_of(x)
+    except KeyError:  # a torch dtype the library has no code for
+        dt = None
+    allowed = [np.dtype(d) for d in (dtype if isinstance(dtype, tuple) else (dtype,))] if dtype is not None else None
+    if allowed is not None and dt not in allowed:
+        raise RuntimeError(f"{what}: {name} must be {' or '.join(d.name for d in allowed)}, not {x.dtype}")
+    if shape is not None and tuple(x.shape) != tuple(shape):
+        raise RuntimeError(f"{what}: {name} has shape {tuple(x.shape)}, expected {tuple(shape)}")
+    if _is_torch(x):
+        if not x.is_contiguous():
+            raise RuntimeError(f"{what}: {name} must be a contiguous tensor")
+        return x
+    if not x.flags.c_contiguous:
+        if not copy:
+            raise RuntimeError(f"{what}: {name} is a strided view; the library writes it as a dense array")
+        x = np.ascontiguousarray(x)
+    elif not copy and not x.flags.writeable:
+        raise RuntimeError(f"{what}: {name} is read-only")
+    return x
 
 
 def _empty_like(x, dtype=None):
@@ -123,7 +158,8 @@ def translate(image, dx, dy, strategy=str(), background=None):
 
 
 def translate_batch(frames, dx, dy, strategy=str(), background=None, out=None):
-    """``translate`` on a stack ``[n, h, w]``; ``dx``/``dy`` scalars or per-frame sequences."""
+    """``translate`` on a stack ``[n, h, w]``; ``dx``/``dy`` scalars or per-frame sequences.  ``out``: same shape and dtype
+    as ``frames``.  A strided numpy ``frames`` is copied first; a strided ``out`` is refused."""
     lib = _lib.load()
     if len(frames.shape) != 3:
         raise RuntimeError("translate_batch: wrong input dimension")
@@ -133,6 +169,7 @@ def translate_batch(frames, dx, dy, strategy=str(), background=None, out=None):
     if strategy == b"constant":
         strategy = b"background"
     _prepare_device_call(frames)
+    frames = _operand(frames, "translate_batch", "frames", copy=True)
     n, h, w = frames.shape
     dt = _dtype_of(frames)
     code = _DTYPES.get(dt)
@@ -140,8 +177,13 @@ def translate_batch(frames, dx, dy, strategy=str(), background=None, out=None):
         raise RuntimeError("An error occured while calling 'translate'")
     if out is None:
         out = frames.clone() if _is_torch(frames) else np.copy(frames, "C")
+    out = _operand(out, "translate_batch", "out", frames.shape, dt)
     if _is_torch(dx):
-        sx, sy, ns = dx, dy, dx.numel()
+        ns = dx.numel()
+        sx = _operand(dx, "translate_batch", "dx", (ns,) if ns != 1 else None, np.float32)
+        sy = _operand(dy, "translate_batch", "dy", tuple(dx.shape), np.float32)
+        if ns not in (1, n):
+            raise RuntimeError(f"translate_batch: dx has {ns} shifts for {n} frames")
     else:
         sx = np.ascontiguousarray(np.atleast_1d(dx), dtype=np.float32)
         sy = np.ascontiguousarray(np.atleast_1d(dy), dtype=np.float32)
@@ -177,15 +219,18 @@ def gaussian_filter(image, sigma=1.0):
 
 
 def gaussian_filter_batch(frames, sigma=1.0, out=None):
-    """Gaussian filter of a stack ``[n, h, w]`` (float32, or uint16 converted on the fly)."""
+    """Gaussian filter of a stack ``[n, h, w]`` (float32, or uint16 converted on the fly) into float32 ``out`` of the same
+    shape.  A strided numpy ``frames`` is copied first; a strided ``out`` is refused."""
     lib = _lib.load()
     if len(frames.shape) != 3:
         raise RuntimeError("gaussian_filter_batch: wrong input dimension")
     _prepare_device_call(frames)
+    frames = _operand(frames, "gaussian_filter_batch", "frames", copy=True)
     n, h, w = frames.shape
     dt = _dtype_of(frames)
     if out is None:
         out = _empty_like(frames, np.float32)
+    out = _operand(out, "gaussian_filter_batch", "out", frames.shape, np.float32)
     if dt == np.uint16:
         r = lib.rirb_gaussian_filter_u16_batch(_ptr(frames), _ptr(out), w, h, n, sigma)
     elif dt == np.float32:
@@ -226,23 +271,41 @@ def bad_pixels_create(first_image):
         img = first_image
     else:
         img = np.array(first_image, dtype=np.uint16, order="C")
+    img = _operand(img, "bad_pixels_create", "first_image", dtype=np.uint16, copy=True)
+    if len(img.shape) != 2:
+        raise RuntimeError("bad_pixels_create: wrong input image dimension")
     ret = lib.bad_pixels_create(_ptr(img), img.shape[1], img.shape[0])
     if ret <= 0:
         raise RuntimeError(f"'bad_pixels_create': {_lib.last_error()}")
+    _BP_SHAPES[ret] = tuple(img.shape)
     return ret
+
+
+_BP_SHAPES = {}  # handle -> (h, w) of the image it was created on: the frame size the batch calls read and write
+
+
+def _bp_frames(handle, frames, what, copy=True):
+    """``frames`` of a batch call on a bad-pixel handle: uint16 ``[n, h, w]`` with the handle's ``(h, w)``."""
+    hw = _BP_SHAPES.get(handle)
+    if len(frames.shape) != 3:
+        raise RuntimeError(f"{what}: wrong input dimension")
+    return _operand(frames, what, "frames", (frames.shape[0],) + hw if hw else None, np.uint16, copy=copy)
 
 
 def bad_pixels_correct_gaussian_batch(handle, frames, sigma=1.0, out=None, smoothed=None):
     """``bad_pixels_correct_batch`` followed by ``gaussian_filter_batch`` of the corrected frames, in one pass over the
-    movie: returns ``(corrected uint16 [n,h,w], smoothed float32 [n,h,w])``."""
+    movie: returns ``(corrected uint16 [n,h,w], smoothed float32 [n,h,w])``.  A strided numpy ``frames`` is copied
+    first; a strided ``out`` or ``smoothed`` is refused."""
     lib = _lib.load()
-    if len(frames.shape) != 3:
-        raise RuntimeError("bad_pixels_correct_gaussian_batch: wrong input dimension")
     _prepare_device_call(frames)
+    what = "bad_pixels_correct_gaussian_batch"
+    frames = _bp_frames(handle, frames, what)
     if out is None:
         out = _empty_like(frames)
     if smoothed is None:
         smoothed = _empty_like(frames, np.float32)
+    out = _operand(out, what, "out", frames.shape, np.uint16)
+    smoothed = _operand(smoothed, what, "smoothed", frames.shape, np.float32)
     res = lib.rirb_bad_pixels_correct_gaussian_batch(handle, _ptr(frames), _ptr(out), _ptr(smoothed), frames.shape[0], float(sigma))
     _lib.check(res, "bad_pixels_correct_gaussian")
     return out, smoothed
@@ -251,6 +314,7 @@ def bad_pixels_correct_gaussian_batch(handle, frames, sigma=1.0, out=None, smoot
 def bad_pixels_destroy(handle):
     """Release a handle obtained from ``bad_pixels_create``."""
     _lib.load().bad_pixels_destroy(handle)
+    _BP_SHAPES.pop(handle, None)
 
 
 def bad_pixels_correct(handle, img):
@@ -265,13 +329,15 @@ def bad_pixels_correct(handle, img):
 
 
 def bad_pixels_correct_batch(handle, frames, out=None):
-    """Correct a stack ``[n, h, w]`` of uint16 frames in one launch."""
+    """Correct a stack ``[n, h, w]`` of uint16 frames in one launch (``out is frames``: in place).  A strided numpy
+    ``frames`` is copied first; a strided ``out`` is refused."""
     lib = _lib.load()
-    if len(frames.shape) != 3:
-        raise RuntimeError("bad_pixels_correct_batch: wrong input dimension")
     _prepare_device_call(frames)
+    inplace = out is frames
+    frames = _bp_frames(handle, frames, "bad_pixels_correct_batch", copy=not inplace)
     if out is None:
         out = _empty_like(frames)
+    out = frames if inplace else _operand(out, "bad_pixels_correct_batch", "out", frames.shape, np.uint16)
     res = lib.rirb_bad_pixels_correct_batch(handle, _ptr(frames), _ptr(out), frames.shape[0])
     _lib.check(res, "bad_pixels_correct")
     return out

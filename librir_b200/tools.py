@@ -17,6 +17,7 @@ from typing import Dict
 import numpy as np
 
 from . import _lib
+from .signal_processing import _operand, _ptr
 
 
 def _bytes_of(x, enc) -> bytes:
@@ -301,8 +302,7 @@ class ZFileWriter:
         """frames ``[n, h, w]`` uint16 (numpy, or a torch CUDA tensor: one download), timestamps ``[n]`` in ns."""
         ts = np.ascontiguousarray(timestamps, dtype=np.int64)
         if _is_torch(frames):
-            if not frames.is_contiguous():
-                raise RuntimeError("librir_b200: tensors must be contiguous")
+            _operand(frames, "ZFileWriter.add_images", "frames", dtype=(np.uint16, np.int16))
             ptr, shape = ct.c_void_p(frames.data_ptr()), tuple(frames.shape)
             if frames.is_cuda:
                 _lib.use_torch_stream()
@@ -351,17 +351,16 @@ class ZFileReader:
         return self.read_images(pos, 1)[0]
 
     def read_images(self, pos=0, count=None, out=None):
-        """Frames ``[pos, pos + count)`` -> uint16 ``[count, h, w]`` (``out``: numpy array or torch CUDA tensor)."""
+        """Frames ``[pos, pos + count)`` -> uint16 ``[count, h, w]`` (``out``: numpy array or torch CUDA tensor of that
+        shape, uint16 or int16 -- the same bits; strided views are refused)."""
         if count is None:
             count = self.images - pos
         if out is None:
             out = np.empty((count, self.height, self.width), dtype=np.uint16)
-        if _is_torch(out):
-            ptr = ct.c_void_p(out.data_ptr())
-            if out.is_cuda:
-                _lib.use_torch_stream()
-        else:
-            ptr = out.ctypes.data_as(ct.c_void_p)
+        _operand(out, "ZFileReader.read_images", "out", (count, self.height, self.width), (np.uint16, np.int16))
+        if _is_torch(out) and out.is_cuda:
+            _lib.use_torch_stream()
+        ptr = _ptr(out)
         _lib.check(_lib.load().rirb_z_read_images(self.handle, int(pos), int(count), ptr, None, self.threads), "z_read_images")
         return out
 

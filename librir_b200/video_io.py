@@ -15,7 +15,7 @@ from __future__ import annotations
 import numpy as np
 
 from . import _lib
-from .signal_processing import _empty_like, _is_torch, _prepare_device_call, _ptr, bad_pixels_create, bad_pixels_destroy
+from .signal_processing import _empty_like, _is_torch, _operand, _prepare_device_call, _ptr, bad_pixels_create, bad_pixels_destroy
 
 DEFAULT_GOP = 50  # H264_Saver default, h264.cpp:1052-1061 / setParameter "GOP"
 
@@ -102,13 +102,19 @@ def merge_yuv420(y, width, u=None):
 def precode_movie(movie, gop=DEFAULT_GOP, delta=False, first_frame=0, out=None, stats=None):
     """Byte-plane split (+ optional temporal delta) of ``movie[t, h, w]`` (numpy or torch CUDA
     uint16).  Returns ``(lo, hi)`` uint8 ``[t, h, w]``.  ``stats``: a :class:`librir_b200.movie.MovieStats`
-    to fold the same frames into (min / max / histogram) in the same pass over them."""
+    to fold the same frames into (min / max / histogram) in the same pass over them.  ``out``: a ``(lo, hi)`` pair of
+    uint8 arrays of ``movie``'s shape.  A strided numpy ``movie`` is copied first; strided planes are refused."""
     lib = _lib.load()
     if len(movie.shape) != 3:
         raise RuntimeError("precode_movie: wrong input dimension")
     _prepare_device_call(movie)
+    movie = _operand(movie, "precode_movie", "movie", dtype=np.uint16, copy=True)
     t, h, w = movie.shape
+    if out is not None and len(out) != 2:
+        raise RuntimeError("precode_movie: out must be a (lo, hi) pair")
     lo, hi = out if out is not None else (_empty_like(movie, np.uint8), _empty_like(movie, np.uint8))
+    lo = _operand(lo, "precode_movie", "lo", movie.shape, np.uint8)
+    hi = _operand(hi, "precode_movie", "hi", movie.shape, np.uint8)
     if stats is not None:
         import ctypes as ct
 
@@ -127,11 +133,17 @@ def precode_movie(movie, gop=DEFAULT_GOP, delta=False, first_frame=0, out=None, 
 
 
 def decode_movie(lo, hi, gop=DEFAULT_GOP, delta=False, first_frame=0, out=None):
-    """Inverse of :func:`precode_movie`."""
+    """Inverse of :func:`precode_movie`: uint8 planes ``lo`` / ``hi`` ``[t, h, w]`` -> uint16 ``out`` of the same shape.
+    Strided numpy planes are copied first; a strided ``out`` is refused."""
     lib = _lib.load()
     _prepare_device_call(lo)
+    if len(lo.shape) != 3:
+        raise RuntimeError("decode_movie: wrong input dimension")
+    lo = _operand(lo, "decode_movie", "lo", dtype=np.uint8, copy=True)
+    hi = _operand(hi, "decode_movie", "hi", lo.shape, np.uint8, copy=True)
     t, h, w = lo.shape
     mov = out if out is not None else _empty_like(lo, np.uint16)
+    mov = _operand(mov, "decode_movie", "out", lo.shape, np.uint16)
     r = lib.rirb_decode_movie(_ptr(lo), _ptr(hi), t, w, h, gop, int(bool(delta)), first_frame, _ptr(mov))
     _lib.check(r, "decode_movie")
     return mov
@@ -191,12 +203,13 @@ class LoaderBadPixels:
             pass
 
     def remove(self, frames):
-        """In place on ``frames[n, h, w]`` (or one ``[h, w]`` frame); returns ``frames``."""
+        """In place on uint16 ``frames[n, h, w]`` (or one ``[h, w]`` frame); returns ``frames``.  Strided views are refused."""
         lib = _lib.load()
         _prepare_device_call(frames)
         n = 1 if len(frames.shape) == 2 else frames.shape[0]
         if tuple(frames.shape[-2:]) != (self.height, self.width):
             raise RuntimeError("remove_bad_pixels: wrong image size")
+        _operand(frames, "remove_bad_pixels", "frames", dtype=np.uint16)
         r = lib.rirb_loader_remove_bad_pixels(self.handle, _ptr(frames), n, self.height * self.width)
         _lib.check(r, "remove_bad_pixels")
         return frames
@@ -204,9 +217,13 @@ class LoaderBadPixels:
 
 def remove_motion(frames, shifts_x, shifts_y, meta_rows=3, out=None):
     """``removeMotionGeneric`` on a stack: frame t is translated by ``(-shifts_x[t], -shifts_y[t])``
-    on rows ``[0, h-meta_rows)``; the metadata rows pass through."""
+    on rows ``[0, h-meta_rows)``; the metadata rows pass through.  uint16 ``frames``; ``out``: same shape and dtype
+    (``out is frames``: in place).  A strided numpy ``frames`` is copied first (unless in place); a strided ``out`` is
+    refused."""
     lib = _lib.load()
     _prepare_device_call(frames)
+    inplace = out is frames
+    frames = _operand(frames, "remove_motion", "frames", dtype=np.uint16, copy=not inplace)
     single = len(frames.shape) == 2
     n = 1 if single else frames.shape[0]
     h, w = frames.shape[-2:]
@@ -216,6 +233,7 @@ def remove_motion(frames, shifts_x, shifts_y, meta_rows=3, out=None):
         raise RuntimeError("remove_motion: one shift per frame expected")
     if out is None:
         out = _empty_like(frames)
+    out = frames if inplace else _operand(out, "remove_motion", "out", frames.shape, np.uint16)
     r = lib.rirb_loader_remove_motion(_ptr(frames), _ptr(out), w, h - meta_rows, n, h * w, _ptr(sx), _ptr(sy))
     _lib.check(r, "remove_motion")
     return out
@@ -224,9 +242,10 @@ def remove_motion(frames, shifts_x, shifts_y, meta_rows=3, out=None):
 def finish_frames(frames, bad_pixels=None, min_T=0, min_T_height=0, shifts_x=None, shifts_y=None, meta_rows=3):
     """The same chain as :func:`read_movie` for frames that are uint16 already (decoded from the zstd movie file):
     ``+= min_T`` -> ``removeBadPixels`` -> ``removeMotion``, IN PLACE on ``frames`` ``[n, h, w]`` (numpy or torch CUDA).
-    What ``load_image`` of ``libvideo_io_b200.so`` runs after the decode."""
+    What ``load_image`` of ``libvideo_io_b200.so`` runs after the decode.  Strided views are refused."""
     lib = _lib.load()
     _prepare_device_call(frames)
+    _operand(frames, "finish_frames", "frames", dtype=np.uint16)
     single = len(frames.shape) == 2
     n = 1 if single else frames.shape[0]
     h, w = frames.shape[-2:]
@@ -247,14 +266,15 @@ def read_movie(lo, hi, bad_pixels=None, min_T=0, min_T_height=0, shifts_x=None, 
     run of decoded frames: byte planes ``lo``/``hi`` ``[n, h, w]`` (what ``VideoGrabber::toArray`` merges,
     h264.cpp:3016-3051) -> ``+= min_T`` on the first ``min_T_height`` rows -> ``removeBadPixels`` on rows
     ``[0, h-meta_rows)`` (``bad_pixels``: a :class:`LoaderBadPixels` or None) -> ``removeMotion`` by the
-    per-frame shifts of the ``.regfile`` (None: off).  Returns uint16 ``[n, h, w]``."""
+    per-frame shifts of the ``.regfile`` (None: off).  Returns uint16 ``[n, h, w]`` (``out``: of ``lo``'s shape).
+    Strided numpy planes are copied first; a strided ``out`` is refused."""
     lib = _lib.load()
     _prepare_device_call(lo)
     single = len(lo.shape) == 2
     n = 1 if single else lo.shape[0]
     h, w = lo.shape[-2:]
-    if tuple(hi.shape) != tuple(lo.shape):
-        raise RuntimeError("read_movie: lo and hi planes differ in shape")
+    lo = _operand(lo, "read_movie", "lo", dtype=np.uint8, copy=True)
+    hi = _operand(hi, "read_movie", "hi", lo.shape, np.uint8, copy=True)
     handle = 0
     if bad_pixels is not None:
         if (bad_pixels.height, bad_pixels.width) != (h, w) or bad_pixels.rows != h - meta_rows:
@@ -268,6 +288,7 @@ def read_movie(lo, hi, bad_pixels=None, min_T=0, min_T_height=0, shifts_x=None, 
             raise RuntimeError("read_movie: one shift per frame expected")
     if out is None:
         out = _empty_like(lo, np.uint16)
+    out = _operand(out, "read_movie", "out", lo.shape, np.uint16)
     r = lib.rirb_loader_read_movie(handle, _ptr(lo), _ptr(hi), n, w, h, int(min_T), int(min_T_height),
                                    _ptr(sx) if sx is not None else None, _ptr(sy) if sy is not None else None, int(meta_rows),
                                    _ptr(out))
@@ -304,15 +325,18 @@ class LossyPreconditioner:
 
     def add_images(self, frames, out=None):
         """``frames``: uint16 ``[n, h, w]`` (or one ``[h, w]`` frame), numpy or torch CUDA.  Returns
-        ``(out, errors)`` with ``errors[t] = (BackgroundError, ForegroundError)`` of frame t."""
+        ``(out, errors)`` with ``errors[t] = (BackgroundError, ForegroundError)`` of frame t.  ``out``: uint16 of
+        ``frames``' shape.  A strided numpy ``frames`` is copied first; a strided ``out`` is refused."""
         lib = _lib.load()
         _prepare_device_call(frames)
+        frames = _operand(frames, "lossy add_images", "frames", dtype=np.uint16, copy=True)
         single = len(frames.shape) == 2
         n = 1 if single else frames.shape[0]
         if tuple(frames.shape[-2:]) != (self.height, self.width):
             raise RuntimeError("lossy add_images: wrong image size")
         if out is None:
             out = _empty_like(frames)
+        out = _operand(out, "lossy add_images", "out", frames.shape, np.uint16)
         errors = np.zeros((n, 2), dtype=np.int32)
         r = lib.rirb_lossy_add_images(self.handle, _ptr(frames), n, _ptr(out), _ptr(errors))
         _lib.check(r, "lossy_add_images")
