@@ -288,7 +288,9 @@ struct EccIterate {  // the scalar state of the loop
 };
 
 // From the sums to the next shift: means / norms under the warped mask, 2 x 2 Hessian inverse, rho, lambda, update --
-// in the float / double types OpenCV's Mats have.
+// in the float / double types OpenCV's Mats have.  Every double multiply, add and subtract is an explicit _rn intrinsic, so
+// the compiler cannot contract a product with its neighbouring add into an FMA (--fmad=true): the roundings are the ones
+// the source text shows, as in OpenCV's x86-64 build, and tests/ecc_kernel.py restates them bit for bit.
 __device__ __forceinline__ void ecc_update(const double* acc, EccIterate& s, int max_it, double eps)
 {
     const double n = acc[A_N], sI = acc[A_I], sT = acc[A_T], sII = acc[A_II], sTT = acc[A_TT], sIT = acc[A_IT];
@@ -301,39 +303,43 @@ __device__ __forceinline__ void ecc_update(const double* acc, EccIterate& s, int
     } else {
         // meanStdDev under the warped mask; subtract(image, mean) works in the image's type: the mean is rounded to float
         const double meanI = sI / n, meanT = sT / n;
-        const double varI = fmax(sII / n - meanI * meanI, 0.0), varT = fmax(sTT / n - meanT * meanT, 0.0);
-        const double img_norm = sqrt(n * varI), tmp_norm = sqrt(n * varT);
+        const double varI = fmax(__dsub_rn(sII / n, __dmul_rn(meanI, meanI)), 0.0);
+        const double varT = fmax(__dsub_rn(sTT / n, __dmul_rn(meanT, meanT)), 0.0);
+        const double img_norm = sqrt(__dmul_rn(n, varI)), tmp_norm = sqrt(__dmul_rn(n, varT));
         const double muI = (double)(float)meanI, muT = (double)(float)meanT;
         const float H11 = (float)h11, H12 = (float)h12, H22 = (float)h22;  // Mat hessian is CV_32F
         // cv::invert of a 2 x 2 float matrix: closed form evaluated in double
-        const double det = (double)H11 * H22 - (double)H12 * H12;
+        const double det = __dsub_rn(__dmul_rn(H11, H22), __dmul_rn(H12, H12));
         const double id = det != 0.0 ? 1.0 / det : 0.0;
-        const float Hi11 = (float)(H22 * id), Hi22 = (float)(H11 * id), Hi12 = (float)(-(double)H12 * id);
-        const double corr = sIT - muT * sI - muI * sT + muI * muT * n;  // templateZM . imageWarped
+        const float Hi11 = (float)__dmul_rn(H22, id), Hi22 = (float)__dmul_rn(H11, id), Hi12 = (float)__dmul_rn(-(double)H12, id);
+        // templateZM . imageWarped = sIT - muT sI - muI sT + muI muT n
+        const double corr = __dadd_rn(__dsub_rn(__dsub_rn(sIT, __dmul_rn(muT, sI)), __dmul_rn(muI, sT)), __dmul_rn(__dmul_rn(muI, muT), n));
         s.last_rho = s.rho;
-        s.rho = corr / (img_norm * tmp_norm);
+        s.rho = corr / __dmul_rn(img_norm, tmp_norm);
         if (isnan(s.rho) || det == 0.0) {
             s.status = 1;
         } else {
-            const double pI1 = b1 - muI * c1, pI2 = b2 - muI * c2;  // J^T (I - mean), exact sums
-            const double pT1 = d1 - muT * c1, pT2 = d2 - muT * c2;  // J^T (T - mean)
+            const double pI1 = __dsub_rn(b1, __dmul_rn(muI, c1)), pI2 = __dsub_rn(b2, __dmul_rn(muI, c2));  // J^T (I - mean), exact sums
+            const double pT1 = __dsub_rn(d1, __dmul_rn(muT, c1)), pT2 = __dsub_rn(d2, __dmul_rn(muT, c2));  // J^T (T - mean)
             const float ip1 = (float)pI1, ip2 = (float)pI2, tp1 = (float)pT1, tp2 = (float)pT2;  // CV_32F projections
-            const float iph1 = (float)((double)Hi11 * ip1 + (double)Hi12 * ip2), iph2 = (float)((double)Hi12 * ip1 + (double)Hi22 * ip2);
-            const double lam_n = img_norm * img_norm - ((double)ip1 * iph1 + (double)ip2 * iph2);
-            const double lam_d = corr - ((double)tp1 * iph1 + (double)tp2 * iph2);
+            const float iph1 = (float)__dadd_rn(__dmul_rn(Hi11, ip1), __dmul_rn(Hi12, ip2));
+            const float iph2 = (float)__dadd_rn(__dmul_rn(Hi12, ip1), __dmul_rn(Hi22, ip2));
+            const double lam_n = __dsub_rn(__dmul_rn(img_norm, img_norm), __dadd_rn(__dmul_rn(ip1, iph1), __dmul_rn(ip2, iph2)));
+            const double lam_d = __dsub_rn(corr, __dadd_rn(__dmul_rn(tp1, iph1), __dmul_rn(tp2, iph2)));
             if (lam_d <= 0.0) {
                 s.rho = -1.0;
                 s.status = 2;
             } else {
                 const double lam = lam_n / lam_d;
-                const float e1 = (float)(lam * pT1 - pI1), e2 = (float)(lam * pT2 - pI2);  // J^T (lambda T - I)
-                const float dp1 = (float)((double)Hi11 * e1 + (double)Hi12 * e2), dp2 = (float)((double)Hi12 * e1 + (double)Hi22 * e2);
+                const float e1 = (float)__dsub_rn(__dmul_rn(lam, pT1), pI1), e2 = (float)__dsub_rn(__dmul_rn(lam, pT2), pI2);  // J^T (lambda T - I)
+                const float dp1 = (float)__dadd_rn(__dmul_rn(Hi11, e1), __dmul_rn(Hi12, e2));
+                const float dp2 = (float)__dadd_rn(__dmul_rn(Hi12, e1), __dmul_rn(Hi22, e2));
                 s.tx = __fadd_rn(s.tx, dp1);
                 s.ty = __fadd_rn(s.ty, dp2);
             }
         }
     }
-    s.done = s.status != 0 || s.it >= max_it || !(fabs(s.rho - s.last_rho) >= eps);
+    s.done = s.status != 0 || s.it >= max_it || !(fabs(__dsub_rn(s.rho, s.last_rho)) >= eps);
 }
 
 // Driver 1: one launch per iteration; the last CTA to finish adds up the slots and runs the update (used when a

@@ -62,6 +62,31 @@ FLARE = 1200.0        # lowers the confidence below the reset threshold, ECC sti
 SMALL_CASES = [(1.37, -0.62), (0.1, 0.05), (-2.5, 3.25), (4.8, -3.9), (0.0, 0.0), (7.3, 5.1)]
 
 
+def ir_window_pair(t=3, h=358, w=448):
+    """The class's default window (448 x 358 of a 640 x 512 frame) of frames 0 and t of the movie, as float32."""
+    sx, sy = trajectory(t + 1)
+    y0, x0 = (512 - h) // 2, (640 - w) // 2
+    crop = (slice(y0, y0 + h), slice(x0, x0 + w))
+    return frame(0, sx[0], sy[0])[crop].astype(np.float32), frame(t, sx[t], sy[t])[crop].astype(np.float32)
+
+
+def ulps(v):
+    """v and the float32 values one ulp either side of it."""
+    v = np.float32(v)
+    return [float(np.nextafter(v, np.float32(-np.inf))), float(v), float(np.nextafter(v, np.float32(np.inf)))]
+
+
+def boundary_starts():
+    """Starts on and one float ulp either side of every (2k+1)/64 px boundary (bilinear fraction), every (2k+1)/2 px
+    boundary (nearest), ties tx * 1024 = m + 1/2 (round half to even), negative starts included."""
+    s = []
+    for k in range(-5, 5):
+        s += ulps((2 * k + 1) / 64.0) + ulps((2 * k + 1) / 2.0) + ulps(k + (2 * k + 1) / 64.0)
+    for m in (-1537, -512, -17, -16, -15, -1, 0, 1, 15, 16, 17, 511, 512, 1535):
+        s += ulps((m + 0.5) / 1024.0)
+    return sorted(set(s))
+
+
 def failing_frames():
     """Second frames on which findTransformECC raises: contrast-inverted (correlation about to be minimised) and flat (NaN)."""
     sx, sy = trajectory(6)
