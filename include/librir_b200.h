@@ -237,6 +237,19 @@ RIRB_API int rirb_hist_quantile(const unsigned long long* hist, long long count,
 /* get_background (h264.cpp:1955-1991) of one image */
 RIRB_API int rirb_get_background(const unsigned short* pixels, int size);
 
+/* ---- connected components of thresholded frames (scipy.ndimage.label's numbering), with statistics ----
+ * A pixel of frame t is foreground iff frames[t][y][x] > thresholds[n_thresholds == 1 ? 0 : t]; n_thresholds is 1 or
+ * nframes and the thresholds may be host or device memory.  connectivity 4 (edge neighbours) or 8 (edges and corners),
+ * -1 otherwise.  labels[t][y][x] (int32): 0 for background, else 1..K_t numbered in raster order of each component's
+ * first pixel -- scipy.ndimage.label(mask, generate_binary_structure(2, 1 or 2)).  counts[t] = K_t, always the true count.
+ * stats: NULL, or int64 [nframes][max_components][10]; row k-1 describes label k for k <= min(K_t, max_components):
+ * area, x_min, y_min, x_max, y_max (inclusive), sum x, sum y, sum value, max value, argmax (y * w + x of the first pixel
+ * in raster order holding the maximum).  Other rows are not written.  Every column is an integer, so the result is
+ * bit-exact; the centroid is sum / area.  w * h < 2^31, any number of frames, the usual operand rules (above). */
+RIRB_API int rirb_label_batch(const unsigned short* frames, int w, int h, long long nframes, const unsigned short* thresholds,
+                              long long n_thresholds, int connectivity, int* labels, int* counts, long long* stats,
+                              int max_components);
+
 /* ===================== Part 3: the file formats either side of the path (host code) ========
  * SURVEY.md 8f-3.  No kernels here: the entropy stage is zstd on the host by design.  What is added
  * over the reference: a run of frames is (de)compressed by a pool of host threads with the records

@@ -2,6 +2,7 @@
 // staging for host-pointer callers, the bad-pixel handle table, forwarding of the out-of-scope
 // entries.  All compute happens in the kernels of this directory; there is no CPU path.
 #include <dlfcn.h>
+#include <limits.h>
 #include <math.h>
 #include <stdarg.h>
 #include <stdlib.h>
@@ -1737,6 +1738,44 @@ int rirb_get_background(const unsigned short* pixels, int size)
     RIRB_CUDA_OK(cudaMemcpyAsync(&r, d_out, sizeof(unsigned), cudaMemcpyDeviceToHost, st));
     RIRB_CUDA_OK(cudaStreamSynchronize(st));
     return (int)r;
+}
+
+// =================================================================================================
+// connected components (label.cu)
+// =================================================================================================
+int rirb_label_batch(const unsigned short* frames, int w, int h, long long nframes, const unsigned short* thresholds,
+                     long long n_thresholds, int connectivity, int* labels, int* counts, long long* stats, int max_components)
+{
+    if (connectivity != 4 && connectivity != 8) {
+        set_error("label_batch: connectivity must be 4 or 8, not %d", connectivity);
+        return -1;
+    }
+    if (!frames || !thresholds || !labels || !counts || w <= 0 || h <= 0 || (long long)w * h > INT_MAX || nframes < 0 ||
+        (n_thresholds != 1 && n_thresholds != nframes) || (stats && max_components < 0)) {
+        set_error("label_batch: bad arguments");
+        return -1;
+    }
+    if (nframes == 0) return 0;
+    RIRB_REQUIRE_DEVICE();
+    const int cap = stats ? max_components : 0;
+    const size_t npx = (size_t)w * h * (size_t)nframes;
+    const size_t sbytes = (size_t)nframes * cap * 10 * sizeof(long long);
+    if (refuse_overlap("label_batch", {{"frames", frames, npx * 2}, {"thresholds", thresholds, 2 * (size_t)n_thresholds}},
+                       {{"labels", labels, npx * 4}, {"counts", counts, 4 * (size_t)nframes}, {"stats", stats, sbytes}}))
+        return -1;
+    cudaStream_t st = tls.stream;
+    const u16* d_frames = (const u16*)stage_in(frames, npx * 2, 0, st);
+    const u16* d_thr = (const u16*)stage_in(thresholds, 2 * (size_t)n_thresholds, 2, st);
+    if (!d_frames || !d_thr) return -1;
+    StagedOut outs[3];
+    if (!stage_out(outs[0], labels, npx * 4, 1, false, st) || !stage_out(outs[1], counts, 4 * (size_t)nframes, 3, false, st))
+        return -1;
+    // rows past K_t keep what the caller had in them: a host stats array goes up first
+    if (sbytes && !stage_out(outs[2], stats, sbytes, 4, true, st)) return -1;
+    if (launch_label(d_frames, w, h, nframes, d_thr, n_thresholds > 1, connectivity, (int*)outs[0].dev, (int*)outs[1].dev,
+                     (long long*)outs[2].dev, cap, st) != 0)
+        return -1;
+    return finish_out(outs, 3, st);
 }
 
 // =================================================================================================

@@ -178,6 +178,11 @@ int launch_lossy_frame(const u16* img, const u16* tmp, u16* tmpT, u16* out, u16*
                        int low0, int high0, double std_factor, int variant, int quirk, void* scalars, int* errors_out_dev,
                        cudaStream_t st);
 
+// label.cu (rirb_label_batch): labels[t] (the parent array while it runs) and counts[t] for nframes frames; stats NULL or
+// [nframes][cap][10].  thr: one threshold, or one per frame when per_frame_thr.  Work space: scratch slot 8.
+int launch_label(const u16* frames, int w, int h, long long nframes, const u16* thr, int per_frame_thr, int connectivity,
+                 int* labels, int* counts, long long* stats, int cap, cudaStream_t st);
+
 // stats.cu
 // minmax[0] = min, minmax[1] = max (unsigned, device); hist = 65536 x u64 (device) or nullptr.
 // Accumulates INTO the outputs: callers zero hist / seed minmax with {65535, 0} first

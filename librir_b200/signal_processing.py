@@ -260,6 +260,64 @@ def find_median_pixel(image, percent=0.5, mask=None):
 
 
 # ----------------------------------------------------------------------------------------
+# connected components
+# ----------------------------------------------------------------------------------------
+# columns of the statistics rows of ``label_batch``; the centroid is ``stats[..., SUM_X] / stats[..., AREA]``
+AREA, X_MIN, Y_MIN, X_MAX, Y_MAX, SUM_X, SUM_Y, SUM_VALUE, MAX_VALUE, ARGMAX = range(10)
+
+
+def label_batch(frames, threshold, connectivity=8, max_components=256, labels=None):
+    """Connected components of ``frames > threshold`` for a uint16 stack ``[n, h, w]``, with per-component statistics.
+
+    ``threshold``: a scalar or one value per frame (sequence, numpy array or tensor of uint16 range).  ``connectivity``:
+    4 or 8.  Returns ``(labels, counts, stats)``: int32 ``labels [n, h, w]`` (0 background, 1..K numbered in raster order
+    of each component's first pixel, as ``scipy.ndimage.label``), int32 ``counts [n]`` (the true K of each frame) and
+    int64 ``stats [n, max_components, 10]`` whose row ``k - 1`` describes label ``k`` (columns ``AREA`` .. ``ARGMAX``;
+    rows past ``min(K, max_components)`` are zero).  numpy in gives numpy out; a torch CUDA tensor gives tensors on its
+    device.  ``labels``: an int32 output of the same shape, or None."""
+    lib = _lib.load()
+    what = "label_batch"
+    if len(frames.shape) != 3:
+        raise RuntimeError(f"{what}: wrong input dimension")
+    if connectivity not in (4, 8):
+        raise RuntimeError(f"{what}: connectivity must be 4 or 8, not {connectivity}")
+    if int(max_components) != max_components or max_components < 0:
+        raise RuntimeError(f"{what}: max_components must be a non-negative integer")
+    max_components = int(max_components)
+    _prepare_device_call(frames)
+    frames = _operand(frames, what, "frames", dtype=np.uint16, copy=True)
+    n, h, w = frames.shape
+    if _is_torch(threshold):
+        thr = _operand(threshold.reshape(-1), what, "threshold", dtype=np.uint16)
+        nt = thr.numel()
+    else:
+        t = np.asarray(threshold).reshape(-1)
+        if t.size and (not np.all(np.isfinite(t)) or np.any(t != np.floor(t)) or t.min() < 0 or t.max() > 65535):
+            raise RuntimeError(f"{what}: thresholds must be integers in [0, 65535]")
+        thr = np.ascontiguousarray(t, dtype=np.uint16)
+        nt = thr.size
+    if nt not in (1, n):
+        raise RuntimeError(f"{what}: {nt} thresholds for {n} frames")
+    if _is_torch(frames):
+        import torch
+
+        if labels is None:
+            labels = torch.empty((n, h, w), dtype=torch.int32, device=frames.device)
+        counts = torch.empty(n, dtype=torch.int32, device=frames.device)
+        stats = torch.zeros((n, max_components, 10), dtype=torch.int64, device=frames.device)
+    else:
+        if labels is None:
+            labels = np.empty((n, h, w), np.int32)
+        counts = np.empty(n, np.int32)
+        stats = np.zeros((n, max_components, 10), np.int64)
+    labels = _operand(labels, what, "labels", (n, h, w), np.int32)
+    r = lib.rirb_label_batch(_ptr(frames), w, h, n, _ptr(thr), nt, connectivity, _ptr(labels), _ptr(counts), _ptr(stats),
+                             max_components)
+    _lib.check(r, what)
+    return labels, counts, stats
+
+
+# ----------------------------------------------------------------------------------------
 # bad pixels
 # ----------------------------------------------------------------------------------------
 def bad_pixels_create(first_image):
@@ -382,6 +440,7 @@ __all__ = [
     "gaussian_filter",
     "gaussian_filter_batch",
     "find_median_pixel",
+    "label_batch",
     "bad_pixels_create",
     "bad_pixels_correct",
     "bad_pixels_correct_batch",
