@@ -250,6 +250,24 @@ RIRB_API int rirb_label_batch(const unsigned short* frames, int w, int h, long l
                               long long n_thresholds, int connectivity, int* labels, int* counts, long long* stats,
                               int max_components);
 
+/* ---- events: connected components of a thresholded movie in space and time, with statistics ----
+ * Voxel (t, y, x) is foreground iff frames[t][y][x] > thresholds[n_thresholds == 1 ? 0 : t], thresholds as in
+ * rirb_label_batch.  connectivity 6, 18 or 26 (axes (t, y, x)), -1 otherwise: in the plane 4, 8 and 8 neighbours; to each
+ * neighbouring frame the same pixel, the same pixel and its 4 edge neighbours, or the 3 x 3 block --
+ * scipy.ndimage.generate_binary_structure(3, 1, 2 or 3).  labels[t][y][x] (int32): 0 for background, else 1..K numbered
+ * in (t, y, x) raster order of each event's first voxel -- scipy.ndimage.label(mask, structure) on the [n, h, w] volume.
+ * *count = K, always the true count; -1 (no result) if K would exceed INT_MAX.  stats: NULL, or int64
+ * [max_events][13]; row k-1 describes event k for k <= min(K, max_events): volume, t_first, t_last, x_min, y_min, x_max,
+ * y_max (inclusive), sum t, sum x, sum y, sum value, max value, argmax (t * h * w + y * w + x of the first voxel in
+ * (t, y, x) raster order holding the maximum).  Other rows are not written.  Every column is an integer, so the result
+ * is bit-exact.  nframes == 0 gives *count = 0.  w * h < 2^31, fewer than 2^48 voxels, the usual operand rules (above).
+ * The whole movie is one call (an event's number is known only once every frame has been seen); the call waits for its
+ * stream once, to read the number of 2-D components, before the rest is enqueued (a second time, to read K, only when
+ * those outnumber INT_MAX). */
+RIRB_API int rirb_label_movie(const unsigned short* frames, int w, int h, long long nframes, const unsigned short* thresholds,
+                              long long n_thresholds, int connectivity, int* labels, int* count, long long* stats,
+                              int max_events);
+
 /* ===================== Part 3: the file formats either side of the path (host code) ========
  * SURVEY.md 8f-3.  No kernels here: the entropy stage is zstd on the host by design.  What is added
  * over the reference: a run of frames is (de)compressed by a pool of host threads with the records

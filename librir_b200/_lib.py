@@ -83,6 +83,7 @@ SIGNATURES = {
     "rirb_hist_quantile": (_i, [_vp, _ll, _f]),
     "rirb_get_background": (_i, [_vp, _i]),
     "rirb_label_batch": (_i, [_vp, _i, _i, _ll, _vp, _ll, _i, _vp, _vp, _vp, _i]),
+    "rirb_label_movie": (_i, [_vp, _i, _i, _ll, _vp, _ll, _i, _vp, _vp, _vp, _i]),
     # Part 3: file formats (host code)
     "rirb_attrs_open_file": (_i, [ct.c_char_p]),
     "rirb_attrs_open_from_memory": (_i, [_vp, _ll]),

@@ -1778,6 +1778,52 @@ int rirb_label_batch(const unsigned short* frames, int w, int h, long long nfram
     return finish_out(outs, 3, st);
 }
 
+int rirb_label_movie(const unsigned short* frames, int w, int h, long long nframes, const unsigned short* thresholds,
+                     long long n_thresholds, int connectivity, int* labels, int* count, long long* stats, int max_events)
+{
+    if (connectivity != 6 && connectivity != 18 && connectivity != 26) {
+        set_error("label_movie: connectivity must be 6, 18 or 26, not %d", connectivity);
+        return -1;
+    }
+    if (!frames || !thresholds || !labels || !count || w <= 0 || h <= 0 || (long long)w * h > INT_MAX || nframes < 0 ||
+        (n_thresholds != 1 && n_thresholds != nframes) || max_events < 0) {
+        set_error("label_movie: bad arguments");
+        return -1;
+    }
+    if (nframes > 0 && (double)w * h * (double)nframes >= 281474976710656.0) {  // 2^48: the argmax column's packing
+        set_error("label_movie: %lld frames of %d x %d are 2^48 voxels or more", nframes, w, h);
+        return -1;
+    }
+    if (nframes == 0) {
+        if (!is_device_ptr(count)) {
+            *count = 0;
+            return 0;
+        }
+        RIRB_REQUIRE_DEVICE();
+        RIRB_CUDA_OK(cudaMemsetAsync(count, 0, sizeof(int), tls.stream));
+        return 0;
+    }
+    RIRB_REQUIRE_DEVICE();
+    const int cap = stats ? max_events : 0;
+    const size_t npx = (size_t)w * h * (size_t)nframes;
+    const size_t sbytes = (size_t)cap * 13 * sizeof(long long);
+    if (refuse_overlap("label_movie", {{"frames", frames, npx * 2}, {"thresholds", thresholds, 2 * (size_t)n_thresholds}},
+                       {{"labels", labels, npx * 4}, {"count", count, sizeof(int)}, {"stats", stats, sbytes}}))
+        return -1;
+    cudaStream_t st = tls.stream;
+    const u16* d_frames = (const u16*)stage_in(frames, npx * 2, 0, st);
+    const u16* d_thr = (const u16*)stage_in(thresholds, 2 * (size_t)n_thresholds, 2, st);
+    if (!d_frames || !d_thr) return -1;
+    StagedOut outs[3];
+    if (!stage_out(outs[0], labels, npx * 4, 1, false, st) || !stage_out(outs[1], count, sizeof(int), 3, false, st)) return -1;
+    // rows past K keep what the caller had in them: a host stats array goes up first
+    if (sbytes && !stage_out(outs[2], stats, sbytes, 4, true, st)) return -1;
+    if (launch_label_movie(d_frames, w, h, nframes, d_thr, n_thresholds > 1, connectivity, (int*)outs[0].dev, (int*)outs[1].dev,
+                           (long long*)outs[2].dev, cap, st) != 0)
+        return -1;
+    return finish_out(outs, 3, st);
+}
+
 // =================================================================================================
 // forwarded entries (outside the hot path)
 // =================================================================================================

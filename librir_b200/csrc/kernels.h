@@ -182,6 +182,11 @@ int launch_lossy_frame(const u16* img, const u16* tmp, u16* tmpT, u16* out, u16*
 // [nframes][cap][10].  thr: one threshold, or one per frame when per_frame_thr.  Work space: scratch slot 8.
 int launch_label(const u16* frames, int w, int h, long long nframes, const u16* thr, int per_frame_thr, int connectivity,
                  int* labels, int* counts, long long* stats, int cap, cudaStream_t st);
+// label.cu (rirb_label_movie): events of the (t, y, x) volume at connectivity 6, 18 or 26; labels [nframes][h][w], *count
+// = K, stats NULL or [cap][13].  nframes >= 1.  Synchronises st once to read the number of 2-D components (twice when
+// that exceeds INT_MAX).  Work space: scratch slots 8 (launch_label) to 11.
+int launch_label_movie(const u16* frames, int w, int h, long long nframes, const u16* thr, int per_frame_thr, int connectivity,
+                       int* labels, int* count, long long* stats, int cap, cudaStream_t st);
 
 // stats.cu
 // minmax[0] = min, minmax[1] = max (unsigned, device); hist = 65536 x u64 (device) or nullptr.

@@ -1,5 +1,5 @@
 // librir_b200/csrc/label.cu -- connected components of thresholded frames with per-component statistics
-// (rirb_label_batch).
+// (rirb_label_batch), and events of the whole (t, y, x) volume built on them (rirb_label_movie, second half of the file).
 //
 // Contract: a pixel is foreground iff frame > threshold; labels are 0 for background and 1..K in raster order of each
 // component's first pixel (scipy.ndimage.label's numbering); statistics are integer sums, extrema and the raster-first
@@ -22,6 +22,8 @@
 // Traffic: 2 B/px read + 4 B/px written (1), 4 B/px read + 2 B/px read + 4 B/px written (5); the border, root and
 // scan passes touch 1/32 of that.
 #include <limits.h>
+
+#include <cub/device/device_scan.cuh>
 
 #include "common.cuh"
 #include "kernels.h"
@@ -57,13 +59,15 @@ __device__ void union_s(int* s, int a, int b)
     }
 }
 
-// ---- union-find in global memory (frame-local indices; L2 loads: other CTAs change the parents) ----------------
-// Root of x with path halving.  Callers pass a tile-local root, so every parent it rewrites is one.
-__device__ int find_g(int* L, int x)
+// ---- union-find in global memory (L2 loads: other CTAs change the parents) --------------------------------------
+// T = int: frame-local pixel indices (rirb_label_batch); T = long long: movie-wide component ids (rirb_label_movie).
+// Root of x with path halving.  The 2-D passes pass a tile-local root, so every parent it rewrites is one.
+template <typename T>
+__device__ T find_g(T* L, T x)
 {
-    int p = __ldcg(L + x);
+    T p = __ldcg(L + x);
     while (p != x) {
-        const int gp = __ldcg(L + p);
+        const T gp = __ldcg(L + p);
         if (gp == p) return p;
         __stcg(L + x, gp);
         x = gp;
@@ -71,18 +75,19 @@ __device__ int find_g(int* L, int x)
     }
     return x;
 }
-__device__ void union_g(int* L, int a, int b)
+template <typename T>
+__device__ void union_g(T* L, T a, T b)
 {
     for (;;) {
         a = find_g(L, a);
         b = find_g(L, b);
         if (a == b) return;
         if (a < b) {
-            const int t = a;
+            const T t = a;
             a = b;
             b = t;
         }
-        const int old = atomicMin(L + a, b);
+        const T old = atomicMin(L + a, b);
         if (old == a) return;
         a = old;
     }
@@ -90,9 +95,10 @@ __device__ void union_g(int* L, int a, int b)
 
 // Root of x without writes: the roots pass points each tile-local root at its component root, and a path-halving store
 // from another thread landing after that would leave the tile-local root on an intermediate node.
-__device__ __forceinline__ int root_of(const int* L, int x)
+template <typename T>
+__device__ __forceinline__ T root_of(const T* L, T x)
 {
-    int p;
+    T p;
     while ((p = __ldcg(L + x)) != x) x = p;
     return x;
 }
@@ -101,6 +107,18 @@ struct LabelGeom {
     int w, h, tiles_x, tiles;  // tiles per frame
     size_t npx, segs;          // pixels and 32-pixel row segments per frame (segs = h * tiles_x)
 };
+
+static LabelGeom label_geom(int w, int h)
+{
+    LabelGeom g;
+    g.w = w;
+    g.h = h;
+    g.tiles_x = (int)ceil_div(w, LB_TW);
+    g.tiles = g.tiles_x * (int)ceil_div(h, LB_TH);
+    g.npx = (size_t)w * h;
+    g.segs = (size_t)h * g.tiles_x;
+    return g;
+}
 
 // ---- 1. tile-local labelling -----------------------------------------------------------------------------------
 template <int CONN>
@@ -373,13 +391,7 @@ __global__ void __launch_bounds__(256) label_stats_split_kernel(long long* __res
 int launch_label(const u16* frames, int w, int h, long long nframes, const u16* thr, int per_frame_thr, int connectivity,
                  int* labels, int* counts, long long* stats, int cap, cudaStream_t st)
 {
-    LabelGeom g;
-    g.w = w;
-    g.h = h;
-    g.tiles_x = (int)ceil_div(w, LB_TW);
-    g.tiles = g.tiles_x * (int)ceil_div(h, LB_TH);
-    g.npx = (size_t)w * h;
-    g.segs = (size_t)h * g.tiles_x;
+    const LabelGeom g = label_geom(w, h);
     if (cap <= 0) stats = nullptr;
     // frames per round: a 1-D grid of tiles, and at most 256 MB of segment masks + offsets
     long long per = INT_MAX / g.tiles;
@@ -416,6 +428,317 @@ int launch_label(const u16* frames, int w, int h, long long nframes, const u16* 
         } else {
             RIRB_LAUNCH(label_final_kernel<false>, grid, tile_block, 0, st, fr, g, Lf, roots, off, sf, cap);
         }
+    }
+    return 0;
+}
+
+// =================================================================================================================
+// rirb_label_movie: events, the connected components of the whole (t, y, x) volume
+// =================================================================================================================
+// 6-, 18- and 26-connectivity are 4-, 8- and 8-connectivity in the plane plus, to the neighbouring frame, the same
+// pixel, the same pixel and its 4 edge neighbours, or the 3 x 3 block.  So the 2-D passes above label every frame at
+// the in-plane connectivity (labels = 2-D labels 1..K_t, counts = K_t), and what is left is a union-find over the
+// 2-D components:
+//   ids:     base[t] = K_0 + .. + K_{t-1} (exclusive scan); component (t, l) has id g = base[t] + l - 1, C = sum K_t.
+//   link:    for every foreground pixel of frame t >= 1 and every foreground stencil neighbour in frame t - 1, union
+//            the two ids (union_g on a 64-bit parent array: the smaller root becomes the parent).  A lane skips a pair
+//            that the lane before it (pixel x - 1 of the same row) or its own previous union already joined, and
+//            union_g finds both roots before any atomic, so an all-foreground volume does one union per warp and tile.
+//   roots:   each id is pointed at its root (path halving first, so a chain of unions through every frame is walked
+//            once, not once per member); root flags.
+//   scan:    inclusive scan of the flags: ids[r] = 1 + roots before r for a root r; ids[C] = K.  Then every non-root
+//            takes its root's number (read-only finds; roots' entries are never written, so the pass does not race).
+//   final:   labels[t][y][x] = ids[base[t] + l - 1] in place; with statistics, each CTA folds its tile per event in a
+//            shared hash (warps pre-reduce equal-event runs of a row) before one set of global atomics per event and
+//            tile.  A last kernel splits the packed (max value, argmax) column.
+// Why this numbering is scipy.ndimage.label's on the volume: the order of g is (t, raster order of the component's
+// first pixel).  Take an event E and its first voxel v in (t, y, x) raster order, in frame t0, the first frame E
+// touches.  Every other 2-D component of E lies in a later frame, or in frame t0 with its first pixel after v, so the
+// component holding v has the smallest g of E, and it is E's root.  Two events are then in the order of their roots'
+// g, i.e. of (t0, raster position of v): the 3-D raster order of their first voxels.
+// Traffic beyond the 2-D passes: link 4 B/px read (the previous frame's labels come from L2) plus 8 B per union,
+// final 4 B/px read + 4 B/px written (+ 2 B/px read with statistics) plus 8 B per 2-D component.
+constexpr int LM_COLS = 13;
+constexpr unsigned long long LM_IDX_MASK = (1ull << 48) - 1;  // argmax indices; the entry refuses movies of >= 2^48 voxels
+
+static size_t align256(size_t b) { return (b + 255) & ~(size_t)255; }
+
+static unsigned flat_grid(long long n)
+{
+    const long long b = ceil_div(n, 256), cap = 8LL * sm_count();
+    return (unsigned)(b < 1 ? 1 : b < cap ? b : cap);
+}
+static unsigned tile_grid(long long items)
+{
+    const long long cap = 32LL * sm_count();
+    return (unsigned)(items < cap ? items : cap);
+}
+
+__global__ void __launch_bounds__(256) movie_init_kernel(long long* __restrict__ P, long long C)
+{
+    for (long long c = (long long)blockIdx.x * blockDim.x + threadIdx.x; c < C; c += (long long)gridDim.x * blockDim.x) P[c] = c;
+}
+
+// K_t (int, from launch_label) -> base[t] (int64, scanned in place), base[n] = 0
+__global__ void __launch_bounds__(256) movie_widen_kernel(const int* __restrict__ kt, long long* __restrict__ base, long long n)
+{
+    for (long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x; t <= n; t += (long long)gridDim.x * blockDim.x)
+        base[t] = t < n ? kt[t] : 0;
+}
+
+// ---- 7. links between consecutive frames -----------------------------------------------------------------------
+// Work item wi: tile (wi % tiles) of frame 1 + wi / tiles, joined to frame t - 1.
+template <int CONN>
+__global__ void __launch_bounds__(LB_TW* LB_BY, 4)  // without a floor on the CTAs per SM, ptxas caps it at 32 registers and spills
+movie_link_kernel(LabelGeom g, const int* __restrict__ labels, const long long* __restrict__ base, long long* __restrict__ P,
+                  long long items)
+{
+    const int lx = threadIdx.x;
+    for (long long wi = blockIdx.x; wi < items; wi += gridDim.x) {
+        const long long t = 1 + wi / g.tiles;
+        const int tile = (int)(wi - (t - 1) * g.tiles);
+        const int tx0 = (tile % g.tiles_x) * LB_TW, ty0 = (tile / g.tiles_x) * LB_TH;
+        const int* Lc = labels + t * g.npx;
+        const int* Lp = Lc - g.npx;
+        const long long gc = base[t] - 1, gp = base[t - 1] - 1;
+        const int x = tx0 + lx;
+        int last_a = 0, last_b = 0;  // this thread's last union
+        for (int ly = threadIdx.y; ly < LB_TH; ly += LB_BY) {
+            const int y = ty0 + ly;
+            const int a = (x < g.w && y < g.h) ? __ldg(Lc + (size_t)y * g.w + x) : 0;
+            if (!__any_sync(0xFFFFFFFFu, a > 0)) continue;
+#pragma unroll
+            for (int dy = -1; dy <= 1; ++dy) {
+#pragma unroll
+                for (int dx = -1; dx <= 1; ++dx) {
+                    if ((CONN == 6 && (dy || dx)) || (CONN == 18 && dy && dx)) continue;
+                    const int ny = y + dy, nx = x + dx;
+                    const int b = (a > 0 && ny >= 0 && ny < g.h && nx >= 0 && nx < g.w) ? __ldg(Lp + (size_t)ny * g.w + nx) : 0;
+                    const int pa = __shfl_up_sync(0xFFFFFFFFu, a, 1), pb = __shfl_up_sync(0xFFFFFFFFu, b, 1);
+                    if (b > 0 && !(lx > 0 && pa == a && pb == b) && !(a == last_a && b == last_b)) {
+                        union_g(P, gc + a, gp + b);
+                        last_a = a;
+                        last_b = b;
+                    }
+                }
+            }
+        }
+    }
+}
+
+// ---- 8. roots and their flags (ids[C] = 0, so that the inclusive scan leaves K there) ---------------------------
+__global__ void __launch_bounds__(256) movie_roots_kernel(long long* __restrict__ P, long long* __restrict__ ids, long long C)
+{
+    for (long long c = (long long)blockIdx.x * blockDim.x + threadIdx.x; c <= C; c += (long long)gridDim.x * blockDim.x) {
+        if (c == C) {
+            ids[C] = 0;
+            continue;
+        }
+        const long long r = find_g(P, c);
+        if (r != c) __stcg(P + c, r);
+        ids[c] = r == c;
+    }
+}
+
+// ---- 9. event numbers of the non-roots, the count, the statistics rows reset -------------------------------------
+__global__ void __launch_bounds__(256)
+movie_number_kernel(const long long* __restrict__ P, long long* __restrict__ ids, long long C, int* __restrict__ count,
+                    long long* __restrict__ stats, int cap)
+{
+    const long long K = ids[C];
+    const long long rows = K < cap ? K : cap;
+    const long long n = C > rows ? C : rows;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+        if (i == 0) *count = (int)K;  // the launcher has checked K <= INT_MAX
+        if (i < C) {
+            const long long r = root_of(P, i);
+            if (r != i) ids[i] = ids[r];
+        }
+        if (stats && i < rows) {
+            long long* row = stats + i * LM_COLS;
+            row[0] = 0;
+            row[1] = LLONG_MAX;  // t first
+            row[2] = -1;         // t last
+            row[3] = row[4] = LLONG_MAX;
+            row[5] = row[6] = -1;
+            row[7] = row[8] = row[9] = row[10] = row[11] = row[12] = 0;
+        }
+    }
+}
+
+// ---- 10. labels in place + statistics ----------------------------------------------------------------------------
+// A 32 x 32 tile holds at most 512 2-D components, so a hash of LB_TPX event slots (linear probing) never fills.
+__device__ __forceinline__ int movie_slot(int* keys, int e)
+{
+    int s = (int)(((unsigned)e * 2654435761u) >> 22);  // LB_TPX = 2^10 slots
+    for (;;) {
+        const int k = atomicCAS(keys + s, 0, e);
+        if (k == 0 || k == e) return s;
+        s = (s + 1) & (LB_TPX - 1);
+    }
+}
+__device__ __forceinline__ void movie_slot_reset(int* keys, unsigned (*acc)[LB_TPX], int k)
+{
+    keys[k] = 0;
+#pragma unroll
+    for (int a = 0; a < A_COUNT; ++a) acc[a][k] = (a == A_XMIN || a == A_YMIN) ? 0xFFFFFFFFu : 0u;
+}
+
+template <bool STATS>
+__global__ void __launch_bounds__(LB_TW* LB_BY)
+movie_final_kernel(const u16* __restrict__ frames, LabelGeom g, int* __restrict__ labels, const long long* __restrict__ base,
+                   const long long* __restrict__ ids, long long* __restrict__ stats, int cap, long long items)
+{
+    __shared__ int keys[STATS ? LB_TPX : 1];
+    __shared__ unsigned acc[STATS ? A_COUNT : 1][STATS ? LB_TPX : 1];
+    const int lx = threadIdx.x, tid = threadIdx.y * LB_TW + lx;
+    if constexpr (STATS) {
+        for (int k = tid; k < LB_TPX; k += LB_TW * LB_BY) movie_slot_reset(keys, acc, k);
+        __syncthreads();
+    }
+    for (long long wi = blockIdx.x; wi < items; wi += gridDim.x) {
+        const long long t = wi / g.tiles;
+        const int tile = (int)(wi - t * g.tiles);
+        const int tx0 = (tile % g.tiles_x) * LB_TW, ty0 = (tile / g.tiles_x) * LB_TH;
+        int* L = labels + t * g.npx;
+        const long long* id = ids + base[t] - 1;  // id[l]: the event of 2-D component l of frame t
+        const int x = tx0 + lx;
+        for (int ly = threadIdx.y; ly < LB_TH; ly += LB_BY) {
+            const int y = ty0 + ly;
+            const size_t p = (size_t)y * g.w + x;
+            const int l = (x < g.w && y < g.h) ? L[p] : 0;
+            const int e = l > 0 ? (int)id[l] : 0;
+            if (l > 0) L[p] = e;
+            if constexpr (STATS) {
+                // the lanes of one event in this row: one leader folds them into the event's slot
+                const unsigned grp = __match_any_sync(0xFFFFFFFFu, e);
+                if (e > 0) {
+                    const unsigned val = frames[t * g.npx + p];
+                    const unsigned sx = __reduce_add_sync(grp, (unsigned)lx);
+                    const unsigned sv = __reduce_add_sync(grp, val);
+                    const unsigned key = __reduce_max_sync(grp, val << 10 | (unsigned)(LB_TPX - 1 - (ly * LB_TW + lx)));
+                    if (lx == __ffs(grp) - 1) {
+                        const int s = movie_slot(keys, e);
+                        const unsigned vol = __popc(grp);
+                        atomicAdd(&acc[A_AREA][s], vol);
+                        atomicAdd(&acc[A_SX][s], sx);
+                        atomicAdd(&acc[A_SY][s], vol * ly);
+                        atomicAdd(&acc[A_SV][s], sv);
+                        atomicMin(&acc[A_XMIN][s], (unsigned)lx);
+                        atomicMin(&acc[A_YMIN][s], (unsigned)ly);
+                        atomicMax(&acc[A_XMAX][s], (unsigned)(31 - __clz(grp)));
+                        atomicMax(&acc[A_YMAX][s], (unsigned)ly);
+                        atomicMax(&acc[A_KEY][s], key);
+                    }
+                }
+            }
+        }
+        if constexpr (STATS) {
+            __syncthreads();
+            for (int k = tid; k < LB_TPX; k += LB_TW * LB_BY) {
+                const int e = keys[k];
+                if (!e) continue;
+                if (e <= cap) {
+                    long long* r = stats + (size_t)(e - 1) * LM_COLS;
+                    const unsigned long long vol = acc[A_AREA][k];
+                    atomicAdd((unsigned long long*)r + 0, vol);
+                    atomicMin(r + 1, t);
+                    atomicMax(r + 2, t);
+                    atomicMin(r + 3, (long long)(tx0 + (int)acc[A_XMIN][k]));
+                    atomicMin(r + 4, (long long)(ty0 + (int)acc[A_YMIN][k]));
+                    atomicMax(r + 5, (long long)(tx0 + (int)acc[A_XMAX][k]));
+                    atomicMax(r + 6, (long long)(ty0 + (int)acc[A_YMAX][k]));
+                    atomicAdd((unsigned long long*)r + 7, vol * (unsigned long long)t);
+                    atomicAdd((unsigned long long*)r + 8, (unsigned long long)acc[A_SX][k] + vol * tx0);
+                    atomicAdd((unsigned long long*)r + 9, (unsigned long long)acc[A_SY][k] + vol * ty0);
+                    atomicAdd((unsigned long long*)r + 10, (unsigned long long)acc[A_SV][k]);
+                    const unsigned key = acc[A_KEY][k];
+                    const int li = LB_TPX - 1 - (int)(key & (LB_TPX - 1));
+                    const unsigned long long at = (unsigned long long)t * g.npx + (unsigned long long)(ty0 + li / LB_TW) * g.w + tx0 + li % LB_TW;
+                    // column 11 holds (max value << 48 | 2^48 - 1 - argmax) until movie_stats_split_kernel
+                    atomicMax((unsigned long long*)r + 11, (unsigned long long)(key >> 10) << 48 | (LM_IDX_MASK - at));
+                }
+                movie_slot_reset(keys, acc, k);
+            }
+            __syncthreads();
+        }
+    }
+}
+
+// ---- 11. the packed (max value, argmax) column -> columns 11 and 12 -----------------------------------------------
+__global__ void __launch_bounds__(256) movie_stats_split_kernel(long long* __restrict__ stats, const long long* __restrict__ K, int cap)
+{
+    const long long rows = *K < cap ? *K : cap;
+    for (long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x; r < rows; r += (long long)gridDim.x * blockDim.x) {
+        long long* row = stats + r * LM_COLS;
+        const unsigned long long key = (unsigned long long)row[11];
+        row[11] = (long long)(key >> 48);
+        row[12] = (long long)(LM_IDX_MASK - (key & LM_IDX_MASK));
+    }
+}
+
+int launch_label_movie(const u16* frames, int w, int h, long long nframes, const u16* thr, int per_frame_thr, int connectivity,
+                       int* labels, int* count, long long* stats, int cap, cudaStream_t st)
+{
+    const LabelGeom g = label_geom(w, h);
+    if (cap <= 0) stats = nullptr;
+    // slot 9: K_t [n] | base [n + 1] | the scan's work space
+    const long long n1 = nframes + 1;
+    size_t tmp1 = 0;
+    RIRB_CUDA_OK(cub::DeviceScan::ExclusiveSum(nullptr, tmp1, (long long*)nullptr, n1, st));
+    const size_t o_base = align256((size_t)nframes * sizeof(int)), o_tmp1 = o_base + align256((size_t)n1 * sizeof(long long));
+    char* s9 = (char*)scratch_buffer(9, o_tmp1 + tmp1);
+    if (!s9) return -1;
+    int* kt = (int*)s9;
+    long long* base = (long long*)(s9 + o_base);
+    if (launch_label(frames, w, h, nframes, thr, per_frame_thr, connectivity == 6 ? 4 : 8, labels, kt, nullptr, 0, st) != 0)
+        return -1;
+    RIRB_LAUNCH(movie_widen_kernel, flat_grid(n1), 256, 0, st, kt, base, nframes);
+    RIRB_CUDA_OK(cub::DeviceScan::ExclusiveSum(s9 + o_tmp1, tmp1, base, n1, st));
+    long long C = 0;  // 2-D components of the whole movie: the one read-back every call waits for
+    RIRB_CUDA_OK(cudaMemcpyAsync(&C, base + nframes, sizeof C, cudaMemcpyDeviceToHost, st));
+    RIRB_CUDA_OK(cudaStreamSynchronize(st));
+    if (C == 0) {  // nothing above the thresholds: every label is already 0
+        RIRB_CUDA_OK(cudaMemsetAsync(count, 0, sizeof(int), st));
+        return 0;
+    }
+    // slot 10: parents [C]; slot 11: root flags -> event ids [C + 1] | the scan's work space
+    size_t tmp2 = 0;
+    RIRB_CUDA_OK(cub::DeviceScan::InclusiveSum(nullptr, tmp2, (long long*)nullptr, C + 1, st));
+    const size_t o_tmp2 = align256((size_t)(C + 1) * sizeof(long long));
+    long long* P = (long long*)scratch_buffer(10, (size_t)C * sizeof(long long));
+    char* s11 = (char*)scratch_buffer(11, o_tmp2 + tmp2);
+    if (!P || !s11) return -1;
+    long long* ids = (long long*)s11;
+    const dim3 tile_block(LB_TW, LB_BY);
+    RIRB_LAUNCH(movie_init_kernel, flat_grid(C), 256, 0, st, P, C);
+    if (nframes > 1) {
+        const long long items = (nframes - 1) * g.tiles;
+        if (connectivity == 6)
+            RIRB_LAUNCH(movie_link_kernel<6>, tile_grid(items), tile_block, 0, st, g, labels, base, P, items);
+        else if (connectivity == 18)
+            RIRB_LAUNCH(movie_link_kernel<18>, tile_grid(items), tile_block, 0, st, g, labels, base, P, items);
+        else
+            RIRB_LAUNCH(movie_link_kernel<26>, tile_grid(items), tile_block, 0, st, g, labels, base, P, items);
+    }
+    RIRB_LAUNCH(movie_roots_kernel, flat_grid(C + 1), 256, 0, st, P, ids, C);
+    RIRB_CUDA_OK(cub::DeviceScan::InclusiveSum(s11 + o_tmp2, tmp2, ids, C + 1, st));
+    if (C > INT_MAX) {  // only then can the events outnumber a 32-bit label
+        long long K = 0;
+        RIRB_CUDA_OK(cudaMemcpyAsync(&K, ids + C, sizeof K, cudaMemcpyDeviceToHost, st));
+        RIRB_CUDA_OK(cudaStreamSynchronize(st));
+        if (K > INT_MAX) {
+            set_error("label_movie: %lld events, more than an int32 label can number", K);
+            return -1;
+        }
+    }
+    RIRB_LAUNCH(movie_number_kernel, flat_grid(C > cap ? C : cap), 256, 0, st, P, ids, C, count, stats, cap);
+    const long long items = nframes * g.tiles;
+    if (stats) {
+        RIRB_LAUNCH(movie_final_kernel<true>, tile_grid(items), tile_block, 0, st, frames, g, labels, base, ids, stats, cap, items);
+        RIRB_LAUNCH(movie_stats_split_kernel, flat_grid(cap), 256, 0, st, stats, ids + C, cap);
+    } else {
+        RIRB_LAUNCH(movie_final_kernel<false>, tile_grid(items), tile_block, 0, st, frames, g, labels, base, ids, stats, cap, items);
     }
     return 0;
 }

@@ -287,17 +287,7 @@ def label_batch(frames, threshold, connectivity=8, max_components=256, labels=No
     _prepare_device_call(frames)
     frames = _operand(frames, what, "frames", dtype=np.uint16, copy=True)
     n, h, w = frames.shape
-    if _is_torch(threshold):
-        thr = _operand(threshold.reshape(-1), what, "threshold", dtype=np.uint16)
-        nt = thr.numel()
-    else:
-        t = np.asarray(threshold).reshape(-1)
-        if t.size and (not np.all(np.isfinite(t)) or np.any(t != np.floor(t)) or t.min() < 0 or t.max() > 65535):
-            raise RuntimeError(f"{what}: thresholds must be integers in [0, 65535]")
-        thr = np.ascontiguousarray(t, dtype=np.uint16)
-        nt = thr.size
-    if nt not in (1, n):
-        raise RuntimeError(f"{what}: {nt} thresholds for {n} frames")
+    thr, nt = _label_thresholds(threshold, what, n)
     if _is_torch(frames):
         import torch
 
@@ -315,6 +305,71 @@ def label_batch(frames, threshold, connectivity=8, max_components=256, labels=No
                              max_components)
     _lib.check(r, what)
     return labels, counts, stats
+
+
+def _label_thresholds(threshold, what, n):
+    """``threshold`` of a labelling call: one uint16 value or one per frame, as a dense host array or a device tensor."""
+    if _is_torch(threshold):
+        thr = _operand(threshold.reshape(-1), what, "threshold", dtype=np.uint16)
+        nt = thr.numel()
+    else:
+        t = np.asarray(threshold).reshape(-1)
+        if t.size and (not np.all(np.isfinite(t)) or np.any(t != np.floor(t)) or t.min() < 0 or t.max() > 65535):
+            raise RuntimeError(f"{what}: thresholds must be integers in [0, 65535]")
+        thr = np.ascontiguousarray(t, dtype=np.uint16)
+        nt = thr.size
+    if nt not in (1, n):
+        raise RuntimeError(f"{what}: {nt} thresholds for {n} frames")
+    return thr, nt
+
+
+# columns of the statistics rows of ``label_movie``; the centroid is ``stats[:, EV_SUM_X] / stats[:, EV_VOLUME]`` (likewise
+# t and y) and the duration ``stats[:, EV_T_LAST] - stats[:, EV_T_FIRST] + 1``
+(EV_VOLUME, EV_T_FIRST, EV_T_LAST, EV_X_MIN, EV_Y_MIN, EV_X_MAX, EV_Y_MAX, EV_SUM_T, EV_SUM_X, EV_SUM_Y, EV_SUM_VALUE,
+ EV_MAX_VALUE, EV_ARGMAX) = range(13)
+
+
+def label_movie(frames, threshold, connectivity=26, max_events=256, labels=None):
+    """Events of a uint16 movie ``[n, h, w]``: the connected components of ``frames > threshold`` in space and time, with
+    per-event statistics.
+
+    ``threshold``: a scalar or one value per frame, as for ``label_batch``.  ``connectivity``: 6, 18 or 26 over the axes
+    ``(t, y, x)`` (``scipy.ndimage.generate_binary_structure(3, 1 | 2 | 3)``).  Returns ``(labels, count, stats)``: int32
+    ``labels [n, h, w]`` (0 background, 1..K numbered in raster order of each event's first voxel, as
+    ``scipy.ndimage.label`` on the volume), ``count`` (K, a Python int) and int64 ``stats [max_events, 13]`` whose row
+    ``k - 1`` describes event ``k`` (columns ``EV_VOLUME`` .. ``EV_ARGMAX``; ``EV_ARGMAX`` is ``t * h * w + y * w + x``;
+    rows past ``min(K, max_events)`` are zero).  numpy in gives numpy out; a torch CUDA tensor gives tensors on its
+    device.  ``labels``: an int32 output of the same shape, or None.  The whole movie is one call: two events that merge
+    in a later frame are one event."""
+    lib = _lib.load()
+    what = "label_movie"
+    if len(frames.shape) != 3:
+        raise RuntimeError(f"{what}: wrong input dimension")
+    if connectivity not in (6, 18, 26):
+        raise RuntimeError(f"{what}: connectivity must be 6, 18 or 26, not {connectivity}")
+    if int(max_events) != max_events or max_events < 0:
+        raise RuntimeError(f"{what}: max_events must be a non-negative integer")
+    max_events = int(max_events)
+    _prepare_device_call(frames)
+    frames = _operand(frames, what, "frames", dtype=np.uint16, copy=True)
+    n, h, w = frames.shape
+    thr, nt = _label_thresholds(threshold, what, n)
+    count = np.zeros(1, np.int32)  # the entry waits for its stream, so a host count is ready when it returns
+    if _is_torch(frames):
+        import torch
+
+        if labels is None:
+            labels = torch.empty((n, h, w), dtype=torch.int32, device=frames.device)
+        stats = torch.zeros((max_events, 13), dtype=torch.int64, device=frames.device)
+    else:
+        if labels is None:
+            labels = np.empty((n, h, w), np.int32)
+        stats = np.zeros((max_events, 13), np.int64)
+    labels = _operand(labels, what, "labels", (n, h, w), np.int32)
+    r = lib.rirb_label_movie(_ptr(frames), w, h, n, _ptr(thr), nt, connectivity, _ptr(labels), _ptr(count), _ptr(stats),
+                             max_events)
+    _lib.check(r, what)
+    return labels, int(count[0]), stats
 
 
 # ----------------------------------------------------------------------------------------
@@ -441,6 +496,7 @@ __all__ = [
     "gaussian_filter_batch",
     "find_median_pixel",
     "label_batch",
+    "label_movie",
     "bad_pixels_create",
     "bad_pixels_correct",
     "bad_pixels_correct_batch",
