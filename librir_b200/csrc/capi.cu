@@ -8,7 +8,6 @@
 #include <stdlib.h>
 #include <string.h>
 
-#include <map>
 #include <memory>
 #include <mutex>
 #include <vector>
@@ -27,13 +26,15 @@ std::atomic<long long> g_launches{0};
 struct ThreadState {
     char err[512] = {0};
     cudaStream_t stream = 0;
-    // grow-only device scratch slots for host-pointer callers (never shared between threads)
-    // slots 0-5: operands of the entry that is running; 6-7: bad_pixels_create, which other entries call
-    // 8-11: launchers' own work space (kernels.h: scratch_buffer)
-    static constexpr int SLOTS = 12;
+    // grow-only device work space (never shared between threads), used as a stack: an entry's Call takes slots from `top`
+    // up -- for host operands, and for the work space its launchers ask for (scratch_buffer) -- and gives them back when
+    // it returns, so an entry called inside another starts above its caller's slots.  The deepest call,
+    // rirb_label_movie with every operand on the host, takes 9: five operands and four work buffers.
+    static constexpr int SLOTS = 9;
     void* dev[SLOTS] = {};
     size_t cap[SLOTS] = {};
     int dev_of[SLOTS] = {};
+    int top = 0;  // the first free slot
     bool enqueued = false;  // something of this thread may still be running on `stream` (device-pointer calls do not synchronise)
     ThreadState()
     {
@@ -105,7 +106,7 @@ int sm_count()
 }
 
 // No device -> every compute entry fails loudly: this library has no CPU fallback.
-static int require_device()
+int require_device()
 {
     static std::atomic<int> state{0};  // 0 unknown, 1 ok, -1 none
     int s = state.load();
@@ -125,8 +126,13 @@ static int require_device()
 
 static bool is_device_ptr(const void* p) { return p && operand_on_device(p); }
 
-static void* scratch(int slot, size_t bytes)
+void* scratch_buffer(size_t bytes)
 {
+    if (tls.top == ThreadState::SLOTS) {
+        set_error("out of staging slots: a call needs more than %d device buffers", ThreadState::SLOTS);
+        return nullptr;
+    }
+    const int slot = tls.top++;
     int dev = 0;
     cudaGetDevice(&dev);
     tls.enqueued = true;  // whoever asks for scratch is about to enqueue work that uses it (see rirb_set_stream)
@@ -145,8 +151,6 @@ static void* scratch(int slot, size_t bytes)
     }
     return tls.dev[slot];
 }
-
-void* scratch_buffer(int slot, size_t bytes) { return (slot >= 8 && slot < ThreadState::SLOTS) ? scratch(slot, bytes) : nullptr; }
 
 // ---- pageable host buffers --------------------------------------------------------------------
 // A device->host cudaMemcpyAsync into pageable memory is staged by the driver at ~5 GB/s for one
@@ -242,55 +246,80 @@ static cudaError_t copy_d2h(void* host, const void* dev, size_t bytes, cudaStrea
 
 #undef pin
 
-// Input operand: device pointer as is, host pointer uploaded into scratch slot `slot`.
-static const void* stage_in(const void* p, size_t bytes, int slot, cudaStream_t st)
-{
-    if (is_device_ptr(p)) return p;
-    void* d = scratch(slot, bytes);
-    if (!d) return nullptr;
-    if (copy_h2d(d, p, bytes, st) != cudaSuccess) {
-        set_error("host->device copy failed: %s", cudaGetErrorString(cudaGetLastError()));
-        return nullptr;
-    }
-    return d;
-}
-
-// Output operand: `preload` uploads the caller's current contents first (outputs that are only
-// partially overwritten, e.g. translate's "noborder" strategy or padded planes).
-struct StagedOut {
-    void* dev = nullptr;
-    void* host = nullptr;
-    size_t bytes = 0;
+// ---- the operands of one entry call -----------------------------------------------------------------
+// An entry names each array operand once, with its size; nullptr is an absent operand.  stage() refuses overlapping
+// operands (refuse_overlap, on the memory kind looked up when the operand was named), then gives every host operand a
+// device copy in the thread's work space: inputs, and outputs that are only partly written (preload: translate's
+// "noborder", padded planes, frames corrected in place, accumulated statistics), go up first.  Device and managed
+// operands are used in place.  finish() copies host outputs back and waits for them; a call whose operands are all on
+// the device returns without synchronising.  The slots the call took, its launchers' included, go back when it ends.
+struct Staged : Operand {
+    void* dev = nullptr;  // what the kernels get: p itself, or its copy in the work space
+    bool load = true;     // host input, preloaded host output: stage() uploads it
+    bool staged = true;   // false: only the overlap rule applies, the entry reads or writes the operand itself
 };
-static bool stage_out(StagedOut& o, void* p, size_t bytes, int slot, bool preload, cudaStream_t st)
-{
-    o.bytes = bytes;
-    if (is_device_ptr(p)) {
-        o.dev = p;
-        o.host = nullptr;
-        return true;
-    }
-    o.host = p;
-    o.dev = scratch(slot, bytes);
-    if (!o.dev) return false;
-    if (preload && copy_h2d(o.dev, p, bytes, st) != cudaSuccess) {
-        set_error("host->device copy failed: %s", cudaGetErrorString(cudaGetLastError()));
-        return false;
-    }
-    return true;
-}
-// Copies staged outputs back and waits; device-pointer outputs return without synchronising.
-static int finish_out(StagedOut* outs, int n, cudaStream_t st)
-{
-    bool any = false;
-    for (int i = 0; i < n; ++i)
-        if (outs[i].host && outs[i].bytes) {
-            RIRB_CUDA_OK(copy_d2h(outs[i].host, outs[i].dev, outs[i].bytes, st));
-            any = true;
+class Call {
+  public:
+    explicit Call(const char* what) : what_(what), base_(tls.top) {}
+    ~Call() { tls.top = base_; }
+    Call(const Call&) = delete;
+    Call& operator=(const Call&) = delete;
+    Staged& in(const char* name, const void* p, size_t bytes) { return add(ins_, nin_, name, p, bytes, true); }
+    Staged& out(const char* name, void* p, size_t bytes, bool preload = false) { return add(outs_, nout_, name, p, bytes, preload); }
+    int stage()
+    {
+        if (nin_ > MAX || nout_ > MAX) {
+            set_error("%s: more than %d inputs or outputs", what_, MAX);
+            return -1;
         }
-    if (any) RIRB_CUDA_OK(cudaStreamSynchronize(st));
-    return 0;
-}
+        if (refuse_overlap(what_, ins_, ins_ + nin_, outs_, outs_ + nout_)) return -1;
+        for (int i = 0; i < nin_ + nout_; ++i) {
+            Staged& o = i < nin_ ? ins_[i] : outs_[i - nin_];
+            if (!o.p || o.on_device || !o.staged) {
+                o.dev = o.on_device ? (void*)o.p : nullptr;
+                continue;
+            }
+            if (!(o.dev = scratch_buffer(o.bytes))) return -1;
+            if (o.load && copy_h2d(o.dev, o.p, o.bytes, st_) != cudaSuccess) {
+                set_error("host->device copy failed: %s", cudaGetErrorString(cudaGetLastError()));
+                return -1;
+            }
+        }
+        return 0;
+    }
+    // sync: wait for the stream even when every output is on the device (the entry's own host buffers are being read)
+    int finish(bool sync = false)
+    {
+        for (int i = 0; i < nout_; ++i) {
+            const Staged& o = outs_[i];
+            if (o.p && !o.on_device && o.staged && o.bytes) {
+                RIRB_CUDA_OK(copy_d2h((void*)o.p, o.dev, o.bytes, st_));
+                sync = true;
+            }
+        }
+        if (sync) RIRB_CUDA_OK(cudaStreamSynchronize(st_));
+        return 0;
+    }
+
+  private:
+    static constexpr int MAX = 4;
+    Staged& add(Staged* list, int& n, const char* name, const void* p, size_t bytes, bool load)
+    {
+        Staged& o = list[n < MAX ? n : MAX - 1];  // stage() refuses a call that names too many
+        ++n;
+        o.name = name;
+        o.p = p;
+        o.bytes = bytes;
+        o.on_device = is_device_ptr(p);
+        o.load = load;
+        return o;
+    }
+    const char* what_;
+    const int base_;
+    const cudaStream_t st_ = tls.stream;
+    Staged ins_[MAX], outs_[MAX];
+    int nin_ = 0, nout_ = 0;
+};
 
 static int strategy_code(const char* s)
 {
@@ -313,8 +342,8 @@ static size_t dtype_size(int type)
 }
 
 // ------------------------------------------------------------------------------------------------
-// bad-pixel handle table (the reference's set_void_ptr / get_void_ptr / rm_void_ptr, tools.cpp:40-85:
-// process-global, mutex-guarded, lowest free positive slot)
+// bad-pixel handle table (the reference's set_void_ptr / get_void_ptr / rm_void_ptr, tools.cpp:40-85: process-global,
+// handles.h's Table)
 // ------------------------------------------------------------------------------------------------
 struct BadPixelState {
     int w = 0, h = 0, device = 0;
@@ -335,44 +364,7 @@ struct BadPixelState {
         if (row_off_dev) cudaFree(row_off_dev);
     }
 };
-static std::mutex g_handles_mutex;
-static std::map<int, std::shared_ptr<BadPixelState>> g_handles;
-
-static int register_handle(std::shared_ptr<BadPixelState> s)
-{
-    std::lock_guard<std::mutex> lock(g_handles_mutex);
-    int id = 1;
-    for (auto& kv : g_handles) {
-        if (kv.first != id) break;
-        ++id;
-    }
-    g_handles[id] = s;
-    return id;
-}
-static std::shared_ptr<BadPixelState> find_handle(int id)
-{
-    std::lock_guard<std::mutex> lock(g_handles_mutex);
-    auto it = g_handles.find(id);
-    return it == g_handles.end() ? nullptr : it->second;
-}
-
-// A handle's tables live in the memory of the device it was created on: entries that launch kernels refuse a handle
-// from another device instead of faulting on its pointers.
-static std::shared_ptr<BadPixelState> find_handle_here(int id, const char* what)
-{
-    auto s = find_handle(id);
-    if (!s) {
-        set_error("%s: unknown handle %d", what, id);
-        return nullptr;
-    }
-    int dev = -1;
-    if (cudaGetDevice(&dev) != cudaSuccess) cudaGetLastError();
-    if (dev != s->device) {
-        set_error("%s: handle %d belongs to CUDA device %d, the calling thread is on device %d", what, id, s->device, dev);
-        return nullptr;
-    }
-    return s;
-}
+static Table<BadPixelState> g_bad_pixels;
 
 // ------------------------------------------------------------------------------------------------
 // forwarding of out-of-scope entries to a reference build
@@ -486,12 +478,15 @@ int rirb_translate_batch(int type, const void* src, void* dst, int w, int h, lon
     RIRB_REQUIRE_DEVICE();
     const size_t bytes = (size_t)w * h * esize * (size_t)nframes;
     const size_t sbytes = sizeof(float) * (size_t)n_shifts;
-    if (refuse_overlap("translate", {{"src", src, bytes}, {"dx", dx, sbytes}, {"dy", dy, sbytes}}, {{"dst", dst, bytes}})) return -1;
+    Call c("translate");
+    auto& in = c.in("src", src, bytes);
+    auto& ddx = c.in("dx", dx, sbytes);
+    auto& ddy = c.in("dy", dy, sbytes);
+    auto& out = c.out("dst", dst, bytes, strat == STRAT_NOBORDER);
+    const bool host_scalar = n_shifts == 1 && !ddx.on_device && !ddy.on_device;  // read here, not uploaded
+    ddx.staged = ddy.staged = !host_scalar;
+    if (c.stage() != 0) return -1;
     cudaStream_t st = tls.stream;
-    const void* d_src = stage_in(src, bytes, 0, st);
-    if (!d_src) return -1;
-    StagedOut out;
-    if (!stage_out(out, dst, bytes, 1, strat == STRAT_NOBORDER, st)) return -1;
     // background: one element, host or device
     unsigned long long bg = 0;
     if (is_device_ptr(background)) {
@@ -500,15 +495,12 @@ int rirb_translate_batch(int type, const void* src, void* dst, int w, int h, lon
     } else {
         memcpy(&bg, background, esize);
     }
-    const float *d_dx = nullptr, *d_dy = nullptr;
+    const float *d_dx = (const float*)ddx.dev, *d_dy = (const float*)ddy.dev;
     float dx0 = 0.f, dy0 = 0.f;
-    if (n_shifts == 1 && !is_device_ptr(dx) && !is_device_ptr(dy)) {
+    if (host_scalar) {
         dx0 = dx[0];
         dy0 = dy[0];
     } else {
-        d_dx = (const float*)stage_in(dx, sizeof(float) * (size_t)n_shifts, 2, st);
-        d_dy = (const float*)stage_in(dy, sizeof(float) * (size_t)n_shifts, 3, st);
-        if (!d_dx || !d_dy) return -1;
         if (n_shifts == 1 && nframes > 1) {  // broadcast a device-resident scalar shift
             float tmp[2];
             RIRB_CUDA_OK(cudaMemcpyAsync(&tmp[0], d_dx, sizeof(float), cudaMemcpyDeviceToHost, st));
@@ -519,8 +511,8 @@ int rirb_translate_batch(int type, const void* src, void* dst, int w, int h, lon
             d_dx = d_dy = nullptr;
         }
     }
-    if (launch_translate(type, d_src, out.dev, w, h, nframes, d_dx, d_dy, dx0, dy0, strat, &bg, st) != 0) return -1;
-    return finish_out(&out, 1, st);
+    if (launch_translate(type, in.dev, out.dev, w, h, nframes, d_dx, d_dy, dx0, dy0, strat, &bg, st) != 0) return -1;
+    return c.finish();
 }
 
 int translate(int type, void* src, void* dst, int w, int h, float dx, float dy, void* background, const char* strategy)
@@ -542,16 +534,15 @@ static int gaussian_any(const void* src, bool src_u16, float* dst, int w, int h,
     if (gaussian_taps_host(sigma, &taps) != 0) return -1;
     RIRB_REQUIRE_DEVICE();
     const size_t npx = (size_t)w * h * (size_t)nframes;
-    if (refuse_overlap("gaussian_filter", {{"src", src, npx * (src_u16 ? 2 : 4)}}, {{"dst", dst, npx * 4}})) return -1;
+    Call c("gaussian_filter");
+    auto& in = c.in("src", src, npx * (src_u16 ? 2 : 4));
+    auto& out = c.out("dst", dst, npx * 4);
+    if (c.stage() != 0) return -1;
     cudaStream_t st = tls.stream;
-    const void* d_src = stage_in(src, npx * (src_u16 ? 2 : 4), 0, st);
-    if (!d_src) return -1;
-    StagedOut out;
-    if (!stage_out(out, dst, npx * 4, 1, false, st)) return -1;
-    int rc = src_u16 ? launch_gaussian_u16((const u16*)d_src, (float*)out.dev, w, h, nframes, taps, st)
-                     : launch_gaussian_f32((const float*)d_src, (float*)out.dev, w, h, nframes, taps, st);
+    int rc = src_u16 ? launch_gaussian_u16((const u16*)in.dev, (float*)out.dev, w, h, nframes, taps, st)
+                     : launch_gaussian_f32((const float*)in.dev, (float*)out.dev, w, h, nframes, taps, st);
     if (rc != 0) return -1;
-    return finish_out(&out, 1, st);
+    return c.finish();
 }
 
 int rirb_gaussian_filter_batch(const float* src, float* dst, int w, int h, long long nframes, float sigma)
@@ -585,10 +576,12 @@ int bad_pixels_create(unsigned short* first_image, int width, int height)
         set_error("bad_pixels_create: %s: %s", what, cudaGetErrorString(cudaGetLastError()));
         return 0;
     };
-    const u16* d_img = (const u16*)stage_in(first_image, n * 2, 6, st);
-    if (!d_img) return 0;
+    Call c("bad_pixels_create");
+    auto& img = c.in("first_image", first_image, n * 2);
+    if (c.stage() != 0) return 0;
+    const u16* d_img = (const u16*)img.dev;
     // (i) frame histogram -> median (sorted[N/2]) and spread, as Filters.h:145-160 / BadPixels.cpp:19-31
-    unsigned* d_hist = (unsigned*)scratch(7, 65536 * sizeof(unsigned));
+    unsigned* d_hist = (unsigned*)scratch_buffer(sizeof(unsigned) * 65536);
     if (!d_hist) return 0;
     if (launch_hist_frame(d_img, n, d_hist, st) != 0) return 0;
     std::vector<unsigned> hist(65536);
@@ -703,12 +696,12 @@ int bad_pixels_create(unsigned short* first_image, int width, int height)
         }
     }
     if (cudaStreamSynchronize(st) != cudaSuccess) return fail("sync");
-    return register_handle(state);
+    return g_bad_pixels.add(state);
 }
 
 int rirb_bad_pixels_correct_batch(int handle, const unsigned short* in, unsigned short* out, long long nframes)
 {
-    auto s = find_handle_here(handle, "bad_pixels_correct");
+    auto s = find_handle_here(g_bad_pixels, handle, "bad_pixels_correct");
     if (!s) return -1;
     if (!in || !out || nframes < 0) {
         set_error("bad_pixels_correct: bad arguments");
@@ -719,21 +712,21 @@ int rirb_bad_pixels_correct_batch(int handle, const unsigned short* in, unsigned
     cudaStream_t st = tls.stream;
     const size_t fpx = (size_t)s->w * s->h;
     const size_t bytes = fpx * 2 * (size_t)nframes;
-    if (in != out && refuse_overlap("bad_pixels_correct", {{"in", in, bytes}}, {{"out", out, bytes}})) return -1;
+    Call c("bad_pixels_correct");
     if (in == out) {  // sequential in-place meaning of the reference (BadPixels.cpp:41-59)
-        StagedOut io;
-        if (!stage_out(io, out, bytes, 0, true, st)) return -1;
+        auto& io = c.out("out", out, bytes, true);
+        if (c.stage() != 0) return -1;
         if (launch_bp_correct_inplace((u16*)io.dev, s->xy_dev, (int)(s->xy.size() / 2), s->w, s->h, s->clamp_value, nframes, fpx,
                                       st) != 0)
             return -1;
-        return finish_out(&io, 1, st);
+        return c.finish();
     }
-    const u16* d_in = (const u16*)stage_in(in, bytes, 0, st);
-    if (!d_in) return -1;
-    StagedOut o;
-    if (!stage_out(o, out, bytes, 1, false, st)) return -1;
-    if (launch_bp_correct(d_in, (u16*)o.dev, s->xy_dev, s->span_off_dev, s->w, s->h, s->clamp_value, nframes, fpx, st) != 0) return -1;
-    return finish_out(&o, 1, st);
+    auto& i = c.in("in", in, bytes);
+    auto& o = c.out("out", out, bytes);
+    if (c.stage() != 0) return -1;
+    if (launch_bp_correct((const u16*)i.dev, (u16*)o.dev, s->xy_dev, s->span_off_dev, s->w, s->h, s->clamp_value, nframes, fpx, st) != 0)
+        return -1;
+    return c.finish();
 }
 
 // bad_pixels_correct + gaussian_filter of the corrected frames, reading the movie once (gaussian.cu, BpFuse):
@@ -742,7 +735,7 @@ int rirb_bad_pixels_correct_batch(int handle, const unsigned short* in, unsigned
 int rirb_bad_pixels_correct_gaussian_batch(int handle, const unsigned short* in, unsigned short* corrected, float* smoothed,
                                            long long nframes, float sigma)
 {
-    auto s = find_handle_here(handle, "bad_pixels_correct_gaussian");
+    auto s = find_handle_here(g_bad_pixels, handle, "bad_pixels_correct_gaussian");
     if (!s) return -1;
     if (!in || !corrected || !smoothed || nframes < 0) {
         set_error("bad_pixels_correct_gaussian: bad arguments");
@@ -756,23 +749,21 @@ int rirb_bad_pixels_correct_gaussian_batch(int handle, const unsigned short* in,
     const size_t fpx = (size_t)s->w * s->h;
     // in place is not supported here: the filter reads corrected pixels of neighbouring rows that the correction of other
     // blocks may not have written yet
-    if (refuse_overlap("bad_pixels_correct_gaussian", {{"in", in, fpx * 2 * (size_t)nframes}},
-                       {{"corrected", corrected, fpx * 2 * (size_t)nframes}, {"smoothed", smoothed, fpx * 4 * (size_t)nframes}}))
-        return -1;
-    const u16* d_in = (const u16*)stage_in(in, fpx * 2 * (size_t)nframes, 0, st);
-    if (!d_in) return -1;
-    StagedOut o[2];
-    if (!stage_out(o[0], corrected, fpx * 2 * (size_t)nframes, 1, false, st)) return -1;
-    if (!stage_out(o[1], smoothed, fpx * 4 * (size_t)nframes, 2, false, st)) return -1;
-    const int rc = launch_gaussian_bp_u16(d_in, (u16*)o[0].dev, (float*)o[1].dev, s->w, s->h, nframes, taps, s->xy_dev, s->row_off_dev,
+    Call c("bad_pixels_correct_gaussian");
+    auto& i = c.in("in", in, fpx * 2 * (size_t)nframes);
+    auto& cor = c.out("corrected", corrected, fpx * 2 * (size_t)nframes);
+    auto& sm = c.out("smoothed", smoothed, fpx * 4 * (size_t)nframes);
+    if (c.stage() != 0) return -1;
+    const u16* d_in = (const u16*)i.dev;
+    const int rc = launch_gaussian_bp_u16(d_in, (u16*)cor.dev, (float*)sm.dev, s->w, s->h, nframes, taps, s->xy_dev, s->row_off_dev,
                                           s->clamp_value, st);
     if (rc < 0) return -1;
     if (rc == 1) {
-        if (launch_bp_correct(d_in, (u16*)o[0].dev, s->xy_dev, s->span_off_dev, s->w, s->h, s->clamp_value, nframes, fpx, st) != 0 ||
-            launch_gaussian_u16((const u16*)o[0].dev, (float*)o[1].dev, s->w, s->h, nframes, taps, st) != 0)
+        if (launch_bp_correct(d_in, (u16*)cor.dev, s->xy_dev, s->span_off_dev, s->w, s->h, s->clamp_value, nframes, fpx, st) != 0 ||
+            launch_gaussian_u16((const u16*)cor.dev, (float*)sm.dev, s->w, s->h, nframes, taps, st) != 0)
             return -1;
     }
-    return finish_out(o, 2, st);
+    return c.finish();
 }
 
 int bad_pixels_correct(int handle, unsigned short* in, unsigned short* out)
@@ -780,15 +771,11 @@ int bad_pixels_correct(int handle, unsigned short* in, unsigned short* out)
     return rirb_bad_pixels_correct_batch(handle, in, out, 1);
 }
 
-void bad_pixels_destroy(int handle)
-{
-    std::lock_guard<std::mutex> lock(g_handles_mutex);
-    g_handles.erase(handle);
-}
+void bad_pixels_destroy(int handle) { g_bad_pixels.remove(handle); }
 
 int rirb_bad_pixels_count(int handle)
 {
-    auto s = find_handle(handle);
+    auto s = g_bad_pixels.get(handle);
     if (!s) {
         set_error("bad_pixels: unknown handle %d", handle);
         return -1;
@@ -798,7 +785,7 @@ int rirb_bad_pixels_count(int handle)
 
 int rirb_bad_pixels_get(int handle, int* xy, int capacity, int* clamp_value)
 {
-    auto s = find_handle(handle);
+    auto s = g_bad_pixels.get(handle);
     if (!s) {
         set_error("bad_pixels: unknown handle %d", handle);
         return -1;
@@ -814,7 +801,7 @@ int rirb_bad_pixels_get(int handle, int* xy, int capacity, int* clamp_value)
 
 int rirb_loader_remove_bad_pixels(int handle, unsigned short* frames, long long nframes, size_t frame_stride)
 {
-    auto s = find_handle_here(handle, "remove_bad_pixels");
+    auto s = find_handle_here(g_bad_pixels, handle, "remove_bad_pixels");
     if (!s) return -1;
     if (!frames || nframes < 0 || frame_stride < (size_t)s->w * s->h) {
         set_error("remove_bad_pixels: bad arguments");
@@ -823,16 +810,37 @@ int rirb_loader_remove_bad_pixels(int handle, unsigned short* frames, long long 
     if (nframes == 0) return 0;
     RIRB_REQUIRE_DEVICE();
     cudaStream_t st = tls.stream;
-    StagedOut io;
-    if (!stage_out(io, frames, frame_stride * 2 * (size_t)nframes, 0, true, st)) return -1;
+    Call c("remove_bad_pixels");
+    auto& io = c.out("frames", frames, frame_stride * 2 * (size_t)nframes, true);
+    if (c.stage() != 0) return -1;
     if (launch_loader_bp((u16*)io.dev, s->xy_dev, s->mask_dev, (int)(s->xy.size() / 2), s->w, s->h, nframes, frame_stride, st) != 0)
         return -1;
-    return finish_out(&io, 1, st);
+    return c.finish();
 }
 
 // =================================================================================================
 // motion-correction variant
 // =================================================================================================
+// The reader's shifts, translate(..., -x[pos], -y[pos], ...) with float arguments (IRFileLoader.cpp:621): doubles on the
+// host or the device -> f = (float)-x then (float)-y.  The entries stage f as their first input: a small pageable upload
+// queued behind the frames' waits for them (6 us more per one-frame call, B200 at 1000 W).  An asynchronous copy reads f,
+// so the entry waits for its stream before f goes away.
+static int narrow_shifts(const double* x, const double* y, long long n, std::vector<float>& f, cudaStream_t st)
+{
+    std::vector<double> v(2 * (size_t)n);
+    if (is_device_ptr(x) || is_device_ptr(y)) {
+        RIRB_CUDA_OK(cudaMemcpyAsync(v.data(), x, sizeof(double) * n, cudaMemcpyDefault, st));
+        RIRB_CUDA_OK(cudaMemcpyAsync(v.data() + n, y, sizeof(double) * n, cudaMemcpyDefault, st));
+        RIRB_CUDA_OK(cudaStreamSynchronize(st));
+    } else {
+        memcpy(v.data(), x, sizeof(double) * n);
+        memcpy(v.data() + n, y, sizeof(double) * n);
+    }
+    f.resize(v.size());
+    for (size_t i = 0; i < v.size(); ++i) f[i] = (float)(-v[i]);
+    return 0;
+}
+
 int rirb_loader_remove_motion(const unsigned short* in, unsigned short* out, int w, int h, long long nframes, size_t frame_stride,
                               const double* shift_x, const double* shift_y)
 {
@@ -843,53 +851,31 @@ int rirb_loader_remove_motion(const unsigned short* in, unsigned short* out, int
     if (nframes == 0) return 0;
     RIRB_REQUIRE_DEVICE();
     const size_t bytes = frame_stride * 2 * (size_t)nframes;
-    if (in != out && refuse_overlap("remove_motion", {{"in", in, bytes}}, {{"out", out, bytes}})) return -1;
     cudaStream_t st = tls.stream;
-    // shifts: doubles on the host (PointF), negated and narrowed to float as the reference's call does
-    std::vector<double> sx((size_t)nframes), sy((size_t)nframes);
-    if (is_device_ptr(shift_x) || is_device_ptr(shift_y)) {
-        RIRB_CUDA_OK(cudaMemcpyAsync(sx.data(), shift_x, sizeof(double) * nframes, cudaMemcpyDefault, st));
-        RIRB_CUDA_OK(cudaMemcpyAsync(sy.data(), shift_y, sizeof(double) * nframes, cudaMemcpyDefault, st));
-        RIRB_CUDA_OK(cudaStreamSynchronize(st));
-    } else {
-        memcpy(sx.data(), shift_x, sizeof(double) * nframes);
-        memcpy(sy.data(), shift_y, sizeof(double) * nframes);
-    }
-    std::vector<float> fx((size_t)nframes), fy((size_t)nframes);
-    for (long long i = 0; i < nframes; ++i) {
-        fx[i] = (float)(-sx[i]);
-        fy[i] = (float)(-sy[i]);
-    }
-    const float* d_dx = (const float*)stage_in(fx.data(), sizeof(float) * nframes, 2, st);
-    const float* d_dy = (const float*)stage_in(fy.data(), sizeof(float) * nframes, 3, st);
-    if (!d_dx || !d_dy) return -1;
     const bool inplace = (in == out);
-    const u16* d_in;
-    StagedOut o;
+    std::vector<float> f;
+    if (narrow_shifts(shift_x, shift_y, nframes, f, st) != 0) return -1;
+    Call c("remove_motion");
+    auto& sh = c.in("shifts", f.data(), sizeof(float) * f.size());
+    auto& i = c.in("in", inplace ? nullptr : in, bytes);
+    auto& o = c.out("out", out, bytes, inplace);
+    if (c.stage() != 0) return -1;
+    const float* d_dx = (const float*)sh.dev;
+    const u16* d_in = (const u16*)i.dev;
     if (inplace) {
         // the reference translates into a temporary and copies back; keep a private copy of the input
-        if (!stage_out(o, out, bytes, 1, true, st)) return -1;
-        void* copy = scratch(0, bytes);
+        void* copy = scratch_buffer(bytes);
         if (!copy) return -1;
         RIRB_CUDA_OK(cudaMemcpyAsync(copy, o.dev, bytes, cudaMemcpyDeviceToDevice, st));
         d_in = (const u16*)copy;
-    } else {
-        d_in = (const u16*)stage_in(in, bytes, 0, st);
-        if (!d_in) return -1;
-        if (!stage_out(o, out, bytes, 1, false, st)) return -1;
-        if (frame_stride > (size_t)w * h)  // pass the untouched tail rows through
-            RIRB_CUDA_OK(cudaMemcpy2DAsync((u16*)o.dev + (size_t)w * h, frame_stride * 2, d_in + (size_t)w * h, frame_stride * 2,
-                                           (frame_stride - (size_t)w * h) * 2, (size_t)nframes, cudaMemcpyDeviceToDevice, st));
+    } else if (frame_stride > (size_t)w * h) {  // pass the untouched tail rows through
+        RIRB_CUDA_OK(cudaMemcpy2DAsync((u16*)o.dev + (size_t)w * h, frame_stride * 2, d_in + (size_t)w * h, frame_stride * 2,
+                                       (frame_stride - (size_t)w * h) * 2, (size_t)nframes, cudaMemcpyDeviceToDevice, st));
     }
-    if (launch_translate_u16(d_in, (u16*)o.dev, w, h, nframes, frame_stride, frame_stride, d_dx, d_dy, 0.f, 0.f, STRAT_NEAREST, 0u,
-                             true, st) != 0)
+    if (launch_translate_u16(d_in, (u16*)o.dev, w, h, nframes, frame_stride, frame_stride, d_dx, d_dx + nframes, 0.f, 0.f,
+                             STRAT_NEAREST, 0u, true, st) != 0)
         return -1;
-    if (o.host) {
-        RIRB_CUDA_OK(copy_d2h(o.host, o.dev, bytes, st));
-    }
-    // fx/fy are stack-owned host vectors read by an async copy: always wait before returning
-    RIRB_CUDA_OK(cudaStreamSynchronize(st));
-    return 0;
+    return c.finish(true);  // f is read by an asynchronous copy
 }
 
 // =================================================================================================
@@ -908,7 +894,7 @@ int rirb_loader_read_movie(int handle, const unsigned char* lo, const unsigned c
     if (min_T_height == 0) min_T_height = hb;
     std::shared_ptr<BadPixelState> s;
     if (handle != 0) {
-        s = find_handle_here(handle, "loader_read_movie");
+        s = find_handle_here(g_bad_pixels, handle, "loader_read_movie");
         if (!s) return -1;
         if (s->w != w || s->h != hb) {
             set_error("loader_read_movie: the handle was created on a %dx%d image, expected %dx%d", s->w, s->h, w, hb);
@@ -919,13 +905,16 @@ int rirb_loader_read_movie(int handle, const unsigned char* lo, const unsigned c
     cudaStream_t st = tls.stream;
     const size_t fpx = (size_t)w * h;
     const size_t pbytes = fpx * (size_t)nframes;
-    if (refuse_overlap("loader_read_movie", {{"lo", lo, pbytes}, {"hi", hi, pbytes}}, {{"out", out, pbytes * 2}})) return -1;
-    const u8* d_lo = (const u8*)stage_in(lo, pbytes, 0, st);
-    const u8* d_hi = (const u8*)stage_in(hi, pbytes, 1, st);
-    if (!d_lo || !d_hi) return -1;
-    StagedOut o;
-    if (!stage_out(o, out, pbytes * 2, 2, false, st)) return -1;
     const bool motion = shift_x != nullptr;
+    std::vector<float> f;
+    if (motion && narrow_shifts(shift_x, shift_y, nframes, f, st) != 0) return -1;
+    Call c("loader_read_movie");
+    auto& sh = c.in("shifts", motion ? f.data() : nullptr, sizeof(float) * f.size());
+    auto& l = c.in("lo", lo, pbytes);
+    auto& hh = c.in("hi", hi, pbytes);
+    auto& o = c.out("out", out, pbytes * 2);
+    if (c.stage() != 0) return -1;
+    const u8 *d_lo = (const u8*)l.dev, *d_hi = (const u8*)hh.dev;
     const int k = s ? (int)(s->xy.size() / 2) : 0;
     const bool fused_bp = s && k > 0 && w >= 3 && hb >= 3;
     if (!motion) {
@@ -935,26 +924,9 @@ int rirb_loader_read_movie(int handle, const unsigned char* lo, const unsigned c
             return -1;
         if (s && k > 0 && !fused_bp)  // degenerate sizes keep the reference's sequential loop (IRFileLoader.cpp:735-752)
             if (launch_loader_bp(merged, s->xy_dev, s->mask_dev, k, w, hb, nframes, fpx, st) != 0) return -1;
-        return finish_out(&o, 1, st);
+        return c.finish();
     }
-    // shifts: translate(..., -x[pos], -y[pos], ...) with float arguments (IRFileLoader.cpp:621)
-    std::vector<double> sx((size_t)nframes), sy((size_t)nframes);
-    if (is_device_ptr(shift_x) || is_device_ptr(shift_y)) {
-        RIRB_CUDA_OK(cudaMemcpyAsync(sx.data(), shift_x, sizeof(double) * nframes, cudaMemcpyDefault, st));
-        RIRB_CUDA_OK(cudaMemcpyAsync(sy.data(), shift_y, sizeof(double) * nframes, cudaMemcpyDefault, st));
-        RIRB_CUDA_OK(cudaStreamSynchronize(st));
-    } else {
-        memcpy(sx.data(), shift_x, sizeof(double) * nframes);
-        memcpy(sy.data(), shift_y, sizeof(double) * nframes);
-    }
-    std::vector<float> fx((size_t)nframes), fy((size_t)nframes);
-    for (long long i = 0; i < nframes; ++i) {
-        fx[i] = (float)(-sx[i]);
-        fy[i] = (float)(-sy[i]);
-    }
-    const float* d_dx = (const float*)stage_in(fx.data(), sizeof(float) * nframes, 4, st);
-    const float* d_dy = (const float*)stage_in(fy.data(), sizeof(float) * nframes, 5, st);
-    if (!d_dx || !d_dy) return -1;
+    const float *d_dx = (const float*)sh.dev, *d_dy = d_dx + nframes;
     // one pass: planes -> merge -> += min_T -> medians -> motion translate (translate.cu, PLANES)
     const int rows_t = (min_T == 0 || min_T_height < 0) ? 0 : (min_T_height > h ? h : min_T_height);
     int rc = (s && k > 0 && !fused_bp)
@@ -964,7 +936,7 @@ int rirb_loader_read_movie(int handle, const unsigned char* lo, const unsigned c
                                        fused_bp ? s->mask_dev : nullptr, d_dx, d_dy, st);
     if (rc < 0) return -1;
     if (rc == 1) {  // layouts the fused kernel does not take: merge pass, then the motion pass through a scratch movie
-        u16* merged = (u16*)scratch(3, pbytes * 2);
+        u16* merged = (u16*)scratch_buffer(pbytes * 2);
         if (!merged) return -1;
         if (launch_loader_merge(d_lo, d_hi, merged, w, h, hb, nframes, fpx, min_T, min_T_height, fused_bp ? s->xy_dev : nullptr,
                                 fused_bp ? s->span_off_dev : nullptr, fused_bp ? s->nbr_dev : nullptr, st) != 0)
@@ -977,9 +949,7 @@ int rirb_loader_read_movie(int handle, const unsigned char* lo, const unsigned c
         if (launch_translate_u16(merged, (u16*)o.dev, w, hb, nframes, fpx, fpx, d_dx, d_dy, 0.f, 0.f, STRAT_NEAREST, 0u, true, st) != 0)
             return -1;
     }
-    if (o.host) RIRB_CUDA_OK(copy_d2h(o.host, o.dev, o.bytes, st));
-    RIRB_CUDA_OK(cudaStreamSynchronize(st));  // fx / fy are host vectors read by an async copy
-    return 0;
+    return c.finish(true);  // f is read by an asynchronous copy
 }
 
 // The same chain for frames that are uint16 already (decoded from the zstd movie file): += min_T -> removeBadPixels ->
@@ -996,7 +966,7 @@ int rirb_loader_finish_frames(int handle, unsigned short* frames, long long nfra
     if (min_T_height == 0) min_T_height = hb;  // IRFileLoader.cpp:918-921
     std::shared_ptr<BadPixelState> s;
     if (handle != 0) {
-        s = find_handle_here(handle, "loader_finish_frames");
+        s = find_handle_here(g_bad_pixels, handle, "loader_finish_frames");
         if (!s) return -1;
         if (s->w != w || s->h != hb) {
             set_error("loader_finish_frames: the handle was created on a %dx%d image, expected %dx%d", s->w, s->h, w, hb);
@@ -1006,8 +976,9 @@ int rirb_loader_finish_frames(int handle, unsigned short* frames, long long nfra
     RIRB_REQUIRE_DEVICE();
     cudaStream_t st = tls.stream;
     const size_t fpx = (size_t)w * h;
-    StagedOut io;
-    if (!stage_out(io, frames, fpx * 2 * (size_t)nframes, 0, true, st)) return -1;
+    Call c("loader_finish_frames");
+    auto& io = c.out("frames", frames, fpx * 2 * (size_t)nframes, true);
+    if (c.stage() != 0) return -1;
     u16* d = (u16*)io.dev;
     const int rows_t = (min_T == 0 || min_T_height < 0) ? 0 : (min_T_height > h ? h : min_T_height);
     if (launch_loader_add_min(d, w, rows_t, nframes, fpx, min_T, st) != 0) return -1;
@@ -1015,12 +986,12 @@ int rirb_loader_finish_frames(int handle, unsigned short* frames, long long nfra
         if (launch_loader_bp(d, s->xy_dev, s->mask_dev, (int)(s->xy.size() / 2), w, hb, nframes, fpx, st) != 0) return -1;
     if (shift_x) {
         // the motion step is out of place: through a scratch copy, on device pointers (no further staging)
-        u16* tmp = (u16*)scratch(4, fpx * 2 * (size_t)nframes);  // not 0-3: rirb_loader_remove_motion stages its shifts there
+        u16* tmp = (u16*)scratch_buffer(fpx * 2 * (size_t)nframes);
         if (!tmp) return -1;
         RIRB_CUDA_OK(cudaMemcpyAsync(tmp, d, fpx * 2 * (size_t)nframes, cudaMemcpyDeviceToDevice, st));
         if (rirb_loader_remove_motion(tmp, d, w, hb, nframes, fpx, shift_x, shift_y) != 0) return -1;
     }
-    return finish_out(&io, 1, st);
+    return c.finish();
 }
 
 // =================================================================================================
@@ -1034,24 +1005,18 @@ int rirb_split_yuv444(const unsigned short* img, const unsigned char* it, int w,
         return -1;
     }
     RIRB_REQUIRE_DEVICE();
-    if (refuse_overlap("split_yuv444", {{"img", img, (size_t)w * h * 2}, {"it", it, (size_t)w * h}},
-                       {{"y_plane", y_plane, (size_t)ls_y * h}, {"u_plane", u_plane, (size_t)ls_u * h}, {"v_plane", v_plane, (size_t)ls_v * h}}))
-        return -1;
     cudaStream_t st = tls.stream;
-    const u16* d_img = (const u16*)stage_in(img, (size_t)w * h * 2, 0, st);
-    if (!d_img) return -1;
-    const u8* d_it = nullptr;
-    if (it) {
-        d_it = (const u8*)stage_in(it, (size_t)w * h, 1, st);
-        if (!d_it) return -1;
-    }
-    StagedOut o[3];
+    Call c("split_yuv444");
+    auto& im = c.in("img", img, (size_t)w * h * 2);
+    auto& t = c.in("it", it, (size_t)w * h);
     // row padding must survive untouched: preload padded planes
-    if (!stage_out(o[1], u_plane, (size_t)ls_u * h, 3, ls_u != w, st)) return -1;
-    if (!stage_out(o[2], v_plane, (size_t)ls_v * h, 4, ls_v != w, st)) return -1;
-    if (y_plane && !stage_out(o[0], y_plane, (size_t)ls_y * h, 2, ls_y != w, st)) return -1;
-    if (launch_split_planes(d_img, d_it, w, h, (u8*)o[0].dev, (u8*)o[1].dev, (u8*)o[2].dev, ls_y, ls_u, ls_v, st) != 0) return -1;
-    return finish_out(o, 3, st);
+    auto& y = c.out("y_plane", y_plane, (size_t)ls_y * h, ls_y != w);
+    auto& u = c.out("u_plane", u_plane, (size_t)ls_u * h, ls_u != w);
+    auto& v = c.out("v_plane", v_plane, (size_t)ls_v * h, ls_v != w);
+    if (c.stage() != 0) return -1;
+    if (launch_split_planes((const u16*)im.dev, (const u8*)t.dev, w, h, (u8*)y.dev, (u8*)u.dev, (u8*)v.dev, ls_y, ls_u, ls_v, st) != 0)
+        return -1;
+    return c.finish();
 }
 
 int rirb_merge_yuv444(const unsigned char* y_plane, const unsigned char* u_plane, const unsigned char* v_plane, int ls_y, int ls_u,
@@ -1062,24 +1027,18 @@ int rirb_merge_yuv444(const unsigned char* y_plane, const unsigned char* u_plane
         return -1;
     }
     RIRB_REQUIRE_DEVICE();
-    if (refuse_overlap("merge_yuv444",
-                       {{"y_plane", it ? y_plane : nullptr, (size_t)ls_y * h}, {"u_plane", u_plane, (size_t)ls_u * h}, {"v_plane", v_plane, (size_t)ls_v * h}},
-                       {{"img", img, (size_t)w * h * 2}, {"it", y_plane ? it : nullptr, (size_t)w * h}}))
-        return -1;
     cudaStream_t st = tls.stream;
-    const u8* d_u = (const u8*)stage_in(u_plane, (size_t)ls_u * h, 0, st);
-    const u8* d_v = (const u8*)stage_in(v_plane, (size_t)ls_v * h, 1, st);
-    if (!d_u || !d_v) return -1;
-    const u8* d_y = nullptr;
-    if (y_plane && it) {
-        d_y = (const u8*)stage_in(y_plane, (size_t)ls_y * h, 2, st);
-        if (!d_y) return -1;
-    }
-    StagedOut o[2];
-    if (!stage_out(o[0], img, (size_t)w * h * 2, 3, false, st)) return -1;
-    if (it && d_y && !stage_out(o[1], it, (size_t)w * h, 4, false, st)) return -1;
-    if (launch_merge_planes(d_y, d_u, d_v, ls_y, ls_u, ls_v, w, h, (u16*)o[0].dev, (u8*)o[1].dev, st) != 0) return -1;
-    return finish_out(o, 2, st);
+    const bool with_y = y_plane && it;
+    Call c("merge_yuv444");
+    auto& y = c.in("y_plane", with_y ? y_plane : nullptr, (size_t)ls_y * h);
+    auto& u = c.in("u_plane", u_plane, (size_t)ls_u * h);
+    auto& v = c.in("v_plane", v_plane, (size_t)ls_v * h);
+    auto& im = c.out("img", img, (size_t)w * h * 2);
+    auto& t = c.out("it", with_y ? it : nullptr, (size_t)w * h);
+    if (c.stage() != 0) return -1;
+    if (launch_merge_planes((const u8*)y.dev, (const u8*)u.dev, (const u8*)v.dev, ls_y, ls_u, ls_v, w, h, (u16*)im.dev, (u8*)t.dev, st) != 0)
+        return -1;
+    return c.finish();
 }
 
 int rirb_split_yuv420(const unsigned short* img, const unsigned char* it, int w, int h, unsigned char* y_plane, int ls_y,
@@ -1090,26 +1049,18 @@ int rirb_split_yuv420(const unsigned short* img, const unsigned char* it, int w,
         return -1;
     }
     RIRB_REQUIRE_DEVICE();
-    const bool with_it = it && u_plane;
-    if (refuse_overlap("split_yuv420", {{"img", img, (size_t)w * h * 2}, {"it", with_it ? it : nullptr, (size_t)w * h}},
-                       {{"y_plane", y_plane, (size_t)ls_y * 2 * h}, {"u_plane", with_it ? u_plane : nullptr, (size_t)ls_u * h}}))
-        return -1;
     cudaStream_t st = tls.stream;
-    const u16* d_img = (const u16*)stage_in(img, (size_t)w * h * 2, 0, st);
-    if (!d_img) return -1;
-    const u8* d_it = nullptr;
-    if (with_it) {
-        d_it = (const u8*)stage_in(it, (size_t)w * h, 1, st);
-        if (!d_it) return -1;
-    }
-    StagedOut o[2];
-    if (!stage_out(o[0], y_plane, (size_t)ls_y * 2 * h, 2, ls_y != w, st)) return -1;
-    if (with_it && !stage_out(o[1], u_plane, (size_t)ls_u * h, 3, ls_u != w, st)) return -1;
-    u8* d_y = (u8*)o[0].dev;
-    if (launch_split_planes(d_img, d_it, w, h, with_it ? (u8*)o[1].dev : nullptr, d_y, d_y + (size_t)h * ls_y, ls_u, ls_y, ls_y,
-                            st) != 0)
+    const bool with_it = it && u_plane;
+    Call c("split_yuv420");
+    auto& im = c.in("img", img, (size_t)w * h * 2);
+    auto& t = c.in("it", with_it ? it : nullptr, (size_t)w * h);
+    auto& y = c.out("y_plane", y_plane, (size_t)ls_y * 2 * h, ls_y != w);
+    auto& u = c.out("u_plane", with_it ? u_plane : nullptr, (size_t)ls_u * h, ls_u != w);
+    if (c.stage() != 0) return -1;
+    u8* d_y = (u8*)y.dev;
+    if (launch_split_planes((const u16*)im.dev, (const u8*)t.dev, w, h, (u8*)u.dev, d_y, d_y + (size_t)h * ls_y, ls_u, ls_y, ls_y, st) != 0)
         return -1;
-    return finish_out(o, 2, st);
+    return c.finish();
 }
 
 int rirb_merge_yuv420(const unsigned char* y_plane, int ls_y, const unsigned char* u_plane, int ls_u, int w, int h,
@@ -1120,24 +1071,18 @@ int rirb_merge_yuv420(const unsigned char* y_plane, int ls_y, const unsigned cha
         return -1;
     }
     RIRB_REQUIRE_DEVICE();
-    const bool with_it = it && u_plane;
-    if (refuse_overlap("merge_yuv420", {{"y_plane", y_plane, (size_t)ls_y * 2 * h}, {"u_plane", with_it ? u_plane : nullptr, (size_t)ls_u * h}},
-                       {{"img", img, (size_t)w * h * 2}, {"it", with_it ? it : nullptr, (size_t)w * h}}))
-        return -1;
     cudaStream_t st = tls.stream;
-    const u8* d_yp = (const u8*)stage_in(y_plane, (size_t)ls_y * 2 * h, 0, st);
-    if (!d_yp) return -1;
-    const u8* d_up = nullptr;
-    if (with_it) {
-        d_up = (const u8*)stage_in(u_plane, (size_t)ls_u * h, 1, st);
-        if (!d_up) return -1;
-    }
-    StagedOut o[2];
-    if (!stage_out(o[0], img, (size_t)w * h * 2, 2, false, st)) return -1;
-    if (with_it && !stage_out(o[1], it, (size_t)w * h, 3, false, st)) return -1;
-    if (launch_merge_planes(d_up, d_yp, d_yp + (size_t)h * ls_y, ls_u, ls_y, ls_y, w, h, (u16*)o[0].dev, (u8*)o[1].dev, st) != 0)
+    const bool with_it = it && u_plane;
+    Call c("merge_yuv420");
+    auto& y = c.in("y_plane", y_plane, (size_t)ls_y * 2 * h);
+    auto& u = c.in("u_plane", with_it ? u_plane : nullptr, (size_t)ls_u * h);
+    auto& im = c.out("img", img, (size_t)w * h * 2);
+    auto& t = c.out("it", with_it ? it : nullptr, (size_t)w * h);
+    if (c.stage() != 0) return -1;
+    const u8* d_yp = (const u8*)y.dev;
+    if (launch_merge_planes((const u8*)u.dev, d_yp, d_yp + (size_t)h * ls_y, ls_u, ls_y, ls_y, w, h, (u16*)im.dev, (u8*)t.dev, st) != 0)
         return -1;
-    return finish_out(o, 2, st);
+    return c.finish();
 }
 
 int rirb_precode_movie(const unsigned short* movie, long long nframes, int w, int h, int gop, int delta, long long first_frame,
@@ -1151,13 +1096,13 @@ int rirb_precode_movie(const unsigned short* movie, long long nframes, int w, in
     RIRB_REQUIRE_DEVICE();
     cudaStream_t st = tls.stream;
     const size_t n = (size_t)w * h * (size_t)nframes;
-    if (refuse_overlap("precode_movie", {{"movie", movie, n * 2}}, {{"lo", lo, n}, {"hi", hi, n}})) return -1;
-    const u16* d_mov = (const u16*)stage_in(movie, n * 2, 0, st);
-    if (!d_mov) return -1;
-    StagedOut o[2];
-    if (!stage_out(o[0], lo, n, 1, false, st) || !stage_out(o[1], hi, n, 2, false, st)) return -1;
-    if (launch_precode_movie(d_mov, nframes, w, h, gop, delta, first_frame, (u8*)o[0].dev, (u8*)o[1].dev, st) != 0) return -1;
-    return finish_out(o, 2, st);
+    Call c("precode_movie");
+    auto& m = c.in("movie", movie, n * 2);
+    auto& l = c.out("lo", lo, n);
+    auto& hh = c.out("hi", hi, n);
+    if (c.stage() != 0) return -1;
+    if (launch_precode_movie((const u16*)m.dev, nframes, w, h, gop, delta, first_frame, (u8*)l.dev, (u8*)hh.dev, st) != 0) return -1;
+    return c.finish();
 }
 
 int rirb_precode_movie_stats(const unsigned short* movie, long long nframes, int w, int h, int gop, int delta, long long first_frame,
@@ -1171,24 +1116,25 @@ int rirb_precode_movie_stats(const unsigned short* movie, long long nframes, int
     RIRB_REQUIRE_DEVICE();
     cudaStream_t st = tls.stream;
     const size_t n = (size_t)w * h * (size_t)nframes;
-    if (refuse_overlap("precode_movie_stats", {{"movie", movie, n * 2}},
-                       {{"lo", lo, n}, {"hi", hi, n}, {"minmax", minmax, 2 * sizeof(unsigned)}, {"hist", hist, 65536 * sizeof(unsigned long long)}}))
-        return -1;
-    const u16* d_mov = (const u16*)stage_in(movie, n * 2, 0, st);
-    if (!d_mov) return -1;
-    StagedOut o[4];
-    if (!stage_out(o[0], lo, n, 1, false, st) || !stage_out(o[1], hi, n, 2, false, st)) return -1;
-    if (!stage_out(o[2], minmax, 2 * sizeof(unsigned), 3, accumulate != 0, st)) return -1;
-    if (!stage_out(o[3], hist, 65536 * sizeof(unsigned long long), 4, accumulate != 0, st)) return -1;
-    if (!accumulate && launch_stats_init((unsigned*)o[2].dev, (unsigned long long*)o[3].dev, st) != 0) return -1;
-    const int rc = launch_precode_movie_stats(d_mov, nframes, w, h, gop, delta, first_frame, (u8*)o[0].dev, (u8*)o[1].dev,
-                                              (unsigned*)o[2].dev, (unsigned long long*)o[3].dev, st);
+    Call c("precode_movie_stats");
+    auto& m = c.in("movie", movie, n * 2);
+    auto& l = c.out("lo", lo, n);
+    auto& hh = c.out("hi", hi, n);
+    auto& mm = c.out("minmax", minmax, 2 * sizeof(unsigned), accumulate != 0);
+    auto& hs = c.out("hist", hist, 65536 * sizeof(unsigned long long), accumulate != 0);
+    if (c.stage() != 0) return -1;
+    const u16* d_mov = (const u16*)m.dev;
+    u8 *d_lo = (u8*)l.dev, *d_hi = (u8*)hh.dev;
+    unsigned* d_mm = (unsigned*)mm.dev;
+    unsigned long long* d_hist = (unsigned long long*)hs.dev;
+    if (!accumulate && launch_stats_init(d_mm, d_hist, st) != 0) return -1;
+    const int rc = launch_precode_movie_stats(d_mov, nframes, w, h, gop, delta, first_frame, d_lo, d_hi, d_mm, d_hist, st);
     if (rc < 0) return -1;
     if (rc == 1) {  // layouts the fused kernel does not take: the two kernels
-        if (launch_precode_movie(d_mov, nframes, w, h, gop, delta, first_frame, (u8*)o[0].dev, (u8*)o[1].dev, st) != 0) return -1;
-        if (launch_movie_stats(d_mov, n, nullptr, (unsigned*)o[2].dev, (unsigned long long*)o[3].dev, st) != 0) return -1;
+        if (launch_precode_movie(d_mov, nframes, w, h, gop, delta, first_frame, d_lo, d_hi, st) != 0) return -1;
+        if (launch_movie_stats(d_mov, n, nullptr, d_mm, d_hist, st) != 0) return -1;
     }
-    return finish_out(o, 4, st);
+    return c.finish();
 }
 
 int rirb_decode_movie(const unsigned char* lo, const unsigned char* hi, long long nframes, int w, int h, int gop, int delta,
@@ -1202,14 +1148,13 @@ int rirb_decode_movie(const unsigned char* lo, const unsigned char* hi, long lon
     RIRB_REQUIRE_DEVICE();
     cudaStream_t st = tls.stream;
     const size_t n = (size_t)w * h * (size_t)nframes;
-    if (refuse_overlap("decode_movie", {{"lo", lo, n}, {"hi", hi, n}}, {{"movie", movie, n * 2}})) return -1;
-    const u8* d_lo = (const u8*)stage_in(lo, n, 0, st);
-    const u8* d_hi = (const u8*)stage_in(hi, n, 1, st);
-    if (!d_lo || !d_hi) return -1;
-    StagedOut o;
-    if (!stage_out(o, movie, n * 2, 2, false, st)) return -1;
-    if (launch_decode_movie(d_lo, d_hi, nframes, w, h, gop, delta, first_frame, (u16*)o.dev, st) != 0) return -1;
-    return finish_out(&o, 1, st);
+    Call c("decode_movie");
+    auto& l = c.in("lo", lo, n);
+    auto& hh = c.in("hi", hi, n);
+    auto& m = c.out("movie", movie, n * 2);
+    if (c.stage() != 0) return -1;
+    if (launch_decode_movie((const u8*)l.dev, (const u8*)hh.dev, nframes, w, h, gop, delta, first_frame, (u16*)m.dev, st) != 0) return -1;
+    return c.finish();
 }
 
 // host-side writer logic, no device involved: AddFrame's key-frame decision (h264.cpp:1050-1061)
@@ -1256,8 +1201,7 @@ struct LossyState {
         if (bp_handle) bad_pixels_destroy(bp_handle);
     }
 };
-std::mutex g_lossy_mutex;
-std::map<int, std::shared_ptr<LossyState>> g_lossy;
+Table<LossyState> g_lossy;
 }  // namespace
 
 int rirb_lossy_open(int w, int h, int stop_lossy_height, int low_error, int high_error, double std_factor, int running_average,
@@ -1291,30 +1235,14 @@ int rirb_lossy_open(int w, int h, int stop_lossy_height, int low_error, int high
         set_error("lossy_open: out of device memory (%zu bytes): %s", off, cudaGetErrorString(cudaGetLastError()));
         return 0;
     }
-    std::lock_guard<std::mutex> lock(g_lossy_mutex);
-    int id = 1;
-    for (auto& kv : g_lossy) {
-        if (kv.first != id) break;
-        ++id;
-    }
-    g_lossy[id] = s;
-    return id;
+    return g_lossy.add(s);
 }
 
-void rirb_lossy_close(int handle)
-{
-    std::lock_guard<std::mutex> lock(g_lossy_mutex);
-    g_lossy.erase(handle);
-}
+void rirb_lossy_close(int handle) { g_lossy.remove(handle); }
 
 int rirb_lossy_set_parameter(int handle, const char* key, const char* value)
 {
-    std::shared_ptr<LossyState> s;
-    {
-        std::lock_guard<std::mutex> lock(g_lossy_mutex);
-        auto it = g_lossy.find(handle);
-        if (it != g_lossy.end()) s = it->second;
-    }
+    auto s = g_lossy.get(handle);
     if (!s || !key || !value) {
         set_error("lossy_set_parameter: unknown handle %d or NULL argument", handle);
         return -1;
@@ -1343,12 +1271,7 @@ int rirb_lossy_set_parameter(int handle, const char* key, const char* value)
 
 int rirb_lossy_get_min(int handle, int* min_value)
 {
-    std::shared_ptr<LossyState> s;
-    {
-        std::lock_guard<std::mutex> lock(g_lossy_mutex);
-        auto it = g_lossy.find(handle);
-        if (it != g_lossy.end()) s = it->second;
-    }
+    auto s = g_lossy.get(handle);
     if (!s || !min_value) {
         set_error("lossy_get_min: unknown handle %d", handle);
         return -1;
@@ -1364,39 +1287,24 @@ int rirb_lossy_get_min(int handle, int* min_value)
 
 int rirb_lossy_add_images(int handle, const unsigned short* frames, long long nframes, unsigned short* out, int* errors)
 {
-    std::shared_ptr<LossyState> s;
-    {
-        std::lock_guard<std::mutex> lock(g_lossy_mutex);
-        auto it = g_lossy.find(handle);
-        if (it != g_lossy.end()) s = it->second;
-    }
-    if (!s) {
-        set_error("lossy_add_images: unknown handle %d", handle);
-        return -1;
-    }
+    auto s = find_handle_here(g_lossy, handle, "lossy_add_images");
+    if (!s) return -1;
     if (!frames || !out || nframes < 0) {
         set_error("lossy_add_images: bad arguments");
         return -1;
     }
     if (nframes == 0) return 0;
     RIRB_REQUIRE_DEVICE();
-    {
-        int dev = -1;
-        if (cudaGetDevice(&dev) != cudaSuccess) cudaGetLastError();
-        if (dev != s->device) {
-            set_error("lossy_add_images: handle %d belongs to CUDA device %d, the calling thread is on device %d", handle, s->device, dev);
-            return -1;
-        }
-    }
     cudaStream_t st = tls.stream;
     const int w = s->w, h = s->h, n = w * h, ns = w * s->stop_h;
     const size_t bytes = (size_t)n * 2 * (size_t)nframes;
-    if (refuse_overlap("lossy_add_images", {{"frames", frames, bytes}}, {{"out", out, bytes}, {"errors", errors, sizeof(int) * 2 * (size_t)nframes}}))
-        return -1;
-    const u16* d_in = (const u16*)stage_in(frames, bytes, 0, st);
-    if (!d_in) return -1;
-    StagedOut o;
-    if (!stage_out(o, out, bytes, 1, false, st)) return -1;
+    Call c("lossy_add_images");
+    auto& i = c.in("frames", frames, bytes);
+    auto& o = c.out("out", out, bytes);
+    auto& e = c.out("errors", errors, sizeof(int) * 2 * (size_t)nframes);
+    e.staged = false;  // copied from the state's own buffer at the end, in any memory
+    if (c.stage() != 0) return -1;
+    const u16* d_in = (const u16*)i.dev;
     if (s->errors_cap < nframes) {
         if (s->errors_dev) cudaFree(s->errors_dev);
         s->errors_dev = nullptr;
@@ -1430,7 +1338,7 @@ int rirb_lossy_add_images(int handle, const unsigned short* frames, long long nf
                     RIRB_CUDA_OK(cudaMalloc((void**)&s->cur_batch, (size_t)lossy_max_run() * n * 2));
                     s->cur_batch_frames = (size_t)lossy_max_run();
                 }
-                auto bp = find_handle(s->bp_handle);
+                auto bp = g_bad_pixels.get(s->bp_handle);
                 if (!bp) {
                     set_error("lossy_add_images: the bad-pixel handle of the first frame is gone");
                     return -1;
@@ -1459,7 +1367,7 @@ int rirb_lossy_add_images(int handle, const unsigned short* frames, long long nf
                 s->bp_handle = bad_pixels_create((unsigned short*)img, w, s->stop_h);
                 if (s->bp_handle == 0) return -1;
             }
-            auto bp = find_handle(s->bp_handle);
+            auto bp = g_bad_pixels.get(s->bp_handle);
             if (launch_bp_correct(img, tmp, bp->xy_dev, bp->span_off_dev, w, s->stop_h, bp->clamp_value, 1, (size_t)n, st) != 0) return -1;
             if (n > ns) RIRB_CUDA_OK(cudaMemcpyAsync(tmp + ns, img + ns, (size_t)(n - ns) * 2, cudaMemcpyDeviceToDevice, st));
             cur = tmp;
@@ -1475,9 +1383,7 @@ int rirb_lossy_add_images(int handle, const unsigned short* frames, long long nf
         ++f;
     }
     if (errors) RIRB_CUDA_OK(cudaMemcpyAsync(errors, s->errors_dev, sizeof(int) * 2 * (size_t)nframes, cudaMemcpyDefault, st));
-    if (o.host) RIRB_CUDA_OK(copy_d2h(o.host, o.dev, o.bytes, st));
-    if (o.host || (errors && !is_device_ptr(errors))) RIRB_CUDA_OK(cudaStreamSynchronize(st));
-    return 0;
+    return c.finish(errors && !e.on_device);
 }
 
 // =================================================================================================
@@ -1512,7 +1418,7 @@ int rirb_process_movie_host(int handle, const unsigned short* frames, long long 
                             const float* dy, const char* strategy, unsigned int background, int gop, int delta,
                             long long first_frame, unsigned char* lo, unsigned char* hi, float* smoothed)
 {
-    auto s = find_handle_here(handle, "process_movie_host");
+    auto s = find_handle_here(g_bad_pixels, handle, "process_movie_host");
     if (!s) return -1;
     const int strat = strategy_code(strategy);
     if (!frames || !dx || !dy || !lo || !hi || w != s->w || h != s->h || nframes < 0 || gop < 1 || strat < 0 ||
@@ -1589,6 +1495,7 @@ int rirb_process_movie_host(int handle, const unsigned short* frames, long long 
     long long k = 0;
     for (long long a = 0; a < nframes && rc == 0; a += sub, ++k) {
         const long long m = (nframes - a < sub) ? nframes - a : sub;
+        Call scope("process_movie_host");  // gives back the order buffer launch_translate_u16 may take, sub-chunk by sub-chunk
         HostPipeSlot& sl = hp.slot[k % HP_SLOTS];
         cudaStream_t st = sl.stream;
         char* base = (char*)sl.buf;
@@ -1648,18 +1555,17 @@ int rirb_movie_stats(const unsigned short* pixels, size_t n, unsigned int* minma
         return -1;
     }
     RIRB_REQUIRE_DEVICE();
-    if (refuse_overlap("movie_stats", {{"pixels", pixels, n * 2}},
-                       {{"minmax", minmax, 2 * sizeof(unsigned)}, {"hist", hist, 65536 * sizeof(unsigned long long)}}))
-        return -1;
     cudaStream_t st = tls.stream;
-    const u16* d_p = (const u16*)stage_in(pixels, n * 2, 0, st);
-    if (!d_p) return -1;
-    StagedOut o[2];
-    if (!stage_out(o[0], minmax, 2 * sizeof(unsigned), 1, accumulate != 0, st)) return -1;
-    if (hist && !stage_out(o[1], hist, 65536 * sizeof(unsigned long long), 2, accumulate != 0, st)) return -1;
-    if (!accumulate && launch_stats_init((unsigned*)o[0].dev, (unsigned long long*)o[1].dev, st) != 0) return -1;
-    if (launch_movie_stats(d_p, n, nullptr, (unsigned*)o[0].dev, (unsigned long long*)o[1].dev, st) != 0) return -1;
-    return finish_out(o, 2, st);
+    Call c("movie_stats");
+    auto& px = c.in("pixels", pixels, n * 2);
+    auto& mm = c.out("minmax", minmax, 2 * sizeof(unsigned), accumulate != 0);
+    auto& hs = c.out("hist", hist, 65536 * sizeof(unsigned long long), accumulate != 0);
+    if (c.stage() != 0) return -1;
+    unsigned* d_mm = (unsigned*)mm.dev;
+    unsigned long long* d_hist = (unsigned long long*)hs.dev;
+    if (!accumulate && launch_stats_init(d_mm, d_hist, st) != 0) return -1;
+    if (launch_movie_stats((const u16*)px.dev, n, nullptr, d_mm, d_hist, st) != 0) return -1;
+    return c.finish();
 }
 
 int rirb_hist_quantile(const unsigned long long* hist, long long count, float percent)
@@ -1670,10 +1576,12 @@ int rirb_hist_quantile(const unsigned long long* hist, long long count, float pe
     }
     RIRB_REQUIRE_DEVICE();
     cudaStream_t st = tls.stream;
-    const unsigned long long* d_h = (const unsigned long long*)stage_in(hist, 65536 * sizeof(unsigned long long), 0, st);
-    int* d_out = (int*)scratch(5, sizeof(int));
-    if (!d_h || !d_out) return -1;
-    if (launch_hist_quantile(d_h, count, percent, 0, d_out, st) != 0) return -1;
+    Call c("hist_quantile");
+    auto& hs = c.in("hist", hist, 65536 * sizeof(unsigned long long));
+    if (c.stage() != 0) return -1;
+    int* d_out = (int*)scratch_buffer(sizeof(int));
+    if (!d_out) return -1;
+    if (launch_hist_quantile((const unsigned long long*)hs.dev, count, percent, 0, d_out, st) != 0) return -1;
     int r = 0;
     RIRB_CUDA_OK(cudaMemcpyAsync(&r, d_out, sizeof(int), cudaMemcpyDeviceToHost, st));
     RIRB_CUDA_OK(cudaStreamSynchronize(st));
@@ -1688,19 +1596,16 @@ static int median_pixel_any(const unsigned short* pixels, const unsigned char* m
     }
     RIRB_REQUIRE_DEVICE();
     cudaStream_t st = tls.stream;
-    const u16* d_p = (const u16*)stage_in(pixels, (size_t)size * 2, 0, st);
-    if (!d_p && size) return -1;
-    const u8* d_m = nullptr;
-    if (mask) {
-        d_m = (const u8*)stage_in(mask, (size_t)size, 1, st);
-        if (!d_m && size) return -1;
-    }
-    unsigned long long* d_hist = (unsigned long long*)scratch(2, 65536 * sizeof(unsigned long long));
-    unsigned* d_mm = (unsigned*)scratch(3, 2 * sizeof(unsigned));
-    int* d_out = (int*)scratch(5, sizeof(int));
+    Call c("find_median_pixel");
+    auto& px = c.in("pixels", pixels, (size_t)size * 2);
+    auto& m = c.in("mask", mask, (size_t)size);
+    if (c.stage() != 0) return -1;
+    unsigned long long* d_hist = (unsigned long long*)scratch_buffer(sizeof(unsigned long long) * 65536);
+    unsigned* d_mm = (unsigned*)scratch_buffer(sizeof(unsigned) * 2);
+    int* d_out = (int*)scratch_buffer(sizeof(int));
     if (!d_hist || !d_mm || !d_out) return -1;
     if (launch_stats_init(d_mm, d_hist, st) != 0) return -1;
-    if (launch_movie_stats(d_p, (size_t)size, d_m, d_mm, d_hist, st) != 0) return -1;
+    if (launch_movie_stats((const u16*)px.dev, (size_t)size, (const u8*)m.dev, d_mm, d_hist, st) != 0) return -1;
     if (launch_hist_quantile(d_hist, mask ? -1 : (long long)size, percent, mask ? 1 : 0, d_out, st) != 0) return -1;
     int r = 0;
     RIRB_CUDA_OK(cudaMemcpyAsync(&r, d_out, sizeof(int), cudaMemcpyDeviceToHost, st));
@@ -1726,13 +1631,15 @@ int rirb_get_background(const unsigned short* pixels, int size)
     }
     RIRB_REQUIRE_DEVICE();
     cudaStream_t st = tls.stream;
-    const u16* d_p = (const u16*)stage_in(pixels, (size_t)size * 2, 0, st);
-    unsigned long long* d_hist = (unsigned long long*)scratch(2, 65536 * sizeof(unsigned long long));
-    unsigned* d_mm = (unsigned*)scratch(3, 2 * sizeof(unsigned));
-    unsigned* d_out = (unsigned*)scratch(5, sizeof(unsigned));
-    if (!d_p || !d_hist || !d_mm || !d_out) return -1;
+    Call c("get_background");
+    auto& px = c.in("pixels", pixels, (size_t)size * 2);
+    if (c.stage() != 0) return -1;
+    unsigned long long* d_hist = (unsigned long long*)scratch_buffer(sizeof(unsigned long long) * 65536);
+    unsigned* d_mm = (unsigned*)scratch_buffer(sizeof(unsigned) * 2);
+    unsigned* d_out = (unsigned*)scratch_buffer(sizeof(unsigned));
+    if (!d_hist || !d_mm || !d_out) return -1;
     if (launch_stats_init(d_mm, d_hist, st) != 0) return -1;
-    if (launch_movie_stats(d_p, (size_t)size, nullptr, d_mm, d_hist, st) != 0) return -1;
+    if (launch_movie_stats((const u16*)px.dev, (size_t)size, nullptr, d_mm, d_hist, st) != 0) return -1;
     if (launch_hist_mode4(d_hist, d_out, st) != 0) return -1;
     unsigned r = 0;
     RIRB_CUDA_OK(cudaMemcpyAsync(&r, d_out, sizeof(unsigned), cudaMemcpyDeviceToHost, st));
@@ -1760,22 +1667,19 @@ int rirb_label_batch(const unsigned short* frames, int w, int h, long long nfram
     const int cap = stats ? max_components : 0;
     const size_t npx = (size_t)w * h * (size_t)nframes;
     const size_t sbytes = (size_t)nframes * cap * 10 * sizeof(long long);
-    if (refuse_overlap("label_batch", {{"frames", frames, npx * 2}, {"thresholds", thresholds, 2 * (size_t)n_thresholds}},
-                       {{"labels", labels, npx * 4}, {"counts", counts, 4 * (size_t)nframes}, {"stats", stats, sbytes}}))
-        return -1;
     cudaStream_t st = tls.stream;
-    const u16* d_frames = (const u16*)stage_in(frames, npx * 2, 0, st);
-    const u16* d_thr = (const u16*)stage_in(thresholds, 2 * (size_t)n_thresholds, 2, st);
-    if (!d_frames || !d_thr) return -1;
-    StagedOut outs[3];
-    if (!stage_out(outs[0], labels, npx * 4, 1, false, st) || !stage_out(outs[1], counts, 4 * (size_t)nframes, 3, false, st))
-        return -1;
+    Call c("label_batch");
+    auto& fr = c.in("frames", frames, npx * 2);
+    auto& th = c.in("thresholds", thresholds, 2 * (size_t)n_thresholds);
+    auto& lb = c.out("labels", labels, npx * 4);
+    auto& ct = c.out("counts", counts, 4 * (size_t)nframes);
     // rows past K_t keep what the caller had in them: a host stats array goes up first
-    if (sbytes && !stage_out(outs[2], stats, sbytes, 4, true, st)) return -1;
-    if (launch_label(d_frames, w, h, nframes, d_thr, n_thresholds > 1, connectivity, (int*)outs[0].dev, (int*)outs[1].dev,
-                     (long long*)outs[2].dev, cap, st) != 0)
+    auto& sts = c.out("stats", sbytes ? stats : nullptr, sbytes, true);
+    if (c.stage() != 0) return -1;
+    if (launch_label((const u16*)fr.dev, w, h, nframes, (const u16*)th.dev, n_thresholds > 1, connectivity, (int*)lb.dev, (int*)ct.dev,
+                     (long long*)sts.dev, cap, st) != 0)
         return -1;
-    return finish_out(outs, 3, st);
+    return c.finish();
 }
 
 int rirb_label_movie(const unsigned short* frames, int w, int h, long long nframes, const unsigned short* thresholds,
@@ -1807,21 +1711,19 @@ int rirb_label_movie(const unsigned short* frames, int w, int h, long long nfram
     const int cap = stats ? max_events : 0;
     const size_t npx = (size_t)w * h * (size_t)nframes;
     const size_t sbytes = (size_t)cap * 13 * sizeof(long long);
-    if (refuse_overlap("label_movie", {{"frames", frames, npx * 2}, {"thresholds", thresholds, 2 * (size_t)n_thresholds}},
-                       {{"labels", labels, npx * 4}, {"count", count, sizeof(int)}, {"stats", stats, sbytes}}))
-        return -1;
     cudaStream_t st = tls.stream;
-    const u16* d_frames = (const u16*)stage_in(frames, npx * 2, 0, st);
-    const u16* d_thr = (const u16*)stage_in(thresholds, 2 * (size_t)n_thresholds, 2, st);
-    if (!d_frames || !d_thr) return -1;
-    StagedOut outs[3];
-    if (!stage_out(outs[0], labels, npx * 4, 1, false, st) || !stage_out(outs[1], count, sizeof(int), 3, false, st)) return -1;
+    Call c("label_movie");
+    auto& fr = c.in("frames", frames, npx * 2);
+    auto& th = c.in("thresholds", thresholds, 2 * (size_t)n_thresholds);
+    auto& lb = c.out("labels", labels, npx * 4);
+    auto& ct = c.out("count", count, sizeof(int));
     // rows past K keep what the caller had in them: a host stats array goes up first
-    if (sbytes && !stage_out(outs[2], stats, sbytes, 4, true, st)) return -1;
-    if (launch_label_movie(d_frames, w, h, nframes, d_thr, n_thresholds > 1, connectivity, (int*)outs[0].dev, (int*)outs[1].dev,
-                           (long long*)outs[2].dev, cap, st) != 0)
+    auto& sts = c.out("stats", sbytes ? stats : nullptr, sbytes, true);
+    if (c.stage() != 0) return -1;
+    if (launch_label_movie((const u16*)fr.dev, w, h, nframes, (const u16*)th.dev, n_thresholds > 1, connectivity, (int*)lb.dev,
+                           (int*)ct.dev, (long long*)sts.dev, cap, st) != 0)
         return -1;
-    return finish_out(outs, 3, st);
+    return c.finish();
 }
 
 // =================================================================================================

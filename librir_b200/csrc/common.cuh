@@ -13,7 +13,10 @@
 #include <stdio.h>
 
 #include <atomic>
+#include <memory>
 #include <string>
+
+#include "handles.h"
 
 namespace rirb {
 
@@ -25,6 +28,7 @@ void set_error(const char* fmt, ...);
 cudaStream_t current_stream();
 extern std::atomic<long long> g_launches;
 int sm_count();
+int require_device();  // -1 (set_error) when there is no usable CUDA device: this library has no CPU fallback
 // run-time switches (rirb_set_parameter; initial values from the environment): kernel variants for A/B runs
 enum { OPT_TRANSLATE_TMA = 0, OPT_GAUSS_TMA = 1, OPT_LOADER_FUSED = 2, OPT_ECC_FUSED = 3, OPT_LOSSY_RUN = 4, OPT_TRANSLATE_ROWS = 5, OPT_ECC_QUEUE = 6, OPT_ZSTD_DECODER = 7, OPT_COUNT = 8 };
 bool option_enabled(int which);
@@ -65,6 +69,24 @@ int option_value(int which);  // the switch's integer value (option_enabled: != 
             _done.fetch_or(_bit, std::memory_order_relaxed);                                               \
         }                                                                                                  \
     } while (0)
+
+// A handle's buffers live in the memory of the device it was created on (T::device): entries that launch kernels refuse a
+// handle from another device instead of faulting on its pointers.  nullptr (set_error) when unknown or elsewhere.
+template <typename T> std::shared_ptr<T> find_handle_here(Table<T>& table, int id, const char* what)
+{
+    auto s = table.get(id);
+    if (!s) {
+        set_error("%s: unknown handle %d", what, id);
+        return nullptr;
+    }
+    int dev = -1;
+    if (cudaGetDevice(&dev) != cudaSuccess) cudaGetLastError();
+    if (dev != s->device) {
+        set_error("%s: handle %d belongs to CUDA device %d, the calling thread is on device %d", what, id, s->device, dev);
+        return nullptr;
+    }
+    return s;
+}
 
 static inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 static inline long long ceil_div(long long a, long long b) { return (a + b - 1) / b; }

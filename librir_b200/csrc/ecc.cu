@@ -530,7 +530,7 @@ ecc_solve_kernel(const float* __restrict__ ref, float* cur, const float* cur_src
 
 // ---- host side ------------------------------------------------------------------------------------
 struct EccState {
-    int w = 0, h = 0, dev = 0;
+    int w = 0, h = 0, device = 0;
     float *ref = nullptr, *cur = nullptr, *T = nullptr, *I = nullptr, *gx = nullptr, *gy = nullptr;
     u8 *mask = nullptr, *qmask = nullptr;  // ECC mask; mask of the quantile thresholds (see rirb_ecc_set_mask)
     bool have_mask = false, have_qmask = false, have_ref = false, have_cur = false;
@@ -582,44 +582,6 @@ struct EccState {
     }
 };
 static Table<EccState> g_ecc;
-
-// Buffers live on the device the handle was opened on: refuse calls from a thread that is on another one.
-static std::shared_ptr<EccState> ecc_get(int handle, const char* what)
-{
-    auto s = g_ecc.get(handle);
-    if (!s) {
-        set_error("%s: unknown handle %d", what, handle);
-        return nullptr;
-    }
-    int dev = -1;
-    if (cudaGetDevice(&dev) != cudaSuccess) cudaGetLastError();
-    if (dev != s->dev) {
-        set_error("%s: handle %d belongs to CUDA device %d, the calling thread is on device %d", what, handle, s->dev, dev);
-        return nullptr;
-    }
-    return s;
-}
-
-static int ecc_need_device()
-{
-    int n = 0;
-    if (cudaGetDeviceCount(&n) != cudaSuccess || n <= 0) {
-        cudaGetLastError();
-        set_error("no usable CUDA device: librir_b200 computes on the GPU only and has no CPU fallback");
-        return -1;
-    }
-    return 0;
-}
-
-static bool is_device_pointer(const void* p)
-{
-    cudaPointerAttributes a;
-    if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
-        cudaGetLastError();
-        return false;
-    }
-    return a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged;
-}
 
 static int ecc_load_window(EccState& s, float* dst, const float* src, int stride, cudaStream_t st)
 {
@@ -895,11 +857,11 @@ int rirb_ecc_open(int width, int height)
         set_error("ecc_open: bad window size %d x %d", width, height);
         return 0;
     }
-    if (ecc_need_device() != 0) return 0;
+    if (require_device() != 0) return 0;
     auto s = std::make_shared<EccState>();
     s->w = width;
     s->h = height;
-    cudaGetDevice(&s->dev);
+    cudaGetDevice(&s->device);
     const size_t n = (size_t)width * height;
     bool ok = true;
     for (float** p : {&s->ref, &s->cur, &s->T, &s->I, &s->gx, &s->gy}) ok = ok && cudaMalloc((void**)p, n * 4) == cudaSuccess;
@@ -917,7 +879,7 @@ int rirb_ecc_open(int width, int height)
     }
     // the one-launch solver needs every CTA resident at once: one per SM, if the device can launch cooperatively
     int coop = 0, per_sm = 0;
-    if (cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, s->dev) == cudaSuccess && coop &&
+    if (cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, s->device) == cudaSuccess && coop &&
         cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ecc_solve_kernel, ECC_THREADS, 0) == cudaSuccess && per_sm >= 1)
         s->coop_grid = (int)min((long long)sm_count(), (long long)ceil_div((long long)n, ECC_THREADS));
     cudaGetLastError();
@@ -932,7 +894,7 @@ void rirb_ecc_close(int handle) { g_ecc.remove(handle); }
 // uint8 mask its thresholds are taken under a different pixel set than the one ECC uses; the Python mirror reproduces that.
 int rirb_ecc_set_mask(int handle, int which, const unsigned char* mask)
 {
-    auto s = ecc_get(handle, "ecc_set_mask");
+    auto s = find_handle_here(g_ecc, handle, "ecc_set_mask");
     if (!s) return -1;
     if (!s || (which != 0 && which != 1)) {
         set_error("ecc: unknown handle %d or mask selector", handle);
@@ -948,7 +910,7 @@ int rirb_ecc_set_mask(int handle, int which, const unsigned char* mask)
 // float image whose rows are `stride` floats apart (host or device).
 int rirb_ecc_set_image(int handle, int which, const float* img, int stride)
 {
-    auto s = ecc_get(handle, "ecc_set_image");
+    auto s = find_handle_here(g_ecc, handle, "ecc_set_image");
     if (!s) return -1;
     if (!s || (which != 0 && which != 1)) {
         set_error("ecc: unknown handle %d or image selector", handle);
@@ -964,7 +926,7 @@ int rirb_ecc_set_image(int handle, int which, const float* img, int stride)
 // with translate's default ("noborder") strategy, on the un-normalised float window.
 int rirb_ecc_reset_reference(int handle, float dx, float dy)
 {
-    auto s = ecc_get(handle, "ecc_reset_reference");
+    auto s = find_handle_here(g_ecc, handle, "ecc_reset_reference");
     if (!s) return -1;
     if (!s || !s->have_cur) {
         set_error("ecc_reset_reference: unknown handle or no current image");
@@ -983,7 +945,7 @@ int rirb_ecc_reset_reference(int handle, float dx, float dy)
 // find_median_pixel(window.astype(uint16), percent, mask) of the reference (0) or current (1) window (:144-145)
 int rirb_ecc_quantile(int handle, int which, float percent, int use_mask)
 {
-    auto s = ecc_get(handle, "ecc_quantile");
+    auto s = find_handle_here(g_ecc, handle, "ecc_quantile");
     if (!s) return -1;
     if (!s || (which != 0 && which != 1) || !(which ? s->have_cur : s->have_ref)) {
         set_error("ecc_quantile: unknown handle or image not set");
@@ -1009,7 +971,7 @@ int rirb_ecc_quantile(int handle, int which, float percent, int use_mask)
 // 2 = "the correlation is going to be minimized" (both are cv2.error in the reference); -1 = bad call.
 int rirb_ecc_compute(int handle, float thresh, int use_mask, int max_iterations, double eps, float* shift, double* rho, int* iterations)
 {
-    auto s = ecc_get(handle, "ecc_compute");
+    auto s = find_handle_here(g_ecc, handle, "ecc_compute");
     if (!s) return -1;
     if (!s || !s->have_ref || !s->have_cur || !shift) {
         set_error("ecc_compute: unknown handle, or reference / current image not set");
@@ -1086,7 +1048,7 @@ int rirb_ecc_track_state(int handle, double* median, double* conf_thresh, float*
 int rirb_ecc_track(int handle, int type, const void* frames, long long nframes, int full_w, int full_h, int x0, int y0, int use_mask,
                    int max_try, double* x, double* y, double* conf, int* iters, long long* processed)
 {
-    auto s = ecc_get(handle, "ecc_track");
+    auto s = find_handle_here(g_ecc, handle, "ecc_track");
     if (!s) return -1;
     if (processed) *processed = 0;
     if (!s || !frames || nframes < 0 || !x || !y || !conf || (type != 'H' && type != 'f') || x0 < 0 || y0 < 0 || x0 + s->w > full_w ||
@@ -1101,7 +1063,7 @@ int rirb_ecc_track(int handle, int type, const void* frames, long long nframes, 
     }
     cudaStream_t st = current_stream();
     const size_t fpx = (size_t)full_w * full_h, esz = type == 'H' ? 2 : 4;
-    const bool on_device = is_device_pointer(frames);
+    const bool on_device = operand_on_device(frames);
     if (!on_device && nframes > 0 && ecc_prefetch(*s, frames, fpx * esz, 0) != 0) return -1;
     if (s->filtered_cap < fpx * 4) {
         if (s->filtered) cudaFree(s->filtered);

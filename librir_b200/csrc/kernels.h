@@ -65,8 +65,9 @@ int launch_gaussian_f32_region(const float* src, size_t src_row, size_t src_fram
 int launch_gaussian_bp_u16(const u16* raw, u16* corrected, float* dst, int w, int h, long long nframes, const GaussTaps& taps,
                            const int* xy_dev, const int* row_off_dev, int clamp_value, cudaStream_t st);
 
-// capi.cu: grow-only per-thread device work space for launchers, slots 8..11 (nullptr + set_error when out of memory)
-void* scratch_buffer(int slot, size_t bytes);
+// capi.cu: grow-only device work space of the calling thread, the next buffer the enclosing C-ABI entry has not taken; it
+// stays the caller's until that entry returns (nullptr + set_error when out of memory or of buffers)
+void* scratch_buffer(size_t bytes);
 
 // The operand checks of the entries, defined here so that every source file that has an entry carries them (the host
 // build of zdecoder.cu in the tests included).  A kernel that writes bytes it (or another kernel of the same call) also
@@ -78,6 +79,7 @@ struct Operand {
     const char* name;
     const void* p;
     size_t bytes;
+    int on_device = -1;  // 1: device or managed memory, 0: host memory, -1: not looked up yet
 };
 inline bool bytes_overlap(const Operand& a, const Operand& b)
 {
@@ -99,21 +101,27 @@ inline bool operand_on_device(const void* p)
     const cudaMemoryType t = operand_memory_type(p);
     return t == cudaMemoryTypeDevice || t == cudaMemoryTypeManaged;
 }
-inline int refuse_overlap(const char* what, std::initializer_list<Operand> ins, std::initializer_list<Operand> outs)
+inline bool operand_on_device(const Operand& o) { return o.on_device >= 0 ? o.on_device != 0 : operand_on_device(o.p); }
+// [ib, ie) inputs and [ob, oe) outputs, each in the order the entry names them (the first offending pair is reported)
+template <typename In, typename Out> inline int refuse_overlap(const char* what, In ib, In ie, Out ob, Out oe)
 {
-    for (auto o = outs.begin(); o != outs.end(); ++o) {
-        for (const Operand& i : ins)
-            if (bytes_overlap(*o, i) && operand_on_device(o->p) && operand_on_device(i.p)) {
-                set_error("%s: %s and %s overlap in device memory", what, i.name, o->name);
+    for (Out o = ob; o != oe; ++o) {
+        for (In i = ib; i != ie; ++i)
+            if (bytes_overlap(*o, *i) && operand_on_device(*o) && operand_on_device(*i)) {
+                set_error("%s: %s and %s overlap in device memory", what, i->name, o->name);
                 return -1;
             }
-        for (auto q = outs.begin(); q != o; ++q)
+        for (Out q = ob; q != o; ++q)
             if (bytes_overlap(*o, *q)) {
                 set_error("%s: the outputs %s and %s overlap", what, q->name, o->name);
                 return -1;
             }
     }
     return 0;
+}
+inline int refuse_overlap(const char* what, std::initializer_list<Operand> ins, std::initializer_list<Operand> outs)
+{
+    return refuse_overlap(what, ins.begin(), ins.end(), outs.begin(), outs.end());
 }
 // -1 (set_error naming the operand) unless every non-null pointer is device, managed or page-locked host memory: what a
 // kernel may dereference directly
@@ -179,12 +187,12 @@ int launch_lossy_frame(const u16* img, const u16* tmp, u16* tmpT, u16* out, u16*
                        cudaStream_t st);
 
 // label.cu (rirb_label_batch): labels[t] (the parent array while it runs) and counts[t] for nframes frames; stats NULL or
-// [nframes][cap][10].  thr: one threshold, or one per frame when per_frame_thr.  Work space: scratch slot 8.
+// [nframes][cap][10].  thr: one threshold, or one per frame when per_frame_thr.  Work space: one scratch_buffer.
 int launch_label(const u16* frames, int w, int h, long long nframes, const u16* thr, int per_frame_thr, int connectivity,
                  int* labels, int* counts, long long* stats, int cap, cudaStream_t st);
 // label.cu (rirb_label_movie): events of the (t, y, x) volume at connectivity 6, 18 or 26; labels [nframes][h][w], *count
 // = K, stats NULL or [cap][13].  nframes >= 1.  Synchronises st once to read the number of 2-D components (twice when
-// that exceeds INT_MAX).  Work space: scratch slots 8 (launch_label) to 11.
+// that exceeds INT_MAX).  Work space: four scratch_buffers, launch_label's included.
 int launch_label_movie(const u16* frames, int w, int h, long long nframes, const u16* thr, int per_frame_thr, int connectivity,
                        int* labels, int* count, long long* stats, int cap, cudaStream_t st);
 

@@ -398,7 +398,7 @@ int launch_label(const u16* frames, int w, int h, long long nframes, const u16* 
     const long long by_scratch = (long long)((256u << 20) / (8 * g.segs));
     if (per > by_scratch) per = by_scratch > 0 ? by_scratch : 1;
     if (per > nframes) per = nframes;
-    unsigned* roots = (unsigned*)scratch_buffer(8, (size_t)per * g.segs * 2 * sizeof(unsigned));
+    unsigned* roots = (unsigned*)scratch_buffer((size_t)per * g.segs * 2 * sizeof(unsigned));
     if (!roots) return -1;
     int* off = (int*)(roots + (size_t)per * g.segs);
     const dim3 tile_block(LB_TW, LB_BY);
@@ -682,19 +682,19 @@ int launch_label_movie(const u16* frames, int w, int h, long long nframes, const
 {
     const LabelGeom g = label_geom(w, h);
     if (cap <= 0) stats = nullptr;
-    // slot 9: K_t [n] | base [n + 1] | the scan's work space
+    // K_t [n] | base [n + 1] | the scan's work space
     const long long n1 = nframes + 1;
     size_t tmp1 = 0;
     RIRB_CUDA_OK(cub::DeviceScan::ExclusiveSum(nullptr, tmp1, (long long*)nullptr, n1, st));
     const size_t o_base = align256((size_t)nframes * sizeof(int)), o_tmp1 = o_base + align256((size_t)n1 * sizeof(long long));
-    char* s9 = (char*)scratch_buffer(9, o_tmp1 + tmp1);
-    if (!s9) return -1;
-    int* kt = (int*)s9;
-    long long* base = (long long*)(s9 + o_base);
+    char* frame_ws = (char*)scratch_buffer(o_tmp1 + tmp1);
+    if (!frame_ws) return -1;
+    int* kt = (int*)frame_ws;
+    long long* base = (long long*)(frame_ws + o_base);
     if (launch_label(frames, w, h, nframes, thr, per_frame_thr, connectivity == 6 ? 4 : 8, labels, kt, nullptr, 0, st) != 0)
         return -1;
     RIRB_LAUNCH(movie_widen_kernel, flat_grid(n1), 256, 0, st, kt, base, nframes);
-    RIRB_CUDA_OK(cub::DeviceScan::ExclusiveSum(s9 + o_tmp1, tmp1, base, n1, st));
+    RIRB_CUDA_OK(cub::DeviceScan::ExclusiveSum(frame_ws + o_tmp1, tmp1, base, n1, st));
     long long C = 0;  // 2-D components of the whole movie: the one read-back every call waits for
     RIRB_CUDA_OK(cudaMemcpyAsync(&C, base + nframes, sizeof C, cudaMemcpyDeviceToHost, st));
     RIRB_CUDA_OK(cudaStreamSynchronize(st));
@@ -702,14 +702,14 @@ int launch_label_movie(const u16* frames, int w, int h, long long nframes, const
         RIRB_CUDA_OK(cudaMemsetAsync(count, 0, sizeof(int), st));
         return 0;
     }
-    // slot 10: parents [C]; slot 11: root flags -> event ids [C + 1] | the scan's work space
+    // parents [C]; root flags -> event ids [C + 1] | the scan's work space
     size_t tmp2 = 0;
     RIRB_CUDA_OK(cub::DeviceScan::InclusiveSum(nullptr, tmp2, (long long*)nullptr, C + 1, st));
     const size_t o_tmp2 = align256((size_t)(C + 1) * sizeof(long long));
-    long long* P = (long long*)scratch_buffer(10, (size_t)C * sizeof(long long));
-    char* s11 = (char*)scratch_buffer(11, o_tmp2 + tmp2);
-    if (!P || !s11) return -1;
-    long long* ids = (long long*)s11;
+    long long* P = (long long*)scratch_buffer((size_t)C * sizeof(long long));
+    char* event_ws = (char*)scratch_buffer(o_tmp2 + tmp2);
+    if (!P || !event_ws) return -1;
+    long long* ids = (long long*)event_ws;
     const dim3 tile_block(LB_TW, LB_BY);
     RIRB_LAUNCH(movie_init_kernel, flat_grid(C), 256, 0, st, P, C);
     if (nframes > 1) {
@@ -722,7 +722,7 @@ int launch_label_movie(const u16* frames, int w, int h, long long nframes, const
             RIRB_LAUNCH(movie_link_kernel<26>, tile_grid(items), tile_block, 0, st, g, labels, base, P, items);
     }
     RIRB_LAUNCH(movie_roots_kernel, flat_grid(C + 1), 256, 0, st, P, ids, C);
-    RIRB_CUDA_OK(cub::DeviceScan::InclusiveSum(s11 + o_tmp2, tmp2, ids, C + 1, st));
+    RIRB_CUDA_OK(cub::DeviceScan::InclusiveSum(event_ws + o_tmp2, tmp2, ids, C + 1, st));
     if (C > INT_MAX) {  // only then can the events outnumber a 32-bit label
         long long K = 0;
         RIRB_CUDA_OK(cudaMemcpyAsync(&K, ids + C, sizeof K, cudaMemcpyDeviceToHost, st));

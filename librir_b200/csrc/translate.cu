@@ -1208,6 +1208,12 @@ int launch_translate_u16(const u16* src, u16* dst, int w, int h, long long nfram
         RIRB_SMEM_ATTR((translate_u16_tma_kernel<false, false>), smem);
         RIRB_SMEM_ATTR((translate_u16_rows_kernel<true>), smem);
         RIRB_SMEM_ATTR((translate_u16_rows_kernel<false>), smem);
+        // per-frame shifts: the row kernel takes the frames grouped by their column offset (one order buffer for every launch)
+        int* order_buf = nullptr;
+        if (option_enabled(OPT_TRANSLATE_ROWS) && (motion || option_value(OPT_TRANSLATE_ROWS) >= 2) && dxs && nframes > 1) {
+            order_buf = (int*)scratch_buffer(sizeof(int) * 65536);
+            if (!order_buf) return -1;
+        }
         // grid = (tile column, frame); gridDim.y <= 65535, so long movies go in several launches
         for (long long f0 = 0; f0 < nframes; f0 += 65535) {
             const long long n = min(nframes - f0, 65535LL);
@@ -1220,12 +1226,8 @@ int launch_translate_u16(const u16* src, u16* dst, int w, int h, long long nfram
             const dim3 tgrid((unsigned)tiles_x, (unsigned)n);
             const PlaneSrc none{};
             if (option_enabled(OPT_TRANSLATE_ROWS)) {  // "translate_rows" = 0: the first-generation tiled kernel (A/B)
-                int* order = nullptr;
-                if ((motion || option_value(OPT_TRANSLATE_ROWS) >= 2) && dx_p && n > 1) {  // per-frame shifts: hand the frames out grouped by their column offset
-                    order = (int*)scratch_buffer(8, sizeof(int) * 65536);
-                    if (!order) return -1;
-                    RIRB_LAUNCH(translate_order_kernel, 1, 1024, 0, st, dx_p, (int)n, w, order);
-                }
+                int* order = n > 1 ? order_buf : nullptr;
+                if (order) RIRB_LAUNCH(translate_order_kernel, 1, 1024, 0, st, dx_p, (int)n, w, order);
                 if (motion)
                     RIRB_LAUNCH((translate_u16_rows_kernel<true>), tgrid, TW_THREADS, smem, st, tmap, s0, d0, w, h, src_stride, dst_stride,
                                 dx_p, dy_p, dx0, dy0, strategy, background, tiles_y, order);

@@ -36,38 +36,13 @@
 
 #include "../../include/librir_b200.h"
 #include "../../include/librir_b200_video_io.h"
+#include "handles.h"
 
 namespace {
 
 typedef std::map<std::string, std::string> AttrMap;
 
-// handles: small positive ints, lowest free slot first (tools.cpp:40-85)
-template <typename T> struct Table {
-    std::mutex mu;
-    std::map<int, std::shared_ptr<T>> items;
-    int add(const std::shared_ptr<T>& p)
-    {
-        std::lock_guard<std::mutex> lock(mu);
-        int id = 1;
-        for (auto& kv : items) {
-            if (kv.first != id) break;
-            ++id;
-        }
-        items[id] = p;
-        return id;
-    }
-    std::shared_ptr<T> get(int id)
-    {
-        std::lock_guard<std::mutex> lock(mu);
-        auto it = items.find(id);
-        return it == items.end() ? nullptr : it->second;
-    }
-    void remove(int id)
-    {
-        std::lock_guard<std::mutex> lock(mu);
-        items.erase(id);
-    }
-};
+using rirb::Table;
 
 thread_local std::string g_last_error;
 void fail(const std::string& what)

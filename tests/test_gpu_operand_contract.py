@@ -526,8 +526,9 @@ def test_a_fresh_stream_waits_for_work_still_using_the_slots(lib, data):
 
 
 def test_nested_entries_give_what_they_give_alone(lib, data):
-    """read_movie with motion stages into slots 0-5 and translates; finish_frames calls remove_motion, which stages its
-    shifts; bad_pixels_create uses slots 6-7 between them.  Host operands throughout, no synchronisation in between."""
+    """read_movie with motion stages its operands and shifts and translates; finish_frames calls remove_motion, which
+    stages its shifts above the frames finish_frames holds; bad_pixels_create stages between them.  Host operands
+    throughout, no synchronisation in between."""
     mov = data["mov"]
     lo, hi, sx, sy = data["lo"], data["hi"], data["sx"], data["sy"]
     bpl = vio.LoaderBadPixels(mov[0])
